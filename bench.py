@@ -36,6 +36,9 @@ BASELINE_MIN, BASELINE_MAX = 4700.0, 5300.0
 EVENT_PAD, MINPOINTS, MAXPOINTS = 100, 8, 100_000
 E2E_SHARDS = 16                      # time sub-shards of the streamed end-to-end run (pipeline.StreamingAnalyzer)
 CUSUM_DELTA, CUSUM_H = 400.0, 10.0
+# --dump-outputs: 512 windows of 8192 filtered samples (17 MB) and 65 536 event rows (30 MB) at most
+DUMP_WINDOWS, DUMP_WINDOW, DUMP_EVENTS, DUMP_SEED = 512, 8192, 1 << 16, 0
+DUMP_BUDGET = 64_000_000
 METRIC = "Msamples/s filtered+CUSUM-segmented"
 FILTER_BYTES_PER_SAMPLE = 6.0     # 2 B uint16 read + 4 B float32 written (SURVEY.md 8d)
 
@@ -338,6 +341,56 @@ def parity_at_size(torch, dist, group, an, raw, r, S, lo_h, n_own, rank, world):
     return out
 
 
+def dump_outputs(path, r, extra=None):
+    """Writes what one step of the timed path returned (the AnalysisResult of TraceAnalyzer.run) as float64 .npy files,
+    float32 for the filtered trace, so that two builds can be compared output for output.  The filtered trace is sampled
+    in DUMP_WINDOWS contiguous windows and the event rows in DUMP_EVENTS rows, both at positions fixed by DUMP_SEED;
+    `*_index` files say which.  level_mean / level_std hold each sampled event's first level_count entries, event after
+    event: the table's entries beyond an event's level count are never written by the kernel."""
+    import torch
+    f64 = lambda t: t.cpu().numpy().astype(np.float64)
+    out = {}
+    y = r.filtered
+    n = y.numel()
+    if n <= DUMP_WINDOWS * DUMP_WINDOW:
+        starts, w = np.zeros(1, np.int64), n
+    else:
+        stride = n // DUMP_WINDOWS
+        rng = np.random.default_rng(DUMP_SEED)
+        starts = np.arange(DUMP_WINDOWS, dtype=np.int64) * stride + rng.integers(0, stride - DUMP_WINDOW + 1, DUMP_WINDOWS)
+        w = DUMP_WINDOW
+    idx = torch.from_numpy(starts).to(y.device)[:, None] + torch.arange(w, device=y.device)
+    out["filtered"] = y[idx].cpu().numpy()
+    out["filtered_index"] = starts.astype(np.float64)
+    n_ev = r.events.starts.numel()
+    rows = np.arange(n_ev)
+    if n_ev > DUMP_EVENTS:
+        rows = np.sort(np.random.default_rng(DUMP_SEED).choice(n_ev, DUMP_EVENTS, replace=False))
+    sel = torch.from_numpy(rows).to(y.device)
+    out["event_index"] = rows.astype(np.float64)
+    out["event_start"], out["event_end"] = f64(r.events.starts[sel]), f64(r.events.ends[sel])
+    out["window_start"], out["window_end"], out["event_type"] = f64(r.win_start[sel]), f64(r.win_end[sel]), f64(r.types[sel])
+    if r.levels is not None:
+        lv = r.levels
+        nl = f64(lv.n_levels[sel])
+        fit = np.arange(lv.max_levels)[None, :] < nl[:, None]
+        out["level_count"], out["level_edges"], out["level_overflow"] = nl, f64(lv.edges[sel]), f64(lv.overflow[sel])
+        out["level_mean"], out["level_std"] = f64(lv.mean[sel])[fit], f64(lv.std[sel])[fit]
+    bl = r.baseline
+    for k in ("mean", "std", "sign", "t_start", "t_end"):
+        out["baseline_" + k] = np.asarray(getattr(bl, k), dtype=np.float64)
+    out["pad_value"] = np.array([r.pad_value])
+    out["median_codes"] = np.array(r.median_codes, dtype=np.float64)
+    out["event_count"] = np.array([n_ev, r.events.open_start, r.first_event_id, r.total_events], dtype=np.float64)
+    out.update(extra or {})
+    size = sum(a.nbytes for a in out.values())
+    if size > DUMP_BUDGET:
+        raise SystemExit(f"--dump-outputs: {size} bytes exceed the {DUMP_BUDGET}-byte budget")
+    os.makedirs(path, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------- ours
 def run_ours(args):
     import torch
@@ -391,7 +444,7 @@ def run_ours(args):
                 "n_levels": r.levels.n_levels, "edges": r.levels.edges, "mean": r.levels.mean, "std": r.levels.std}
         g = pipeline.gather_tables(cols, group, dst=0)
         hook("gather")
-        last.update(psd_segments=nseg, gathered=None if g is None else int(g["starts"].shape[0]))
+        last.update(psd_segments=nseg, psd_sums=acc, gathered=None if g is None else int(g["starts"].shape[0]))
         return acc, g
 
     def step(hook=None):
@@ -452,6 +505,10 @@ def run_ours(args):
         torch.cuda.profiler.stop()
     tm1 = time.time()
     launches = _lib.launch_count()
+    if args.dump_outputs:
+        # before anything else runs the analyzer: `res` is a view of its buffers
+        extra = {"psd_sums": np.asarray(last["psd_sums"], dtype=np.float64)} if c5 else None
+        dump_outputs(os.path.join(args.dump_outputs, f"rank{rank}") if rank else args.dump_outputs, res, extra)
     for _ in range(2):
         staged_step()
     res = step()
@@ -667,7 +724,14 @@ def main():
                     help="reader threads of the from-file leg (default: the host cores, at most 16: 17.4 against 15.8 Gsamples/s with 8)")
     ap.add_argument("--profile-range", action="store_true",
                     help="bracket the timed region with cudaProfilerStart/Stop (ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (sampled to at most 64 MB; rank r > 0 "
+                         "of a multi-GPU run under DIR/rank<r>)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

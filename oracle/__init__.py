@@ -11,7 +11,7 @@ Pinning status (see DESIGN.md "Oracle"):
     SpectrumSample) restate reference call sequences whose arithmetic lives in numpy/scipy
     (unpinned third-party: scipy 1.18.1 / numpy 2.3.5 in this image).  The reference ships
     no tests or golden vectors, so the restatement is pinned against OUTPUTS OF THE
-    REFERENCE ITSELF: `oracle/reference_shim.py` imports /root/reference/plot-trace.py and
+    REFERENCE ITSELF: `oracle/reference_shim.py` imports the reference's plot-trace.py and
     noise-fit.py headlessly and `tests/golden/make_golden.py` commits input/output vectors.
   * stages 2 and 3 (threshold detection, CUSUM+) have NO implementation in the reference
     (it only consumes their output).  `oracle/events_oracle.py` is the NumPy definition of

@@ -4,7 +4,7 @@ Every function follows a reference call sequence line by line; the arithmetic it
 in numpy/scipy exactly as in the reference (third-party, unpinned: numpy 2.3.5 /
 scipy 1.18.1 here).  Pinned against the reference's own code by
 tests/test_oracle_pins.py (golden vectors in tests/golden/ + live comparison through
-oracle/reference_shim.py whenever /root/reference is present).
+oracle/reference_shim.py whenever CUSUMTOOLS_REFERENCE names a cusumtools checkout).
 """
 from __future__ import annotations
 

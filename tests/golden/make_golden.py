@@ -1,8 +1,6 @@
 """Generates tests/golden/*.npz by running the REFERENCE'S OWN code headlessly
-(/root/reference/plot-trace.py and noise-fit.py through oracle/reference_shim.py).
-
-Run in the build container only (the GPU box has no /root/reference):
-    python tests/golden/make_golden.py
+(plot-trace.py and noise-fit.py of a cusumtools checkout, through oracle/reference_shim.py):
+    CUSUMTOOLS_REFERENCE=<cusumtools checkout> python tests/golden/make_golden.py
 The fixtures pin oracle/trace_oracle.py (and, through it, the CUDA path) to outputs of the
 reference itself; the reference ships no tests or golden vectors of its own.
 Library versions used are recorded inside the fixture.
@@ -23,6 +21,16 @@ from cusumtools_b200 import synth  # noqa: E402
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
+def savez_lzma(path, **arrays):
+    """np.savez with LZMA members (np.load reads them as it reads any .npz): noisy float64 traces deflate poorly,
+    and a fixture stays under 1 MB."""
+    import zipfile
+    with zipfile.ZipFile(path, "w", zipfile.ZIP_LZMA) as z:
+        for k, v in arrays.items():
+            with z.open(k + ".npy", "w", force_zip64=True) as f:
+                np.lib.format.write_array(f, np.asanyarray(v), allow_pickle=False)
+
+
 def edge_fixture():
     """fixture 5: the odd-extension boundary mode of legacy/bessel-filter.py:124-131 on the tool's own 26-sample
     step (generate_step) and on a 3 000-sample noisy step, orders 2 / 4 / 8."""
@@ -39,7 +47,7 @@ def edge_fixture():
 
 
 def main():
-    assert ref.available(), "reference not mounted"
+    assert ref.available(), "set CUSUMTOOLS_REFERENCE to a cusumtools checkout"
     if "--only-edge" in sys.argv:
         edge_fixture()
         return
@@ -64,7 +72,7 @@ def main():
         out[f"filt_{cutoff}_{order}"] = ref.ref_filter_data(data, fs, cutoff, order)
     # even-length variant (median = mean of the two middle values)
     out["filt_even_100000_8"] = ref.ref_filter_data(data[:-1], fs, 100000, 8)
-    np.savez_compressed(os.path.join(HERE, "filter_fixture.npz"), **out)
+    savez_lzma(os.path.join(HERE, "filter_fixture.npz"), **out)
 
     # ---- fixture 2: integrate_noise and the welch call as update_psd issues it
     from scipy.signal import welch

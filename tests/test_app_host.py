@@ -120,11 +120,12 @@ def test_fit_helpers_match_the_reference_formulas():
 
 
 def test_overlay_cusum_agrees_with_the_live_reference(tmp_path):
-    """plot-trace.py:172-203 run headlessly on the same analysis directory (when /root/reference is mounted)."""
+    """plot-trace.py:172-203 run headlessly on the same analysis directory (when CUSUMTOOLS_REFERENCE names a
+    cusumtools checkout)."""
     from types import SimpleNamespace
     from oracle import reference_shim as ref
     if not ref.available():
-        pytest.skip("reference not mounted (GPU box)")
+        pytest.skip("CUSUMTOOLS_REFERENCE does not name a cusumtools checkout")
     pt = ref.load("plot-trace.py")
     d = str(tmp_path / "an")
     make_analysis_dir(d)
