@@ -83,7 +83,11 @@ SIGNATURES = {
     "ct_intra_crossings_f32": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _i64, _vp, _i64, _i64, _vp, _vp, _vp, C.c_int32, _vp, _vp, _vp]),
     "ct_cusum_batch_dev": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _i64, _f32, _f32, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
     "ct_cusum_batch": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _i64, _f32, _f32, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
+    "ct_stepfit_select": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp]),
+    "ct_stepfit_batch": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _i64, _i64, _f32, C.c_int, C.c_int, _vp, _vp, _vp, _vp, _vp,
+                                   _vp, _vp, _vp]),
 }
+STEPFIT_MAX_WINDOW = 8192     # CT_STEPFIT_MAX_WINDOW
 
 _lib = None
 

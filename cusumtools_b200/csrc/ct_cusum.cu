@@ -720,7 +720,8 @@ __global__ void __launch_bounds__(256) ct_event_extrema_kernel(const float* __re
 //   cols[e][0..10] = baseline before, baseline after, effective baseline, sub-level duration (samples),
 //                    average blockage, max blockage, its level's length (samples), min blockage, its level's
 //                    length, residual (rms of trace minus step fit), max deviation from the effective baseline
-// and the event's final type (0 accepted, 5 CUSUM+ found no sub-level, 6 level overflow; other codes pass through).
+// and the event's final type (0 accepted, 1 step-response fit, 5 CUSUM+ found no sub-level, 6 level overflow; other
+// codes pass through).
 // Conventions: cusumtools_b200/writer.py (blockage = sign(baseline) (baseline - level); in-event statistics run over
 // the sub-levels 1 .. L-2; ties keep the first level).  Sums run level by level in index order.
 constexpr int kEventCols = 12;
@@ -734,11 +735,12 @@ __global__ void ct_event_columns_kernel(const int* __restrict__ n_levels, const 
     for (long long ev = (long long)blockIdx.x * blockDim.x + threadIdx.x; ev < nev; ev += (long long)gridDim.x * blockDim.x) {
         const int L = n_levels[ev];
         int t = type ? type[ev] : 0;
-        if (t == 0 && overflow[ev]) t = 6;
-        if (t == 0 && L < 3) t = 5;
+        // type 1 (step-response fit, level rows from ct_stepfit_batch) goes through the same arithmetic as type 0
+        if ((t == 0 || t == 1) && overflow[ev]) t = 6;
+        if ((t == 0 || t == 1) && L < 3) t = 5;
         type_out[ev] = t;
         double* c = cols + ev * kEventCols;
-        if (t != 0) {
+        if (t != 0 && t != 1) {
 #pragma unroll
             for (int i = 0; i < kEventCols; ++i) c[i] = 0.0;
             continue;

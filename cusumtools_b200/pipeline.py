@@ -19,7 +19,7 @@ from dataclasses import dataclass
 import numpy as np
 import torch
 
-from . import _lib, cusum, detect, filters
+from . import _lib, cusum, detect, filters, stepfit
 from .design import bessel_lowpass
 
 
@@ -249,6 +249,7 @@ class AnalysisResult:
     first_event_id: int = 0
     total_events: int = 0
     intra: "tuple[torch.Tensor, torch.Tensor] | None" = None     # (count int32 [E], pairs int32 [E, 2K]) crossings
+    stepfit: "stepfit.StepFitTable | None" = None                # step-response fit of the short events (type 1 / 7)
 
 
 class TraceAnalyzer:
@@ -270,7 +271,7 @@ class TraceAnalyzer:
                  cusum_h: float | None = None, max_levels: int = cusum.DEFAULT_MAX_LEVELS,
                  event_capacity: int | None = None, group=None, device="cuda", fuse_stats: bool = True,
                  fused_count: bool = True, intra_threshold: float = 0.0, intra_hysteresis: float = 0.0,
-                 max_crossings: int = 8, halos_clipped_by_trace_ends: bool = False):
+                 max_crossings: int = 8, halos_clipped_by_trace_ends: bool = False, stepfit_samples: int = 0):
         self.n_ext, self.lo_halo, self.hi_halo = int(n_ext), int(lo_halo), int(hi_halo)
         self.n_own = self.n_ext - self.lo_halo - self.hi_halo
         self.n_det = self.n_ext
@@ -292,6 +293,15 @@ class TraceAnalyzer:
         # intra-event threshold crossings (readevents.py:1340-1343, 1363-1367); 0 = off, as in summary.txt
         self.intra_threshold, self.intra_hysteresis = float(intra_threshold), float(intra_hysteresis)
         self.max_crossings = int(max_crossings)
+        # step-response fit of the accepted events shorter than `stepfit_samples` (type 1, stepfit.py); 0 = off
+        self.stepfit_samples = int(stepfit_samples)
+        if self.stepfit_samples < 0:
+            raise ValueError("stepfit_samples must be >= 0")
+        if self.stepfit_samples and self.stepfit_samples + 2 * self.event_padding > stepfit.MAX_WINDOW:
+            raise ValueError(f"stepfit_samples + 2 * event_padding = {self.stepfit_samples + 2 * self.event_padding} exceeds "
+                             f"the {stepfit.MAX_WINDOW}-sample window of the step-response fit")
+        self.tau0 = (stepfit.zero_phase_rise_tau(float(np.floor(np.squeeze(settings["ADCSAMPLERATE"]))), cutoff, order)
+                     if self.stepfit_samples else 0.0)
         self.group = group
         self.device = torch.device(device)
         self.mask = filters.chimera_bitmask(settings)
@@ -324,12 +334,17 @@ class TraceAnalyzer:
         if self.intra_threshold > 0:
             self.ic = torch.zeros(cap, dtype=torch.int32, device=dev)
             self.ip = torch.full((cap, 2 * self.max_crossings), -1, dtype=torch.int32, device=dev)
-        if self.delta is not None:
+        if self.delta is not None or self.stepfit_samples:
             self.nl = torch.empty(cap, dtype=torch.int32, device=dev)
             self.ed = torch.empty((cap, ML + 1), dtype=torch.int32, device=dev)
             self.mu = torch.empty((cap, ML), dtype=torch.float64, device=dev)
             self.sd = torch.empty((cap, ML), dtype=torch.float64, device=dev)
             self.ov = torch.empty(cap, dtype=torch.uint8, device=dev)
+        if self.stepfit_samples:
+            self.sf = {"params": torch.empty((cap, 6), dtype=torch.float64, device=dev),
+                       "cost": torch.empty(cap, dtype=torch.float64, device=dev),
+                       "iters": torch.empty(cap, dtype=torch.int32, device=dev)}
+        if self.delta is not None:
             self.cws_bytes = int(_lib.lib().ct_cusum_workspace_bytes(cap))
             self.cws = torch.empty((self.cws_bytes + 7) // 8, dtype=torch.int64, device=dev)
 
@@ -488,6 +503,9 @@ class TraceAnalyzer:
                                     self.w1.data_ptr(), self.typ.data_ptr(), sc[2:].data_ptr(), st)
             _lib.check(rc, "ct_event_windows")
             hook("detect")
+            if self.stepfit_samples:             # before CUSUM+, which then skips the short events
+                stepfit.select_short(self.w0, self.w1, self.typ, padding=self.event_padding,
+                                     stepfit_samples=self.stepfit_samples, n_events_dev=sc[2:])
             if self.delta is not None:
                 rc = L.ct_cusum_batch_dev(yd.data_ptr(), self.n_det, self.w0.data_ptr(), self.w1.data_ptr(),
                                           self.typ.data_ptr(), sc[2:].data_ptr(), self.cap, float(self.delta),
@@ -495,6 +513,12 @@ class TraceAnalyzer:
                                           self.mu.data_ptr(), self.sd.data_ptr(), self.ov.data_ptr(), self.cws.data_ptr(),
                                           self.cws_bytes, st)
                 _lib.check(rc, "ct_cusum_batch_dev")
+            elif self.stepfit_samples:           # no CUSUM+: the rows of the events the fit does not take stay empty
+                self.nl.zero_(); self.ov.zero_(); self.ed.fill_(-1)
+            if self.stepfit_samples:             # after CUSUM+, which writes n_levels = 0 for every event not of type 0
+                stepfit.launch(yd, self.w0, self.w1, self.typ, self.sf,
+                               {"n_levels": self.nl, "edges": self.ed, "mean": self.mu, "std": self.sd},
+                               padding=self.event_padding, tau0=self.tau0, n_events_dev=sc[2:], capacity=self.cap)
             if self.intra_threshold > 0:
                 # the block of the event start: win_start + padding (windows are compacted, the start list is not)
                 detect.intra_crossings(yd, self.w0, self.w1, self.w0 + self.event_padding, bl, self.intra_threshold,
@@ -529,13 +553,15 @@ class TraceAnalyzer:
             open_start = o if 0 <= o < n_own else -1
         # event indices are reported relative to the first owned sample
         ev = detect.EventList(self.starts[i0:i0 + nk] - lo, self.ends[i0:i0 + nk] - lo, open_start)
-        lv = None
-        if self.delta is not None:
+        lv = sf = None
+        if self.delta is not None or self.stepfit_samples:
             lv = cusum.LevelTable(self.nl[:nk], self.ed[:nk], self.mu[:nk], self.sd[:nk], self.ov[:nk], self.max_levels)
+        if self.stepfit_samples:
+            sf = stepfit.StepFitTable(self.sf["params"][:nk], self.sf["cost"][:nk], self.sf["iters"][:nk], self.typ[:nk])
         return AnalysisResult(filtered=y[lo:lo + n_own], detect_trace=yd, lo_halo=lo, baseline=bl, events=ev,
                               win_start=self.w0[:nk], win_end=self.w1[:nk], types=self.typ[:nk], levels=lv,
                               pad_value=pad_value, median_codes=(c1, c2), first_event_id=first_id, total_events=total,
-                              intra=(self.ic[:nk], self.ip[:nk]) if self.intra_threshold > 0 else None)
+                              intra=(self.ic[:nk], self.ip[:nk]) if self.intra_threshold > 0 else None, stepfit=sf)
 
 
     def tables_to_host(self, r: AnalysisResult) -> dict:
@@ -552,6 +578,8 @@ class TraceAnalyzer:
                        overflow=r.levels.overflow)
         if r.intra is not None:
             src.update(intra_count=r.intra[0], intra_pairs=r.intra[1])
+        if r.stepfit is not None:
+            src.update(stepfit_params=r.stepfit.params, stepfit_cost=r.stepfit.cost, stepfit_iters=r.stepfit.iters)
         out = {}
         for k, t in src.items():
             if k not in self._pinned:
@@ -569,7 +597,8 @@ class StreamResult:
     table on the device, the event / level tables already in (pinned) host memory."""
     filtered: torch.Tensor          # float32 CUDA, the rank's owned samples
     baseline: detect.Baseline       # blocks of the owned range
-    tables: dict                    # numpy: starts, ends (relative to the first owned sample), types[, n_levels, edges, mean, std, overflow]
+    tables: dict                    # numpy: starts, ends (relative to the first owned sample), types[, n_levels, edges, mean, std,
+                                    # overflow][, stepfit_params, stepfit_cost, stepfit_iters]
     pad_value: float
     median_codes: tuple[int, int]
     first_event_id: int = 0
@@ -697,7 +726,7 @@ class StreamingAnalyzer:
         self.padding = int(kw.get("padding", 1000))
         self.mask = filters.chimera_bitmask(settings)
         self.max_levels = int(kw.get("max_levels", cusum.DEFAULT_MAX_LEVELS))
-        self.with_levels = kw.get("cusum_delta") is not None
+        self.with_levels = kw.get("cusum_delta") is not None or bool(kw.get("stepfit_samples"))
         fs = float(np.floor(np.squeeze(settings["ADCSAMPLERATE"])))
         max_event = int(kw.get("maxpoints", 100_000)) + 2 * int(kw.get("event_padding", 100))
         self.h = required_halo(self.cutoff, self.order, fs, max_event, self.padding, block=self.block)
@@ -760,6 +789,8 @@ class StreamingAnalyzer:
                         overflow=r.levels.overflow)
         if r.intra is not None:
             cols.update(intra_count=r.intra[0], intra_pairs=r.intra[1])
+        if r.stepfit is not None:
+            cols.update(stepfit_params=r.stepfit.params, stepfit_cost=r.stepfit.cost, stepfit_iters=r.stepfit.iters)
         if end_at is not None:
             if nk > end_at:
                 return -1

@@ -64,11 +64,14 @@ def c1_trace(n: int = 4166666, n_events: int = 1000, seed: int = 0, settings=CHI
 
 
 def device_trace(n: int, device, seed: int = 1234, events_per_s: float = 1000.0, jitter: int = 500,
-                 settings=CHIMERA_SETTINGS, chunk: int = 1 << 26, start_index: int = 0):
+                 settings=CHIMERA_SETTINGS, chunk: int = 1 << 26, start_index: int = 0, levels=None):
     """Configs C2/C5: the same signal model generated on the GPU in chunks (Philox),
     events every fs/events_per_s samples with uniform +-jitter on the start.  Returns a
     uint16 CUDA tensor.  `start_index` is the global index of sample 0 (time sharding):
-    the event grid is global, the noise stream is per shard (seed)."""
+    the event grid is global, the noise stream is per shard (seed).  `levels`: the event
+    template as ((depth pA, samples), ...), default EVENT_LEVELS (e.g. ((-1000.0, 100),) for
+    short single-level pulses)."""
+    levels = EVENT_LEVELS if levels is None else tuple((float(d), int(l)) for d, l in levels)
     import torch
     g = torch.Generator(device=device)
     g.manual_seed(seed)
@@ -77,7 +80,7 @@ def device_trace(n: int, device, seed: int = 1234, events_per_s: float = 1000.0,
     step = 1 << (16 - bits)
     period = int(round(FS / events_per_s))
     out = torch.empty(n, dtype=torch.uint16, device=device)
-    tot = sum(l for _, l in EVENT_LEVELS)
+    tot = sum(l for _, l in levels)
     jg = torch.Generator(device="cpu")
     jg.manual_seed(seed + 7919)
     for c0 in range(0, n, chunk):
@@ -93,7 +96,7 @@ def device_trace(n: int, device, seed: int = 1234, events_per_s: float = 1000.0,
             st = 1500 + kk * period + jit
             rel = gidx - st
             o = 0
-            for depth, length in EVENT_LEVELS:
+            for depth, length in levels:
                 cur += depth * ((rel >= o) & (rel < o + length) & (kk >= 0))
                 o += length
         code = torch.round((cur - beta) / alpha / step) * step
@@ -160,3 +163,50 @@ def c3_events_device(n_events: int, device, seed: int = 2024, min_len: int = 500
         x[a:b] = seg + d * inside
         del ev, r, L, inside, lvl, d, seg
     return x, offsets, nlev
+
+
+SHORT_PAD = 100              # baseline samples either side of a short event's window
+SHORT_GUARD = 400            # extra baseline between the windows of neighbouring events before filtering
+
+
+def short_events_device(n_events: int, device, seed: int = 77, min_len: int = 20, max_len: int = 400, pad: int = SHORT_PAD,
+                        min_depth: float = 300.0, max_depth: float = 2000.0, noise: float = NOISE_PA,
+                        cutoff: float = 1e5, order: int = 8, chunk_events: int = 200_000):
+    """Short events for the step-response fit: rectangular pulses of log-uniform length in [min_len, max_len]
+    samples and blockage depth uniform in [min_depth, max_depth] pA on a baseline of +-5000 pA (the sign drawn per
+    event; the pulse moves the current toward zero), sigma = `noise` pA raw white noise, filtered with the
+    project's own zero-phase Bessel (ct_filtfilt_f32) at `cutoff` / `order` and FS.  Every event is filtered
+    inside a continuous stretch of baseline (its window plus SHORT_GUARD samples each side), then its window of
+    `pad` + length + `pad` samples is cut out.  Returns (samples float32 [sum of windows], offsets int64 [E+1],
+    lengths int64 [E], depths float64 [E] signed like the baseline) as CUDA tensors."""
+    import torch
+    from .filters import bessel_filtfilt
+    g = torch.Generator(device=device)
+    g.manual_seed(seed)
+    u = torch.rand(n_events, generator=g, device=device, dtype=torch.float64)
+    lens = torch.exp(u * (np.log(max_len) - np.log(min_len)) + np.log(min_len)).to(torch.int64)
+    depth = min_depth + (max_depth - min_depth) * torch.rand(n_events, generator=g, device=device, dtype=torch.float64)
+    sgn = torch.where(torch.rand(n_events, generator=g, device=device) < 0.5, -1.0, 1.0).to(torch.float64)
+    win = lens + 2 * pad
+    offsets = torch.zeros(n_events + 1, dtype=torch.int64, device=device)
+    offsets[1:] = torch.cumsum(win, 0)
+    out = torch.empty(int(offsets[-1].item()), dtype=torch.float32, device=device)
+    for e0 in range(0, n_events, chunk_events):
+        e1 = min(n_events, e0 + chunk_events)
+        seg = win[e0:e1] + 2 * SHORT_GUARD
+        soff = torch.zeros(e1 - e0 + 1, dtype=torch.int64, device=device)
+        soff[1:] = torch.cumsum(seg, 0)
+        m = int(soff[-1].item())
+        ev = torch.repeat_interleave(torch.arange(e1 - e0, device=device), seg)
+        r = torch.arange(m, device=device) - soff[ev] - SHORT_GUARD - pad          # index relative to the event start
+        inside = (r >= 0) & (r < lens[e0 + ev])
+        # the trace of a positive baseline; the event's own sign is applied to its window afterwards (the filter is
+        # linear with DC gain 1, and the guards keep the neighbours' pulses out of the window)
+        z = torch.randn(m, generator=g, device=device, dtype=torch.float32) * noise - depth[e0 + ev].to(torch.float32) * inside
+        y = bessel_filtfilt(z.contiguous(), FS, cutoff, order, pad_value=0.0)
+        keep = (r >= -pad) & (r < lens[e0 + ev] + pad)
+        w = y[keep].to(torch.float64) + BASELINE_PA
+        ek = ev[keep]
+        out[int(offsets[e0].item()):int(offsets[e1].item())] = (w * sgn[e0 + ek]).to(torch.float32)
+        del ev, r, inside, z, y, keep, w, ek
+    return out, offsets, lens, depth * sgn

@@ -17,13 +17,18 @@ fixed here (SURVEY.md Appendix A.4 lists the open points):
   the first to the last changepoint; `area_pC` = average blockage (pA) x that duration (s);
 * `residual_pA` = rms of trace minus step fit over the whole window = sqrt(sum len*std^2 / sum len);
 * `max_deviation_pA` = largest |sample - effective baseline| in the window;
-* `type`: 0 accepted (CUSUM fit; 3-column event file), 2 too short, 3 too long, 4 padding
+* `type`: 0 accepted (CUSUM fit; 3-column event file), 1 step-response fit (4-column event file
+  `time_us,current_pA,cusum_fit,stepfit`, readevents.py:1334-1337), 2 too short, 3 too long, 4 padding
   overlaps a neighbour or leaves the trace, 5 CUSUM+ found no sub-level, 6 more levels than
-  the table holds; types > 1 appear in rate.csv only (`plot-trace.py:354-357`);
+  the table holds, 7 step fit failed; types > 1 appear in rate.csv only (`plot-trace.py:354-357`);
+* a type-1 event has three level rows from its fit p = (i0, a, u1, u2, tau1, tau2) (stepfit.py):
+  edges [0, ceil u1, ceil u2, n], means [i0, i0 - a, i0], std = rms of trace minus fitted step response
+  over each; the derived columns follow from them as for a CUSUM fit.  `rc_const1_us` / `rc_const2_us`
+  are tau1 / tau2 in us (0 for type 0);
 * intra-event threshold crossings (`intra_crossings`, rate.csv `intra_crossing_times_us`) are
   produced when the analyzer is given `intra_threshold` > 0 (detect.intra_crossings; the lines the
   consumer draws at readevents.py:1363-1366); at most `max_crossings` pairs are listed per event,
-  the count is complete.  No step-response fit: `rc_const1_us` = `rc_const2_us` = 0.
+  the count is complete.
 
 The derived per-event statistics (baselines, blockages, area, residual, max deviation, final type) are computed on
 the device, one thread per event from the level table (ct_event_columns, after ct_event_extrema_f32); this module
@@ -49,7 +54,8 @@ EVENT_COLUMNS = ["id", "type", "start_time_s", "event_delay_s", "duration_us", "
                  "min_blockage_pA", "relative_min_blockage", "min_blockage_duration_us", "level_current_pA",
                  "level_duration_us", "blockages_pA", "stdev_pA"]
 RATE_COLUMNS = ["id", "type", "start_time_s", "end_time_s", "intra_crossing_times_us", "local_stdev", "local_baseline"]
-TYPE_NO_SUBLEVEL, TYPE_LEVEL_OVERFLOW = 5, 6
+TYPE_STEPFIT, TYPE_NO_SUBLEVEL, TYPE_LEVEL_OVERFLOW, TYPE_STEPFIT_FAILED = 1, 5, 6, 7
+GOOD_TYPES = (0, TYPE_STEPFIT)     # the types plot-trace.py:354-357 counts as good events (events.csv rows)
 
 
 def event_extrema(y: torch.Tensor, win_start: torch.Tensor, win_end: torch.Tensor):
@@ -94,10 +100,10 @@ def event_columns_host(types, n_levels, edges, level_mean, level_std, overflow, 
     mu = np.asarray(level_mean, np.float64).reshape(E, -1)
     sd = np.asarray(level_std, np.float64).reshape(E, -1)
     ML = mu.shape[1] if E else 0
-    types[(types == 0) & (np.asarray(overflow) != 0)] = TYPE_LEVEL_OVERFLOW
-    types[(types == 0) & (nl < 3)] = TYPE_NO_SUBLEVEL
+    types[np.isin(types, GOOD_TYPES) & (np.asarray(overflow) != 0)] = TYPE_LEVEL_OVERFLOW
+    types[np.isin(types, GOOD_TYPES) & (nl < 3)] = TYPE_NO_SUBLEVEL
     cols = np.zeros((E, 12))
-    ok = types == 0
+    ok = np.isin(types, GOOD_TYPES)
     rows = np.nonzero(ok)[0]
     if rows.size:
         L = nl[rows]
@@ -161,7 +167,7 @@ class RaggedColumn:
 @dataclass
 class EventTable:
     """Column-oriented event table (numpy).  `rate` holds every detected event, `events`
-    the accepted ones (type 0) with the full column set; list columns are object arrays of
+    the accepted ones (types 0 and 1) with the full column set; list columns are object arrays of
     float64 vectors until they are serialised."""
     events: dict
     rate: dict
@@ -177,10 +183,12 @@ def _fmt_list(v) -> str:
 def build_event_table(*, starts, ends, types, n_levels, edges, level_mean, level_std, overflow, xmin, xmax,
                       samplerate: float, threshold: float, baseline_mean, baseline_std, baseline_block: int,
                       padding: int, first_id: int = 0, time_offset_s: float = 0.0, index_offset: int = 0,
-                      block_offset: int = 0, intra_count=None, intra_pairs=None, columns=None) -> EventTable:
-    """Per-event columns from the detector / CUSUM+ tables (numpy arrays, one row per detected
+                      block_offset: int = 0, intra_count=None, intra_pairs=None, columns=None,
+                      stepfit_params=None) -> EventTable:
+    """Per-event columns from the detector / CUSUM+ / step-fit tables (numpy arrays, one row per detected
     event).  `index_offset` is the global sample index of the shard's first owned sample,
-    `first_id` the global id of its first event (multi-GPU: pipeline.AnalysisResult)."""
+    `first_id` the global id of its first event (multi-GPU: pipeline.AnalysisResult).
+    `stepfit_params` [E, 6] (stepfit.StepFitTable.params) gives the rc columns of type-1 rows."""
     starts = np.asarray(starts, np.int64); ends = np.asarray(ends, np.int64)
     E = starts.size
     types = np.asarray(types, np.int32).copy()
@@ -212,8 +220,14 @@ def build_event_table(*, starts, ends, types, n_levels, edges, level_mean, level
             "local_stdev": np.asarray(baseline_std, np.float64)[blk] if E else np.zeros(0),
             "local_baseline": np.asarray(baseline_mean, np.float64)[blk] if E else np.zeros(0)}
 
-    ok = np.nonzero(types == 0)[0]
+    ok = np.nonzero(np.isin(types, GOOD_TYPES))[0]
     n = ok.size
+    rc1, rc2 = np.zeros(n), np.zeros(n)
+    if stepfit_params is not None and n:
+        sp = np.asarray(stepfit_params, np.float64).reshape(E, 6)[ok]
+        fitted = types[ok] == TYPE_STEPFIT
+        rc1 = np.where(fitted, sp[:, 4] * (1e6 / fs), 0.0)
+        rc2 = np.where(fitted, sp[:, 5] * (1e6 / fs), 0.0)
     L = nl[ok]
     col = np.arange(ML)[None, :]
     valid = col < L[:, None]                       # levels of the window
@@ -238,14 +252,14 @@ def build_event_table(*, starts, ends, types, n_levels, edges, level_mean, level
         if n:
             delay[0] = ts[0]
             delay[1:] = ts[1:] - ts[:-1]                                   # mosaicConverter.py:73-76
-        events = {"id": ids[ok], "type": np.zeros(n, np.int64), "start_time_s": ts, "event_delay_s": delay,
+        events = {"id": ids[ok], "type": types[ok].astype(np.int64), "start_time_s": ts, "event_delay_s": delay,
                   "duration_us": (ends[ok] - starts[ok]) * us, "threshold": np.full(n, float(threshold)),
                   "baseline_before_pA": before, "baseline_after_pA": after, "effective_baseline_pA": eff,
                   "area_pC": avg_block * dur_in / fs, "average_blockage_pA": avg_block,
                   "relative_average_blockage": avg_block / aeff, "max_blockage_pA": c[:, 5],
                   "relative_max_blockage": c[:, 5] / aeff, "max_blockage_duration_us": c[:, 6] * us,
-                  "n_levels": L - 1, "intra_crossings": ic[ok], "rc_const1_us": np.zeros(n),
-                  "rc_const2_us": np.zeros(n), "residual_pA": c[:, 9], "max_deviation_pA": c[:, 10],
+                  "n_levels": L - 1, "intra_crossings": ic[ok], "rc_const1_us": rc1,
+                  "rc_const2_us": rc2, "residual_pA": c[:, 9], "max_deviation_pA": c[:, 10],
                   "min_blockage_pA": c[:, 7], "relative_min_blockage": c[:, 7] / aeff,
                   "min_blockage_duration_us": c[:, 8] * us, **lists}
     return EventTable(events=events, rate=rate)
@@ -263,7 +277,8 @@ def event_table_from_result(an, r, *, samplerate: float, time_offset_s: float = 
                              samplerate=samplerate, threshold=an.threshold, baseline_mean=r.baseline.mean,
                              baseline_std=r.baseline.std, baseline_block=an.block, padding=an.event_padding,
                              first_id=r.first_event_id, time_offset_s=time_offset_s, index_offset=index_offset,
-                             block_offset=r.lo_halo, intra_count=tabs.get("intra_count"), intra_pairs=tabs.get("intra_pairs"))
+                             block_offset=r.lo_halo, intra_count=tabs.get("intra_count"), intra_pairs=tabs.get("intra_pairs"),
+                             stepfit_params=tabs.get("stepfit_params"))
 
 
 def event_table_from_stream(san, rs, *, samplerate: float, time_offset_s: float = 0.0, index_offset: int = 0) -> EventTable:
@@ -289,7 +304,8 @@ def event_table_from_stream(san, rs, *, samplerate: float, time_offset_s: float 
                              threshold=float(san.kw.get("threshold", 5.0)), baseline_mean=rs.baseline.mean,
                              baseline_std=rs.baseline.std, baseline_block=san.block, padding=pad,
                              first_id=rs.first_event_id, time_offset_s=time_offset_s, index_offset=index_offset,
-                             intra_count=t.get("intra_count"), intra_pairs=t.get("intra_pairs"))
+                             intra_count=t.get("intra_count"), intra_pairs=t.get("intra_pairs"),
+                             stepfit_params=t.get("stepfit_params"))
 
 
 def _write_csv(path: str, columns, table: dict) -> None:
@@ -304,14 +320,17 @@ def _write_csv(path: str, columns, table: dict) -> None:
 def write_analysis_dir(path: str, table: EventTable, *, baseline_mean, baseline_std, baseline_block: int,
                        samplerate: float, threshold: float, hysteresis: float, cutoff: float, poles: int,
                        extra_summary: dict | None = None, event_samples=None, time_offset_s: float = 0.0,
-                       append: bool = False, intra_threshold: float = 0.0, intra_hysteresis: float = 0.0) -> None:
+                       append: bool = False, intra_threshold: float = 0.0, intra_hysteresis: float = 0.0,
+                       stepfit_samples: int = 0) -> None:
     """Write `events.csv`, `rate.csv`, `baseline.csv`, `summary.txt` and (if `event_samples`
     is given) `events/event_%08d.csv` under `path`.
 
     `event_samples` maps event id -> (window_start_index, samples float array, edges, level
-    means): the rows of the per-event file are `time_us, current_pA, cusum_fit`
+    means[, step-fit parameters]): the rows of the per-event file are `time_us, current_pA, cusum_fit`
     (`readevents.py:1334-1337` names them time, current, cusum) WITH a header line, because
-    the consumer reads them with an implicit header row (`readevents.py:1319`)."""
+    the consumer reads them with an implicit header row (`readevents.py:1319`).  An entry with
+    parameters (a type-1 event) gets a fourth column `stepfit`, the fitted step response f(t).
+    `stepfit_samples` > 0 (the analyzer's length threshold of the fit) is recorded in summary.txt."""
     os.makedirs(os.path.join(path, "events"), exist_ok=True)
     _write_csv(os.path.join(path, "events.csv"), EVENT_COLUMNS, table.events)
     _write_csv(os.path.join(path, "rate.csv"), RATE_COLUMNS, table.rate)
@@ -327,6 +346,8 @@ def write_analysis_dir(path: str, table: EventTable, *, baseline_mean, baseline_
                "intra_hysteresis": repr(float(intra_hysteresis)) if intra_hysteresis else "0", "samplerate": repr(fs),
                "baseline_block_samples": str(int(baseline_block)), "events_detected": str(len(table.rate["id"])),
                "events_accepted": str(len(table))}
+    if stepfit_samples:
+        summary["stepfit_samples"] = str(int(stepfit_samples))
     for k, v in (extra_summary or {}).items():
         if any(w in k for w in ("threshold", "hysteresis", "cutoff", "poles")):
             raise ValueError(f"summary key {k!r} would be mis-parsed by the consumers' substring match")
@@ -337,26 +358,40 @@ def write_analysis_dir(path: str, table: EventTable, *, baseline_mean, baseline_
             f.write(f"{k}={v}\n")
     if event_samples:
         us = 1e6 / fs
-        for eid, (w0, x, ed, mu) in event_samples.items():
+        from .stepfit import model
+        for eid, entry in event_samples.items():
+            w0, x, ed, mu = entry[:4]
+            params = entry[4] if len(entry) > 4 else None
             x = np.asarray(x, np.float64)
             fit = np.empty_like(x)
             for i in range(len(ed) - 1):
                 fit[ed[i]:ed[i + 1]] = mu[i]
             t = np.arange(x.size) * us
             with open(os.path.join(path, "events", "event_%08d.csv" % int(eid)), "w") as f:
-                f.write("time_us,current_pA,cusum_fit\n")
-                np.savetxt(f, np.c_[t, x, fit], delimiter=",", fmt="%.16g")
+                if params is None:
+                    f.write("time_us,current_pA,cusum_fit\n")
+                    np.savetxt(f, np.c_[t, x, fit], delimiter=",", fmt="%.16g")
+                else:
+                    f.write("time_us,current_pA,cusum_fit,stepfit\n")
+                    np.savetxt(f, np.c_[t, x, fit, model(params, x.size)], delimiter=",", fmt="%.16g")
 
 
 def gather_event_samples(an, r, ids, table: EventTable) -> dict:
-    """Samples + step fit of the chosen event ids (global ids) for the per-event files."""
+    """Samples + step fit of the chosen event ids (global ids) for the per-event files; type-1 events also
+    carry their step-response parameters (the `stepfit` column)."""
     tabs = {k: v for k, v in zip(("w0", "w1"), (r.win_start.cpu().numpy(), r.win_end.cpu().numpy()))}
     nl = r.levels.n_levels.cpu().numpy(); ed = r.levels.edges.cpu().numpy(); mu = r.levels.mean.cpu().numpy()
+    sf = getattr(r, "stepfit", None)
+    typ = r.types.cpu().numpy() if sf is not None else None
+    par = sf.params.cpu().numpy() if sf is not None else None
     out = {}
     for eid in ids:
         i = int(eid) - r.first_event_id
         if i < 0 or i >= len(nl) or nl[i] <= 0:
             continue
         a, b = int(tabs["w0"][i]), int(tabs["w1"][i])
-        out[int(eid)] = (a, r.detect_trace[a:b].cpu().numpy(), ed[i, :nl[i] + 1].astype(np.int64), mu[i, :nl[i]])
+        entry = (a, r.detect_trace[a:b].cpu().numpy(), ed[i, :nl[i] + 1].astype(np.int64), mu[i, :nl[i]])
+        if sf is not None and typ[i] == TYPE_STEPFIT:
+            entry = entry + (par[i].copy(),)          # u1, u2 are relative to the window start, as the samples
+        out[int(eid)] = entry
     return out

@@ -216,6 +216,30 @@ int ct_cusum_batch_dev(const float* y, int64_t n_total, const int64_t* win_start
                        int max_levels, int32_t* n_levels, int32_t* edges, double* level_mean, double* level_std,
                        uint8_t* overflow, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- stage 3b: step-response fit of short events (type 1) ---------------------------
+ * No reference implementation exists: readevents.py:1334-1337 reads a type-1 event file with the four columns
+ * time, current, cusum, stepfit, and events.csv carries rc_const1_us / rc_const2_us (writer convention:
+ * cusumtools_b200/writer.py, type 1 = step-response fit, 7 = step fit failed, rate.csv only).  Definition of record:
+ * oracle/stepfit_oracle.py.  For window sample t (window = [win_start, win_end)) and p = (i0, a, u1, u2, tau1, tau2):
+ *   f(t) = i0 - a (1 - exp(-(t-u1)/tau1)) H(t-u1) + a (1 - exp(-(t-u2)/tau2)) H(t-u2),   H(s) = [s >= 0].
+ * ct_stepfit_select turns the accepted events (type 0) shorter than `stepfit_samples` (event length =
+ * win_end - win_start - 2 padding) into type 1; it must run BEFORE ct_cusum_batch_dev, so that CUSUM+ skips them.
+ * n_events_dev may be NULL (all `capacity` rows).                                                                 */
+#define CT_STEPFIT_MAX_WINDOW 8192                /* longest window ct_stepfit_batch fits (longer: type 7) */
+int ct_stepfit_select(const int64_t* win_start, const int64_t* win_end, int32_t* type, const int64_t* n_events_dev,
+                      int64_t capacity, int64_t padding, int64_t stepfit_samples, void* stream);
+/* Levenberg-Marquardt fit of every type-1 event from the initial guess i0 = mean of the first and last `padding`
+ * samples, a = i0 - mean of the rest, u1 = padding, u2 = n - padding, tau1 = tau2 = tau0 (samples), at most
+ * `max_iters` model evaluations.  A valid fit writes its level rows (n_levels = 3, edges = {0, ceil u1, ceil u2, n},
+ * mean = {i0, i0 - a, i0}, std = rms of the residual over each level); an invalid one sets type 7 and n_levels = 0.
+ * params6 [capacity][6] (i0 and a in pA, the rest in samples), cost (sum of squared residuals, pA^2) and iters
+ * (evaluations) are written for every row below the count, zero for events that are not type 1.  It must run AFTER
+ * ct_cusum_batch_dev, which writes n_levels = 0 for every event whose type is not 0.                               */
+int ct_stepfit_batch(const float* y, int64_t n_total, const int64_t* win_start, const int64_t* win_end, int32_t* type,
+                     const int64_t* n_events_dev, int64_t capacity, int64_t padding, float tau0, int max_iters, int max_levels,
+                     double* params6, double* cost, int32_t* iters, int32_t* n_levels, int32_t* edges, double* level_mean,
+                     double* level_std, void* stream);
+
 /* Intra-event threshold crossings (rate.csv intra_crossing_times_us / events.csv intra_crossings;
  * consumer: readevents.py:1340-1343,1363-1367, summary.txt keys intra_threshold / intra_hysteresis
  * readevents.py:73-79).  The detector's automaton over each event window with the lines
@@ -238,8 +262,8 @@ int ct_event_extrema_f32(const float* y, int64_t n_total, const int64_t* win_sta
  *   cols12[e] = { baseline_before, baseline_after, effective_baseline, sub-level duration (samples), average_blockage,
  *                 max_blockage, length of its level (samples), min_blockage, length of its level, residual,
  *                 max_deviation, 0 }                                (pA; conventions: cusumtools_b200/writer.py)
- *   type_out[e] = type[e], or 5 (accepted but CUSUM+ found no sub-level) / 6 (level overflow); rows of events with
- *   type_out != 0 are zero.  xmin / xmax: ct_event_extrema_f32.  type and n_events_dev may be NULL.                */
+ *   type_out[e] = type[e], or 5 (accepted but CUSUM+ found no sub-level) / 6 (level overflow); type 1 (step-response
+ *   fit, level rows from ct_stepfit_batch) is treated as type 0; rows of events with type_out > 1 are zero.  xmin / xmax: ct_event_extrema_f32.  type and n_events_dev may be NULL.                */
 int ct_event_columns(const int32_t* n_levels, const int32_t* edges, const double* level_mean, const double* level_std,
                      const int32_t* type, const uint8_t* overflow, const float* xmin, const float* xmax, int64_t n_events,
                      const int64_t* n_events_dev, int max_levels, double* cols12, int32_t* type_out, void* stream);

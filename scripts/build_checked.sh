@@ -9,7 +9,7 @@ OUT=../../build_ab
 mkdir -p $OUT/checked
 FLAGS="-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC -I../../include -DCT_BOUNDS_CHECK"
 PIDS=""
-for f in ct_api ct_filter ct_filter_seq ct_detect ct_cusum ct_welch ct_loader; do
+for f in ct_api ct_filter ct_filter_seq ct_detect ct_cusum ct_stepfit ct_welch ct_loader; do
   ( $NVCC $FLAGS -c $f.cu -o $OUT/checked/$f.o ) &
   PIDS="$PIDS $!"
 done
