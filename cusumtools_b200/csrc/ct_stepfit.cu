@@ -229,6 +229,7 @@ __global__ void __launch_bounds__(kSfWarps * 32, 2) ct_stepfit_kernel(StepArgs a
     if (p0 < 0 || p1 > a.ntot || nn <= 2LL * pad || nn > CT_STEPFIT_MAX_WINDOW) {
         if (lane < 6) prow[lane] = 0.0;
         if (lane == 0) { a.cost[ev] = 0.0; a.iters[ev] = 0; a.n_levels[ev] = 0; a.type[ev] = kTypeStepFitFailed; }
+        for (int i = lane; i <= a.max_levels; i += 32) ed[i] = -1;   // as a failed fit: no level rows
         return;
     }
     const int n = (int)nn;

@@ -29,7 +29,8 @@ MAX_WINDOW = _lib.STEPFIT_MAX_WINDOW
 @dataclass
 class StepFitTable:
     """Per-event fit.  params[e] = (i0 pA, a pA, u1, u2, tau1, tau2 samples, relative to the window start); cost = sum
-    of squared residuals (pA^2) at the fit; iters = model evaluations; status = 1 (valid fit), 7 (fit failed), or the
+    of squared residuals (pA^2) at the fit; iters = LM trials (the initial evaluation and every trial, evaluated or
+    not: a trial without a positive-definite matrix or outside the domain still counts); status = 1 (valid fit), 7 (fit failed), or the
     event's type if it was not fitted (its row is then zero)."""
     params: torch.Tensor       # float64 [E, 6]
     cost: torch.Tensor         # float64 [E]

@@ -230,10 +230,13 @@ int ct_stepfit_select(const int64_t* win_start, const int64_t* win_end, int32_t*
                       int64_t capacity, int64_t padding, int64_t stepfit_samples, void* stream);
 /* Levenberg-Marquardt fit of every type-1 event from the initial guess i0 = mean of the first and last `padding`
  * samples, a = i0 - mean of the rest, u1 = padding, u2 = n - padding, tau1 = tau2 = tau0 (samples), at most
- * `max_iters` model evaluations.  A valid fit writes its level rows (n_levels = 3, edges = {0, ceil u1, ceil u2, n},
- * mean = {i0, i0 - a, i0}, std = rms of the residual over each level); an invalid one sets type 7 and n_levels = 0.
- * params6 [capacity][6] (i0 and a in pA, the rest in samples), cost (sum of squared residuals, pA^2) and iters
- * (evaluations) are written for every row below the count, zero for events that are not type 1.  It must run AFTER
+ * `max_iters` LM trials.  A valid fit writes its level rows (n_levels = 3, edges = {0, ceil u1, ceil u2, n},
+ * mean = {i0, i0 - a, i0}, std = rms of the residual over each level); an invalid fit or a window it rejects (outside
+ * [0, n_total), not longer than 2 padding, longer than CT_STEPFIT_MAX_WINDOW) sets type 7, n_levels = 0 and the edge
+ * row to -1.  params6 [capacity][6] (i0 and a in pA, the rest in samples), cost (sum of squared residuals, pA^2) and
+ * iters (LM trials: the initial evaluation and every trial after it, including those never evaluated because the
+ * matrix was not positive definite or the trial point left the domain tau > 0, u1 < u2) are written for every row
+ * below the count, zero for events that are not type 1 and for rejected windows.  It must run AFTER
  * ct_cusum_batch_dev, which writes n_levels = 0 for every event whose type is not 0.                               */
 int ct_stepfit_batch(const float* y, int64_t n_total, const int64_t* win_start, const int64_t* win_end, int32_t* type,
                      const int64_t* n_events_dev, int64_t capacity, int64_t padding, float tau0, int max_iters, int max_levels,

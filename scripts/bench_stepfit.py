@@ -1,7 +1,7 @@
 """Step-response fit timings on one GPU, in one run:
   * ct_stepfit_batch alone on 1 M short events (synth.short_events_device: pulses of 20-400 samples, log-uniform,
     100 baseline samples either side, 150 pA raw noise, 100 kHz / 8-pole zero-phase Bessel at 4.17 MHz), timed with
-    CUDA events around each launch after warm-up: events/s, window samples/s, LM evaluations, fraction fitted;
+    CUDA events around each launch after warm-up: events/s, window samples/s, LM trials (the `iters` column), fraction fitted;
   * the TraceAnalyzer step on a 10-minute trace of short single-level pulses with stepfit on and off, alternated.
 The card's name and power limit are read in the same run.  Output: one JSON document (stdout and --out).
     python scripts/bench_stepfit.py [--events 1000000] [--launches 10] [--minutes 10] [--out FILE]"""

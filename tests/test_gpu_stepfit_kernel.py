@@ -1,0 +1,306 @@
+"""The step-fit kernel (ct_stepfit_batch) against the float64 twin of its own LM loop (oracle/stepfit_twin.py), at every
+window size it accepts: the evaluation pass, the first LM step, the first K trials, full fits as local minima, the
+row contract of its outputs, flat windows and the pipeline without CUSUM+.  Where the kernel's float32 sums may
+decide a comparison differently from float64 (a margin below the bound), the event is skipped; the measured maxima are
+recorded as junit properties."""
+import numpy as np
+import pytest
+import torch
+
+from cusumtools_b200 import pipeline, stepfit, synth
+from oracle import stepfit_oracle as so
+from oracle import stepfit_twin as tw
+
+pytestmark = pytest.mark.gpu
+FS = synth.FS
+PAD = synth.SHORT_PAD
+TAU0 = stepfit.zero_phase_rise_tau(FS, 1e5, 8)
+GAP = 37                                   # samples between neighbouring windows of the test trace
+# windows at both ends of the accepted range, around the shared-memory staging slot (2048) and at the 8192 limit
+EDGE_SIZES = [2 * PAD + 1, 2 * PAD + 2, 2 * PAD + 31, 2 * PAD + 32, 2 * PAD + 33, 2047, 2048, 2049, 4095, 8191, 8192]
+# decisions closer to their threshold than this may go the other way in float32 (stepfit_twin.fit lists the units):
+# the cost carries ~1e-7 relative error, the predicted decrease and the relative step that of the gradient sums
+TIES = dict(pd=1e-4, pred=1e-2, rel=1e-2, domain=1e-4, accept=1e-5, decrease=1e-5)
+
+
+def _tie(f, **over):
+    lim = {**TIES, **over}
+    return any(m < lim[k] for k, m in f.margins if k in lim)
+
+
+def _sizes():
+    rng = np.random.default_rng(21)
+    short = np.exp(rng.uniform(np.log(2 * PAD + 20), np.log(2 * PAD + 1200), 44)).astype(int)
+    long_ = rng.integers(2100, 8193, 10)
+    # every size twice: once above a positive baseline, once below a negative one
+    return [int(n) for n in EDGE_SIZES for _ in range(2)] + [int(n) for n in short] + [int(n) for n in long_]
+
+
+@pytest.fixture(scope="module")
+def trace():
+    """The windows laid out in one trace, the first at w0 = 0 and the last ending at w1 = n_total; y is an offset-1
+    view of its buffer (4-byte aligned only)."""
+    sizes = _sizes()
+    wins = tw.filtered_pulse_windows(sizes, PAD, seed=5)
+    w0 = np.zeros(len(wins), np.int64)
+    pos = 0
+    for i, w in enumerate(wins):
+        w0[i] = pos
+        pos += w.size + GAP
+    n_total = pos - GAP
+    host = np.full(n_total + 1, 1234.5, np.float32)
+    for a, w in zip(w0, wins):
+        host[1 + a:1 + a + w.size] = w
+    buf = torch.from_numpy(host).cuda()
+    y = buf[1:]
+    w1 = w0 + np.array([w.size for w in wins], np.int64)
+    assert w0[0] == 0 and w1[-1] == n_total and y.data_ptr() % 8 == 4
+    return dict(y=y, wins=wins, w0=w0, w1=w1, n_total=n_total,
+                w0d=torch.from_numpy(w0).cuda(), w1d=torch.from_numpy(w1).cuda())
+
+
+def _fit(t, max_iters, max_levels=3):
+    r = stepfit.step_fit(t["y"], t["w0d"], t["w1d"], padding=PAD, tau0=TAU0, max_iters=max_iters, max_levels=max_levels)
+    lv = r.levels
+    return dict(params=r.params.cpu().numpy(), cost=r.cost.cpu().numpy(), iters=r.iters.cpu().numpy(),
+                type=r.status.cpu().numpy(), n_levels=lv.n_levels.cpu().numpy(), edges=lv.edges.cpu().numpy(),
+                mean=lv.mean.cpu().numpy(), std=lv.std.cpu().numpy())
+
+
+def _anorm(x, p, v):
+    xr, x0 = tw.window(x)
+    q = np.array(p, np.float64)
+    q[0] -= x0
+    _, _, A = tw.sums(xr, q)
+    return float(np.sqrt(v @ A @ v))
+
+
+def test_evaluation_pass(trace, record_property):
+    g = _fit(trace, max_iters=1)
+    worst = 0.0
+    for e, x in enumerate(trace["wins"]):
+        f = tw.fit(x, PAD, TAU0, max_iters=1)
+        assert np.allclose(g["params"][e], f.initial, rtol=1e-12, atol=0), (e, x.size, g["params"][e], f.initial)
+        c = tw.cost_at(x, g["params"][e])
+        worst = max(worst, abs(g["cost"][e] - c) / c)
+        assert g["cost"][e] == pytest.approx(c, rel=2e-6), (e, x.size)              # 1.7e-7 measured (B200)
+    assert np.all(g["iters"] == 1) and np.all(g["type"] == 7) and np.all(g["n_levels"] == 0) and np.all(g["edges"] == -1)
+    record_property("evaluation_cost_rel_err_max", worst)
+
+
+def test_first_step_follows_the_twin(trace, record_property):
+    g = _fit(trace, max_iters=2)
+    worst_a, worst_c, n_step, n_skip = 0.0, 0.0, 0, 0
+    for e, x in enumerate(trace["wins"]):
+        f = tw.fit(x, PAD, TAU0, max_iters=2)
+        if _tie(f, accept=1e-4):
+            n_skip += 1
+            continue
+        st = f.steps[0]
+        assert g["iters"][e] == f.iters, (e, x.size, st.kind)
+        d = g["params"][e] - f.initial
+        if st.kind != "accept":
+            # a rejected trial, one outside the domain, no positive-definite matrix, or a stop: the initial guess
+            assert np.array_equal(g["params"][e], f.initial), (e, x.size, st.kind)
+            continue
+        n_step += 1
+        dn = _anorm(x, f.initial, st.d)
+        ea = _anorm(x, f.initial, d - st.d) / dn
+        ec = float(np.max(np.abs(d - st.d) / np.abs(st.d)))
+        worst_a, worst_c = max(worst_a, ea), max(worst_c, ec)
+        assert ea <= 2e-5 and ec <= 1e-3, (e, x.size, d, st.d)                     # 2.2e-6 and 1.3e-4 measured
+    assert n_step >= 0.8 * len(trace["wins"]) and n_skip <= 0.1 * len(trace["wins"])
+    record_property("first_step_anorm_rel_err_max", worst_a)
+    record_property("first_step_component_rel_err_max", worst_c)
+    record_property("first_step_compared", n_step)
+
+
+@pytest.mark.parametrize("K", range(3, 9))
+def test_first_trials_follow_the_twin(trace, K, record_property):
+    g = _fit(trace, max_iters=K)
+    worst, n_cmp = 0.0, 0
+    for e, x in enumerate(trace["wins"]):
+        f = tw.fit(x, PAD, TAU0, max_iters=K)
+        if _tie(f):
+            continue
+        n_cmp += 1
+        assert g["iters"][e] == f.iters, (e, x.size, [s.kind for s in f.steps])
+        moved = f.params - f.initial
+        if not np.any(moved):
+            assert np.array_equal(g["params"][e], f.initial), (e, x.size)
+            continue
+        err = _anorm(x, f.params, g["params"][e] - f.params) / _anorm(x, f.params, moved)
+        worst = max(worst, err)
+        assert err <= 3e-5, (e, x.size, g["params"][e], f.params)                   # 3.1e-6 measured (K = 3)
+    assert n_cmp >= 0.7 * len(trace["wins"])
+    record_property(f"trials{K}_anorm_rel_err_max", worst)
+    record_property(f"trials{K}_compared", n_cmp)
+
+
+def _check_full_fits(wins, g, record_property, tag):
+    worst_cost, worst_dc, worst_move, worst_sd = 0.0, 0.0, 0.0, 0.0
+    for e, x in enumerate(wins):
+        if g["type"][e] not in (1, 7):
+            continue
+        c = tw.cost_at(x, g["params"][e])
+        worst_cost = max(worst_cost, abs(g["cost"][e] - c) / c)
+        if g["type"][e] != 1:
+            assert g["n_levels"][e] == 0 and np.all(g["edges"][e] == -1)
+            continue
+        dc, move = tw.local_minimum_gap(x, g["params"][e])
+        worst_dc, worst_move = max(worst_dc, dc), max(worst_move, move)
+        # measured: 2.0e-7 and 0.018 se (a long event); 0.02 se is the bound a converged float32 fit is held to
+        assert dc <= 1e-6 and move <= 0.02, (e, x.size, dc, move)
+        edges, mean, std = so.level_rows(x, g["params"][e])
+        assert g["n_levels"][e] == 3 and np.array_equal(g["edges"][e, :4], edges) and np.all(g["edges"][e, 4:] == -1)
+        assert np.allclose(g["mean"][e, :3], mean, rtol=1e-12, atol=0)
+        sd_err = float(np.max(np.abs(g["std"][e, :3] - std) / std))
+        worst_sd = max(worst_sd, sd_err)
+        assert sd_err <= 5e-6, (e, x.size, g["std"][e, :3], std)                   # 7.8e-7 measured
+    assert worst_cost <= 5e-6, worst_cost                                  # 7.7e-7 measured
+    record_property(f"{tag}_cost_rel_err_max", worst_cost)
+    record_property(f"{tag}_lm_cost_decrease_max", worst_dc)
+    record_property(f"{tag}_lm_move_se_max", worst_move)
+    record_property(f"{tag}_level_std_rel_err_max", worst_sd)
+    return int(np.count_nonzero(g["type"] == 1))
+
+
+@pytest.mark.parametrize("kind", ["short", "long"])
+def test_full_fits_are_local_minima(kind, record_property):
+    if kind == "short":
+        x, off, _, _ = synth.short_events_device(600, "cuda:0", seed=31)
+    else:
+        x, off, _, _ = synth.short_events_device(40, "cuda:0", seed=32, min_len=800, max_len=7700)
+    r = stepfit.stepfit_flat(x, off, padding=PAD, tau0=TAU0)
+    lv = r.levels
+    g = dict(params=r.params.cpu().numpy(), cost=r.cost.cpu().numpy(), type=r.status.cpu().numpy(),
+             n_levels=lv.n_levels.cpu().numpy(), edges=lv.edges.cpu().numpy(), mean=lv.mean.cpu().numpy(),
+             std=lv.std.cpu().numpy())
+    xs, of = x.cpu().numpy(), off.cpu().numpy()
+    wins = [xs[of[e]:of[e + 1]] for e in range(len(of) - 1)]
+    n_valid = _check_full_fits(wins, g, record_property, kind)
+    assert n_valid >= 0.9 * len(wins)
+
+
+def test_full_fits_at_every_window_size(trace, record_property):
+    g = _fit(trace, max_iters=stepfit.DEFAULT_MAX_ITERS)
+    _check_full_fits(trace["wins"], g, record_property, "sizes")
+
+
+SENT_F, SENT_I = -3.25, 777
+
+
+def _contract_rows(t):
+    """(w0, w1, type) of 64 rows and the count 40: fitted windows, rows of other types, rejected windows, and
+    type-1 rows at or beyond the count."""
+    w0, w1, n = list(t["w0"]), list(t["w1"]), t["n_total"]
+    typ = [1] * len(w0)
+    sel = [0, 1, 10, 12, 13, 14, 16, 18, 20, 21, 23, 30, 40]          # fitted: 201 ... 8192 samples, both signs
+    rows = [(w0[i], w1[i], 1) for i in sel]
+    rows += [(w0[i], w1[i], k) for i, k in zip((31, 32, 33, 34), (0, 2, 5, 7))]  # not type 1: not fitted
+    rows += [(-1, w1[3], 1), (w0[5], n + 1, 1), (100, 100 + 2 * PAD, 1), (100, 100 + 2 * PAD - 7, 1),
+             (100, 100, 1), (0, 8193, 1), (0, 1 << 20, 1)]              # rejected windows
+    while len(rows) < 40:
+        rows.append((w0[len(rows)], w1[len(rows)], 1))
+    rows += [(w0[i], w1[i], 1) for i in range(24)]                      # beyond the count
+    return np.array([r[0] for r in rows]), np.array([r[1] for r in rows]), np.array([r[2] for r in rows], np.int32), 40
+
+
+def _launch_sentinel(t, max_levels, w0, w1, typ, count):
+    dev = t["y"].device
+    cap = w0.size
+    types = torch.from_numpy(typ.copy()).to(dev)
+    out = {"params": torch.full((cap, 6), SENT_F, dtype=torch.float64, device=dev),
+           "cost": torch.full((cap,), SENT_F, dtype=torch.float64, device=dev),
+           "iters": torch.full((cap,), SENT_I, dtype=torch.int32, device=dev)}
+    lv = {"n_levels": torch.full((cap,), SENT_I, dtype=torch.int32, device=dev),
+          "edges": torch.full((cap, max_levels + 1), SENT_I, dtype=torch.int32, device=dev),
+          "mean": torch.full((cap, max_levels), SENT_F, dtype=torch.float64, device=dev),
+          "std": torch.full((cap, max_levels), SENT_F, dtype=torch.float64, device=dev)}
+    stepfit.launch(t["y"], torch.from_numpy(w0).to(dev), torch.from_numpy(w1).to(dev), types, out, lv, padding=PAD,
+                   tau0=TAU0, n_events_dev=torch.tensor([count], dtype=torch.int64, device=dev), capacity=cap)
+    res = {k: v.cpu().numpy() for k, v in {**out, **lv}.items()}
+    res["type"] = types.cpu().numpy()
+    return res
+
+
+def test_row_contract(trace):
+    t = trace
+    w0, w1, typ, count = _contract_rows(t)
+    base = None
+    for ml in (3, 5, 16, 40):
+        g = _launch_sentinel(t, ml, w0, w1, typ, count)
+        below = np.arange(w0.size) < count
+        # rows at or beyond the count: untouched
+        for k in ("params", "cost", "mean", "std"):
+            assert np.all(g[k][~below] == SENT_F), k
+        for k in ("iters", "n_levels", "edges"):
+            assert np.all(g[k][~below] == SENT_I), k
+        assert np.array_equal(g["type"][~below], typ[~below])
+        # rows of other types: params, cost, iters zero; type and level rows untouched
+        other = below & (typ != 1)
+        assert np.all(g["params"][other] == 0) and np.all(g["cost"][other] == 0) and np.all(g["iters"][other] == 0)
+        assert np.array_equal(g["type"][other], typ[other]) and np.all(g["n_levels"][other] == SENT_I)
+        assert np.all(g["edges"][other] == SENT_I) and np.all(g["mean"][other] == SENT_F) and np.all(g["std"][other] == SENT_F)
+        # rejected windows: type 7 with zero params, no level rows (edges -1), mean / std untouched
+        n = w1 - w0
+        rej = below & (typ == 1) & ((w0 < 0) | (w1 > t["n_total"]) | (n <= 2 * PAD) | (n > stepfit.MAX_WINDOW))
+        assert rej.sum() == 7
+        assert np.all(g["type"][rej] == 7) and np.all(g["n_levels"][rej] == 0) and np.all(g["edges"][rej] == -1)
+        assert np.all(g["params"][rej] == 0) and np.all(g["cost"][rej] == 0) and np.all(g["iters"][rej] == 0)
+        assert np.all(g["mean"][rej] == SENT_F) and np.all(g["std"][rej] == SENT_F)
+        # fitted rows: three level rows and -1 to the end of the edge row (max_levels 40: two rounds of lanes)
+        fit = below & (typ == 1) & ~rej
+        ok, bad = fit & (g["type"] == 1), fit & (g["type"] == 7)
+        assert ok.sum() >= 10 and np.all(np.isin(g["type"][fit], (1, 7)))
+        assert np.all(g["n_levels"][ok] == 3) and np.all(g["edges"][ok, 4:] == -1)
+        assert np.all(g["mean"][ok, 3:] == SENT_F) and np.all(g["std"][ok, 3:] == SENT_F)
+        assert np.all(g["n_levels"][bad] == 0) and np.all(g["edges"][bad] == -1) and np.all(g["mean"][bad] == SENT_F)
+        assert np.all(g["iters"][fit] >= 1) and np.all(g["cost"][fit] > 0)
+        # the same rows whatever the stride
+        rows = {k: g[k] for k in ("params", "cost", "iters", "type", "n_levels")}
+        rows.update(edges=g["edges"][:, :4], mean=g["mean"][:, :3], std=g["std"][:, :3])
+        if base is None:
+            base = rows
+        for k in rows:
+            assert np.array_equal(rows[k], base[k]), (ml, k)
+
+
+def test_flat_windows_fail_with_finite_params():
+    n = 300
+    levels = (5000.0, -5000.0, 0.0)
+    x = np.concatenate([np.full(n, v, np.float32) for v in levels])
+    off = torch.arange(len(levels) + 1, dtype=torch.int64, device="cuda") * n
+    r = stepfit.stepfit_flat(torch.from_numpy(x).cuda(), off, padding=PAD, tau0=TAU0)
+    p, it = r.params.cpu().numpy(), r.iters.cpu().numpy()
+    assert np.all(r.status.cpu().numpy() == 7) and np.all(np.isfinite(p)) and np.all(r.levels.n_levels.cpu().numpy() == 0)
+    for e in range(len(levels)):
+        f = tw.fit(x[e * n:(e + 1) * n], PAD, TAU0)
+        # a = 0: no positive-definite matrix, mu grows x10 per trial until the guard mu < 1e30 stops the loop
+        assert it[e] == f.iters == 35 and np.array_equal(p[e], f.initial)
+
+
+def test_pipeline_without_cusum_keeps_the_fitted_rows():
+    kw = dict(threshold=5.0, hysteresis=1.0, baseline_block=1 << 16, baseline_min=4700.0, baseline_max=5300.0,
+              cusum_h=10.0, stepfit_samples=500)
+    # test_gpu_stepfit's pulse trace (L = 100: every event is fitted), then the default two-level events (2000
+    # samples: every event is left to CUSUM+)
+    codes = torch.cat((synth.device_trace(4_194_304, "cuda:0", seed=200, levels=((-1000.0, 100),)),
+                       synth.device_trace(4_194_304, "cuda:0", seed=201)))
+    runs = {}
+    for delta in (400.0, None):
+        an = pipeline.TraceAnalyzer(codes.numel(), synth.CHIMERA_SETTINGS, 1e5, 8, device="cuda:0", cusum_delta=delta, **kw)
+        runs[delta] = an.tables_to_host(an.run(codes))
+        runs[delta] = {k: v.copy() for k, v in runs[delta].items()}
+    on, off = runs[400.0], runs[None]
+    assert np.array_equal(on["types"], off["types"])
+    fit = np.isin(on["types"], (1, 7))
+    assert np.count_nonzero(on["types"] == 1) > 900
+    for k in ("stepfit_params", "stepfit_cost", "stepfit_iters", "n_levels", "edges"):
+        assert np.array_equal(on[k][fit], off[k][fit]), k
+    ok = on["types"] == 1                                                # type 7 rows hold no level rows
+    for k in ("mean", "std"):
+        assert np.array_equal(on[k][ok, :3], off[k][ok, :3]), k
+    assert np.count_nonzero(~fit) > 900
+    assert np.all(off["n_levels"][~fit] == 0) and np.all(off["edges"][~fit] == -1)
+    assert np.mean(on["n_levels"][~fit] > 0) > 0.9                       # CUSUM+ filled them in the other run
