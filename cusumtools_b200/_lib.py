@@ -86,8 +86,13 @@ SIGNATURES = {
     "ct_stepfit_select": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp]),
     "ct_stepfit_batch": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _i64, _i64, _f32, C.c_int, C.c_int, _vp, _vp, _vp, _vp, _vp,
                                    _vp, _vp, _vp]),
+    "ct_stepfit_fallback_select": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp]),
+    "ct_stepfit_long_batch": (C.c_int, [_vp, _i64, _vp, _vp, _vp, _vp, _i64, _i64, _f32, C.c_int, C.c_int, _vp, _vp, _vp, _vp,
+                                        _vp, _vp, _vp, _vp, _vp]),
 }
 STEPFIT_MAX_WINDOW = 8192     # CT_STEPFIT_MAX_WINDOW
+STEPFIT_LONG_MAX_WINDOW = 131072     # CT_STEPFIT_LONG_MAX_WINDOW
+TYPE_STEPFIT_LONG = 8         # CT_TYPE_STEPFIT_LONG
 
 _lib = None
 

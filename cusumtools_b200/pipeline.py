@@ -271,7 +271,8 @@ class TraceAnalyzer:
                  cusum_h: float | None = None, max_levels: int = cusum.DEFAULT_MAX_LEVELS,
                  event_capacity: int | None = None, group=None, device="cuda", fuse_stats: bool = True,
                  fused_count: bool = True, intra_threshold: float = 0.0, intra_hysteresis: float = 0.0,
-                 max_crossings: int = 8, halos_clipped_by_trace_ends: bool = False, stepfit_samples: int = 0):
+                 max_crossings: int = 8, halos_clipped_by_trace_ends: bool = False, stepfit_samples: int = 0,
+                 stepfit_fallback: bool = False):
         self.n_ext, self.lo_halo, self.hi_halo = int(n_ext), int(lo_halo), int(hi_halo)
         self.n_own = self.n_ext - self.lo_halo - self.hi_halo
         self.n_det = self.n_ext
@@ -300,8 +301,15 @@ class TraceAnalyzer:
         if self.stepfit_samples and self.stepfit_samples + 2 * self.event_padding > stepfit.MAX_WINDOW:
             raise ValueError(f"stepfit_samples + 2 * event_padding = {self.stepfit_samples + 2 * self.event_padding} exceeds "
                              f"the {stepfit.MAX_WINDOW}-sample window of the step-response fit")
+        # the same fit of every event CUSUM+ leaves without a sub-level (type 5 otherwise), whatever its length; with
+        # cusum_delta None, of every accepted event
+        self.stepfit_fallback = bool(stepfit_fallback)
+        if self.stepfit_fallback and self.maxpoints + 2 * self.event_padding > stepfit.LONG_MAX_WINDOW:
+            raise ValueError(f"maxpoints + 2 * event_padding = {self.maxpoints + 2 * self.event_padding} exceeds the "
+                             f"{stepfit.LONG_MAX_WINDOW}-sample window of the step-response fallback")
+        self.fit_on = bool(self.stepfit_samples) or self.stepfit_fallback
         self.tau0 = (stepfit.zero_phase_rise_tau(float(np.floor(np.squeeze(settings["ADCSAMPLERATE"]))), cutoff, order)
-                     if self.stepfit_samples else 0.0)
+                     if self.fit_on else 0.0)
         self.group = group
         self.device = torch.device(device)
         self.mask = filters.chimera_bitmask(settings)
@@ -334,13 +342,15 @@ class TraceAnalyzer:
         if self.intra_threshold > 0:
             self.ic = torch.zeros(cap, dtype=torch.int32, device=dev)
             self.ip = torch.full((cap, 2 * self.max_crossings), -1, dtype=torch.int32, device=dev)
-        if self.delta is not None or self.stepfit_samples:
+        if self.delta is not None or self.fit_on:
             self.nl = torch.empty(cap, dtype=torch.int32, device=dev)
             self.ed = torch.empty((cap, ML + 1), dtype=torch.int32, device=dev)
             self.mu = torch.empty((cap, ML), dtype=torch.float64, device=dev)
             self.sd = torch.empty((cap, ML), dtype=torch.float64, device=dev)
             self.ov = torch.empty(cap, dtype=torch.uint8, device=dev)
-        if self.stepfit_samples:
+        if self.stepfit_fallback:
+            self.sf_counter = torch.empty(1, dtype=torch.int64, device=dev)     # rows claimed by the long fit
+        if self.fit_on:
             self.sf = {"params": torch.empty((cap, 6), dtype=torch.float64, device=dev),
                        "cost": torch.empty(cap, dtype=torch.float64, device=dev),
                        "iters": torch.empty(cap, dtype=torch.int32, device=dev)}
@@ -513,12 +523,18 @@ class TraceAnalyzer:
                                           self.mu.data_ptr(), self.sd.data_ptr(), self.ov.data_ptr(), self.cws.data_ptr(),
                                           self.cws_bytes, st)
                 _lib.check(rc, "ct_cusum_batch_dev")
-            elif self.stepfit_samples:           # no CUSUM+: the rows of the events the fit does not take stay empty
+            elif self.fit_on:                    # no CUSUM+: the rows of the events the fit does not take stay empty
                 self.nl.zero_(); self.ov.zero_(); self.ed.fill_(-1)
-            if self.stepfit_samples:             # after CUSUM+, which writes n_levels = 0 for every event not of type 0
-                stepfit.launch(yd, self.w0, self.w1, self.typ, self.sf,
-                               {"n_levels": self.nl, "edges": self.ed, "mean": self.mu, "std": self.sd},
-                               padding=self.event_padding, tau0=self.tau0, n_events_dev=sc[2:], capacity=self.cap)
+            if self.stepfit_fallback:            # the events CUSUM+ left without a sub-level: type 1, or 8 (long)
+                stepfit.select_fallback({"n_levels": self.nl, "overflow": self.ov}, self.w0, self.w1, self.typ,
+                                        n_events_dev=sc[2:], capacity=self.cap)
+            if self.fit_on:                      # after CUSUM+, which writes n_levels = 0 for every event not of type 0
+                lvd = {"n_levels": self.nl, "edges": self.ed, "mean": self.mu, "std": self.sd}
+                stepfit.launch(yd, self.w0, self.w1, self.typ, self.sf, lvd, padding=self.event_padding, tau0=self.tau0,
+                               n_events_dev=sc[2:], capacity=self.cap)
+            if self.stepfit_fallback:            # after the short fit, which zeroes the params of every row not of type 1
+                stepfit.launch_long(yd, self.w0, self.w1, self.typ, self.sf, lvd, padding=self.event_padding,
+                                    tau0=self.tau0, n_events_dev=sc[2:], capacity=self.cap, row_counter=self.sf_counter)
             if self.intra_threshold > 0:
                 # the block of the event start: win_start + padding (windows are compacted, the start list is not)
                 detect.intra_crossings(yd, self.w0, self.w1, self.w0 + self.event_padding, bl, self.intra_threshold,
@@ -554,9 +570,9 @@ class TraceAnalyzer:
         # event indices are reported relative to the first owned sample
         ev = detect.EventList(self.starts[i0:i0 + nk] - lo, self.ends[i0:i0 + nk] - lo, open_start)
         lv = sf = None
-        if self.delta is not None or self.stepfit_samples:
+        if self.delta is not None or self.fit_on:
             lv = cusum.LevelTable(self.nl[:nk], self.ed[:nk], self.mu[:nk], self.sd[:nk], self.ov[:nk], self.max_levels)
-        if self.stepfit_samples:
+        if self.fit_on:
             sf = stepfit.StepFitTable(self.sf["params"][:nk], self.sf["cost"][:nk], self.sf["iters"][:nk], self.typ[:nk])
         return AnalysisResult(filtered=y[lo:lo + n_own], detect_trace=yd, lo_halo=lo, baseline=bl, events=ev,
                               win_start=self.w0[:nk], win_end=self.w1[:nk], types=self.typ[:nk], levels=lv,
@@ -726,7 +742,8 @@ class StreamingAnalyzer:
         self.padding = int(kw.get("padding", 1000))
         self.mask = filters.chimera_bitmask(settings)
         self.max_levels = int(kw.get("max_levels", cusum.DEFAULT_MAX_LEVELS))
-        self.with_levels = kw.get("cusum_delta") is not None or bool(kw.get("stepfit_samples"))
+        self.with_levels = (kw.get("cusum_delta") is not None or bool(kw.get("stepfit_samples"))
+                            or bool(kw.get("stepfit_fallback")))
         fs = float(np.floor(np.squeeze(settings["ADCSAMPLERATE"])))
         max_event = int(kw.get("maxpoints", 100_000)) + 2 * int(kw.get("event_padding", 100))
         self.h = required_halo(self.cutoff, self.order, fs, max_event, self.padding, block=self.block)

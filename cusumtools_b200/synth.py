@@ -70,8 +70,12 @@ def device_trace(n: int, device, seed: int = 1234, events_per_s: float = 1000.0,
     uint16 CUDA tensor.  `start_index` is the global index of sample 0 (time sharding):
     the event grid is global, the noise stream is per shard (seed).  `levels`: the event
     template as ((depth pA, samples), ...), default EVENT_LEVELS (e.g. ((-1000.0, 100),) for
-    short single-level pulses)."""
-    levels = EVENT_LEVELS if levels is None else tuple((float(d), int(l)) for d, l in levels)
+    short single-level pulses), or a sequence of such templates: event k takes template
+    k mod len(levels) (mixed traces: two-level events, short pulses, shallow long events)."""
+    if levels is None:
+        levels = EVENT_LEVELS
+    templates = ([levels] if np.ndim(levels[0]) == 1 else list(levels))
+    templates = [tuple((float(d), int(l)) for d, l in tpl) for tpl in templates]
     import torch
     g = torch.Generator(device=device)
     g.manual_seed(seed)
@@ -80,7 +84,7 @@ def device_trace(n: int, device, seed: int = 1234, events_per_s: float = 1000.0,
     step = 1 << (16 - bits)
     period = int(round(FS / events_per_s))
     out = torch.empty(n, dtype=torch.uint16, device=device)
-    tot = sum(l for _, l in levels)
+    tot = max(sum(l for _, l in tpl) for tpl in templates)
     jg = torch.Generator(device="cpu")
     jg.manual_seed(seed + 7919)
     for c0 in range(0, n, chunk):
@@ -95,10 +99,13 @@ def device_trace(n: int, device, seed: int = 1234, events_per_s: float = 1000.0,
             jit = (h % (2 * jitter + 1)) - jitter if jitter > 0 else torch.zeros_like(h)
             st = 1500 + kk * period + jit
             rel = gidx - st
-            o = 0
-            for depth, length in levels:
-                cur += depth * ((rel >= o) & (rel < o + length) & (kk >= 0))
-                o += length
+            for j, tpl in enumerate(templates):
+                o = 0
+                # (one template: no selection term, so the single-template trace is the one it always was)
+                sel = (kk >= 0) if len(templates) == 1 else (kk >= 0) & (kk % len(templates) == j)
+                for depth, length in tpl:
+                    cur += depth * ((rel >= o) & (rel < o + length) & sel)
+                    o += length
         code = torch.round((cur - beta) / alpha / step) * step
         out[c0:c1] = code.clamp_(0, 65536 - step).to(torch.int32).to(torch.uint16)
         del cur, gidx, k, code

@@ -21,6 +21,8 @@ fixed here (SURVEY.md Appendix A.4 lists the open points):
   `time_us,current_pA,cusum_fit,stepfit`, readevents.py:1334-1337), 2 too short, 3 too long, 4 padding
   overlaps a neighbour or leaves the trace, 5 CUSUM+ found no sub-level, 6 more levels than
   the table holds, 7 step fit failed; types > 1 appear in rate.csv only (`plot-trace.py:354-357`);
+  type 1 is a short event (`stepfit_samples`) or, with `stepfit_fallback`, an event CUSUM+ left without a
+  sub-level (type 5 without it), of any accepted length; type 7 may then be an event of any length;
 * a type-1 event has three level rows from its fit p = (i0, a, u1, u2, tau1, tau2) (stepfit.py):
   edges [0, ceil u1, ceil u2, n], means [i0, i0 - a, i0], std = rms of trace minus fitted step response
   over each; the derived columns follow from them as for a CUSUM fit.  `rc_const1_us` / `rc_const2_us`
@@ -321,7 +323,7 @@ def write_analysis_dir(path: str, table: EventTable, *, baseline_mean, baseline_
                        samplerate: float, threshold: float, hysteresis: float, cutoff: float, poles: int,
                        extra_summary: dict | None = None, event_samples=None, time_offset_s: float = 0.0,
                        append: bool = False, intra_threshold: float = 0.0, intra_hysteresis: float = 0.0,
-                       stepfit_samples: int = 0) -> None:
+                       stepfit_samples: int = 0, stepfit_fallback: bool = False) -> None:
     """Write `events.csv`, `rate.csv`, `baseline.csv`, `summary.txt` and (if `event_samples`
     is given) `events/event_%08d.csv` under `path`.
 
@@ -330,7 +332,8 @@ def write_analysis_dir(path: str, table: EventTable, *, baseline_mean, baseline_
     (`readevents.py:1334-1337` names them time, current, cusum) WITH a header line, because
     the consumer reads them with an implicit header row (`readevents.py:1319`).  An entry with
     parameters (a type-1 event) gets a fourth column `stepfit`, the fitted step response f(t).
-    `stepfit_samples` > 0 (the analyzer's length threshold of the fit) is recorded in summary.txt."""
+    `stepfit_samples` > 0 (the analyzer's length threshold of the fit) and `stepfit_fallback` (the analyzer fitted
+    the events CUSUM+ left without a sub-level) are recorded in summary.txt."""
     os.makedirs(os.path.join(path, "events"), exist_ok=True)
     _write_csv(os.path.join(path, "events.csv"), EVENT_COLUMNS, table.events)
     _write_csv(os.path.join(path, "rate.csv"), RATE_COLUMNS, table.rate)
@@ -348,6 +351,8 @@ def write_analysis_dir(path: str, table: EventTable, *, baseline_mean, baseline_
                "events_accepted": str(len(table))}
     if stepfit_samples:
         summary["stepfit_samples"] = str(int(stepfit_samples))
+    if stepfit_fallback:
+        summary["stepfit_fallback"] = "1"
     for k, v in (extra_summary or {}).items():
         if any(w in k for w in ("threshold", "hysteresis", "cutoff", "poles")):
             raise ValueError(f"summary key {k!r} would be mis-parsed by the consumers' substring match")

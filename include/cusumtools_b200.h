@@ -243,6 +243,32 @@ int ct_stepfit_batch(const float* y, int64_t n_total, const int64_t* win_start, 
                      double* params6, double* cost, int32_t* iters, int32_t* n_levels, int32_t* edges, double* level_mean,
                      double* level_std, void* stream);
 
+/* Fallback of the events CUSUM+ leaves without a sub-level (the events ct_event_columns would report as type 5):
+ * ct_stepfit_fallback_select runs AFTER ct_cusum_batch_dev (or after the level rows were zeroed when CUSUM+ is off) and
+ * marks every row below the count with type 0, overflow 0 and n_levels < 3: type 1 if its window is at most
+ * CT_STEPFIT_MAX_WINDOW samples, else CT_TYPE_STEPFIT_LONG.  No other row changes.  n_events_dev may be NULL.
+ * ct_stepfit_long_batch takes the arguments of ct_stepfit_batch and fits the rows of type CT_TYPE_STEPFIT_LONG with one
+ * CTA per event, with the same initial guess, LM loop, stop tests, validity rule and level rows; each such row becomes
+ * type 1 or 7 (a window outside [0, n_total), not longer than 2 padding or longer than CT_STEPFIT_LONG_MAX_WINDOW: type 7,
+ * n_levels = 0, edge row -1, zero params / cost / iters).  It does not touch any row of another type.
+ * row_counter: one int64 of device scratch (the CTAs claim rows from it; reset by the call), not shared with a call that
+ * may run at the same time.
+ * Launch order: ct_stepfit_batch, then ct_stepfit_long_batch.  ct_stepfit_batch zeroes the params row of every row
+ * that is not type 1, which the long fit then overwrites; the other way round, ct_stepfit_batch would take the long
+ * rows that had just become type 1 and reject their windows as too long.
+ * Type codes of the step: 1 step-response fit (short events, or fallback), 5 (ct_event_columns) accepted but no
+ * sub-level, 7 step fit failed (an event of any length), 8 = CT_TYPE_STEPFIT_LONG: long fit pending, internal to the
+ * step (never left in a result).                                                                                    */
+#define CT_TYPE_STEPFIT_LONG 8
+#define CT_STEPFIT_LONG_MAX_WINDOW 131072         /* longest window ct_stepfit_long_batch fits; t - k exact in float32 */
+int ct_stepfit_fallback_select(const int32_t* n_levels, const uint8_t* overflow, const int64_t* win_start,
+                               const int64_t* win_end, int32_t* type, const int64_t* n_events_dev, int64_t capacity,
+                               void* stream);
+int ct_stepfit_long_batch(const float* y, int64_t n_total, const int64_t* win_start, const int64_t* win_end, int32_t* type,
+                          const int64_t* n_events_dev, int64_t capacity, int64_t padding, float tau0, int max_iters,
+                          int max_levels, double* params6, double* cost, int32_t* iters, int32_t* n_levels, int32_t* edges,
+                          double* level_mean, double* level_std, int64_t* row_counter, void* stream);
+
 /* Intra-event threshold crossings (rate.csv intra_crossing_times_us / events.csv intra_crossings;
  * consumer: readevents.py:1340-1343,1363-1367, summary.txt keys intra_threshold / intra_hysteresis
  * readevents.py:73-79).  The detector's automaton over each event window with the lines

@@ -1,0 +1,434 @@
+"""The long step-fit kernel (ct_stepfit_long_batch, one CTA per window of 8 k - 131 k samples) against the float64 twin of
+the fit's LM loop (oracle/stepfit_twin.py), its row contract, the fallback selection (ct_stepfit_fallback_select), and
+`TraceAnalyzer(stepfit_fallback=True)`: the events CUSUM+ leaves without a sub-level (type 5) become type 1 / 7 and
+nothing else changes.  Where the kernel's float32 sums may decide a comparison differently from float64 (a margin below
+the bound), the event is skipped; the measured maxima are recorded as junit properties.
+
+The file fails against each of these single-line kernel mutations (each run on a B200): one warp's partial dropped
+from the cross-warp sum of the evaluation pass; the last sample of a staged window not copied into the slot; the long
+kernel fitting rows of type 1 as well as type 8; the fallback selection ignoring the overflow flag.  (Moving the
+staging bound itself by one, n <= slot + 1, changes no output: the staged and the global path compute the same float
+values; the staging branch checks n against the slot with CT_CHECK_RANGE in the -DCT_BOUNDS_CHECK build.)"""
+import os
+
+import numpy as np
+import pandas as pd
+import pytest
+import torch
+
+from cusumtools_b200 import pipeline, stepfit, synth, writer
+from oracle import stepfit_oracle as so
+from oracle import stepfit_twin as tw
+
+pytestmark = pytest.mark.gpu
+FS = synth.FS
+PAD = synth.SHORT_PAD
+TAU0 = stepfit.zero_phase_rise_tau(FS, 1e5, 8)
+LONG = stepfit.TYPE_STEPFIT_LONG
+GAP = 37
+SLOT = 16384                               # kSfLongSlot: windows up to this many samples are staged in shared memory
+EDGE_SIZES = [8193, 8194, SLOT - 1, SLOT, SLOT + 1, 65537, 100_200, 131_072]
+TIES = dict(pd=1e-4, pred=1e-2, rel=1e-2, domain=1e-4, accept=1e-5, decrease=1e-5)
+
+
+def _tie(f, **over):
+    lim = {**TIES, **over}
+    return any(m < lim[k] for k, m in f.margins if k in lim)
+
+
+def _sizes():
+    rng = np.random.default_rng(22)
+    rand = np.exp(rng.uniform(np.log(8200), np.log(131_000), 8)).astype(int)
+    return [int(n) for n in EDGE_SIZES for _ in range(2)] + [int(n) for n in rand]
+
+
+@pytest.fixture(scope="module")
+def trace():
+    """The windows laid out in one trace, the first at w0 = 0 and the last ending at w1 = n_total; y is an offset-1
+    view of its buffer (4-byte aligned only)."""
+    sizes = _sizes()
+    wins = tw.filtered_pulse_windows(sizes, PAD, seed=6)
+    w0 = np.zeros(len(wins), np.int64)
+    pos = 0
+    for i, w in enumerate(wins):
+        w0[i] = pos
+        pos += w.size + GAP
+    n_total = pos - GAP
+    host = np.full(n_total + 1, 1234.5, np.float32)
+    for a, w in zip(w0, wins):
+        host[1 + a:1 + a + w.size] = w
+    y = torch.from_numpy(host).cuda()[1:]
+    w1 = w0 + np.array([w.size for w in wins], np.int64)
+    assert w0[0] == 0 and w1[-1] == n_total and y.data_ptr() % 8 == 4
+    return dict(y=y, wins=wins, w0=w0, w1=w1, n_total=n_total, twins={},
+                w0d=torch.from_numpy(w0).cuda(), w1d=torch.from_numpy(w1).cuda())
+
+
+def _twin(t, e, max_iters):
+    key = (e, max_iters)
+    if key not in t["twins"]:
+        t["twins"][key] = tw.fit(t["wins"][e], PAD, TAU0, max_iters=max_iters)
+    return t["twins"][key]
+
+
+def _fit(t, max_iters, max_levels=3):
+    r = stepfit.step_fit_long(t["y"], t["w0d"], t["w1d"], padding=PAD, tau0=TAU0, max_iters=max_iters,
+                              max_levels=max_levels)
+    lv = r.levels
+    return dict(params=r.params.cpu().numpy(), cost=r.cost.cpu().numpy(), iters=r.iters.cpu().numpy(),
+                type=r.status.cpu().numpy(), n_levels=lv.n_levels.cpu().numpy(), edges=lv.edges.cpu().numpy(),
+                mean=lv.mean.cpu().numpy(), std=lv.std.cpu().numpy())
+
+
+def _anorm(x, p, v):
+    xr, x0 = tw.window(x)
+    q = np.array(p, np.float64)
+    q[0] -= x0
+    _, _, A = tw.sums(xr, q)
+    return float(np.sqrt(v @ A @ v))
+
+
+def test_evaluation_pass(trace, record_property):
+    g = _fit(trace, max_iters=1)
+    worst = 0.0
+    for e, x in enumerate(trace["wins"]):
+        f = _twin(trace, e, 1)
+        assert np.allclose(g["params"][e], f.initial, rtol=1e-12, atol=0), (e, x.size, g["params"][e], f.initial)
+        c = tw.cost_at(x, g["params"][e])
+        worst = max(worst, abs(g["cost"][e] - c) / c)
+        # the short kernel's bound; 1.5e-7 measured (NVIDIA B200, 1000 W)
+        assert g["cost"][e] == pytest.approx(c, rel=2e-6), (e, x.size)
+    assert np.all(g["iters"] == 1) and np.all(g["type"] == 7) and np.all(g["n_levels"] == 0) and np.all(g["edges"] == -1)
+    record_property("evaluation_cost_rel_err_max", worst)
+
+
+def test_first_step_follows_the_twin(trace, record_property):
+    g = _fit(trace, max_iters=2)
+    worst_a, worst_c, n_step, n_skip = 0.0, 0.0, 0, 0
+    for e, x in enumerate(trace["wins"]):
+        f = _twin(trace, e, 2)
+        if _tie(f, accept=1e-4):
+            n_skip += 1
+            continue
+        st = f.steps[0]
+        assert g["iters"][e] == f.iters, (e, x.size, st.kind)
+        d = g["params"][e] - f.initial
+        if st.kind != "accept":
+            assert np.array_equal(g["params"][e], f.initial), (e, x.size, st.kind)
+            continue
+        n_step += 1
+        ea = _anorm(x, f.initial, d - st.d) / _anorm(x, f.initial, st.d)
+        ec = float(np.max(np.abs(d - st.d) / np.abs(st.d)))
+        worst_a, worst_c = max(worst_a, ea), max(worst_c, ec)
+        assert ea <= 2e-5 and ec <= 1e-3, (e, x.size, d, st.d)                     # 8.1e-6 and 7.6e-5 measured
+    assert n_step >= 0.8 * len(trace["wins"]) and n_skip <= 0.1 * len(trace["wins"])
+    record_property("first_step_anorm_rel_err_max", worst_a)
+    record_property("first_step_component_rel_err_max", worst_c)
+
+
+@pytest.mark.parametrize("K", [3, 5, 8])
+def test_first_trials_follow_the_twin(trace, K, record_property):
+    g = _fit(trace, max_iters=K)
+    worst, n_cmp = 0.0, 0
+    for e, x in enumerate(trace["wins"]):
+        f = _twin(trace, e, K)
+        if _tie(f):
+            continue
+        n_cmp += 1
+        assert g["iters"][e] == f.iters, (e, x.size, [s.kind for s in f.steps])
+        moved = f.params - f.initial
+        if not np.any(moved):
+            assert np.array_equal(g["params"][e], f.initial), (e, x.size)
+            continue
+        err = _anorm(x, f.params, g["params"][e] - f.params) / _anorm(x, f.params, moved)
+        worst = max(worst, err)
+        assert err <= 3e-5, (e, x.size, g["params"][e], f.params)                   # 6.2e-6 measured (K = 3)
+    assert n_cmp >= 0.7 * len(trace["wins"])
+    record_property(f"trials{K}_anorm_rel_err_max", worst)
+
+
+def test_full_fits_at_every_window_size(trace, record_property):
+    g = _fit(trace, max_iters=stepfit.DEFAULT_MAX_ITERS)
+    worst_cost, worst_dc, worst_move, worst_sd, n_valid = 0.0, 0.0, 0.0, 0.0, 0
+    for e, x in enumerate(trace["wins"]):
+        assert g["type"][e] in (1, 7)
+        c = tw.cost_at(x, g["params"][e])
+        worst_cost = max(worst_cost, abs(g["cost"][e] - c) / c)
+        f = _twin(trace, e, stepfit.DEFAULT_MAX_ITERS)
+        if not _tie(f, valid=1e-6):
+            assert g["type"][e] == f.type, (e, x.size)
+        if g["type"][e] != 1:
+            assert g["n_levels"][e] == 0 and np.all(g["edges"][e] == -1)
+            continue
+        n_valid += 1
+        dc, move = tw.local_minimum_gap(x, g["params"][e])
+        worst_dc, worst_move = max(worst_dc, dc), max(worst_move, move)
+        # 0.02 se for the short kernel; here 0.022 measured (an 83 k-sample window: its standard errors are small
+        # against the float32 stop floor n (2^-24 max|x - x0|)^2, which grows with n)
+        assert dc <= 1e-6 and move <= 0.05, (e, x.size, dc, move)
+        edges, mean, std = so.level_rows(x, g["params"][e])
+        assert g["n_levels"][e] == 3 and np.array_equal(g["edges"][e, :4], edges)
+        assert np.allclose(g["mean"][e, :3], mean, rtol=1e-12, atol=0)
+        sd_err = float(np.max(np.abs(g["std"][e, :3] - std) / std))
+        worst_sd = max(worst_sd, sd_err)
+        assert sd_err <= 5e-6, (e, x.size, g["std"][e, :3], std)                   # 4.1e-7 measured
+    assert worst_cost <= 5e-6, worst_cost                                  # 1.1e-7 measured
+    assert n_valid >= 0.85 * len(trace["wins"])
+    record_property("full_cost_rel_err_max", worst_cost)
+    record_property("full_lm_cost_decrease_max", worst_dc)
+    record_property("full_lm_move_se_max", worst_move)
+    record_property("full_level_std_rel_err_max", worst_sd)
+
+
+SENT_F, SENT_I = -3.25, 777
+
+
+def _contract_rows(t):
+    """(w0, w1, type) of 48 rows and the count 32: long-fit rows, rows of other types, rejected windows, and rows at
+    or beyond the count."""
+    w0, w1, n = list(t["w0"]), list(t["w1"]), t["n_total"]
+    rows = [(w0[i], w1[i], LONG) for i in (0, 1, 4, 5, 7, 10, 12, 15, 17)]
+    rows += [(w0[i], w1[i], k) for i, k in zip((2, 3, 6, 8, 9, 11), (0, 1, 2, 5, 6, 7))]     # not type 8: untouched
+    rows += [(-1, w1[3], LONG), (w0[5], n + 1, LONG), (100, 100 + 2 * PAD, LONG), (100, 100 + 2 * PAD - 7, LONG),
+             (100, 100, LONG), (0, stepfit.LONG_MAX_WINDOW + 1, LONG), (0, 1 << 20, LONG)]   # rejected windows
+    while len(rows) < 32:
+        i = len(rows) % len(w0)
+        rows.append((w0[i], w1[i], LONG))
+    rows += [(w0[i], w1[i], LONG) for i in range(16)]                                        # beyond the count
+    return (np.array([r[0] for r in rows], np.int64), np.array([r[1] for r in rows], np.int64),
+            np.array([r[2] for r in rows], np.int32), 32)
+
+
+def _launch_sentinel(t, max_levels, w0, w1, typ, count):
+    dev = t["y"].device
+    cap = w0.size
+    types = torch.from_numpy(typ.copy()).to(dev)
+    out = {"params": torch.full((cap, 6), SENT_F, dtype=torch.float64, device=dev),
+           "cost": torch.full((cap,), SENT_F, dtype=torch.float64, device=dev),
+           "iters": torch.full((cap,), SENT_I, dtype=torch.int32, device=dev)}
+    lv = {"n_levels": torch.full((cap,), SENT_I, dtype=torch.int32, device=dev),
+          "edges": torch.full((cap, max_levels + 1), SENT_I, dtype=torch.int32, device=dev),
+          "mean": torch.full((cap, max_levels), SENT_F, dtype=torch.float64, device=dev),
+          "std": torch.full((cap, max_levels), SENT_F, dtype=torch.float64, device=dev)}
+    stepfit.launch_long(t["y"], torch.from_numpy(w0).to(dev), torch.from_numpy(w1).to(dev), types, out, lv, padding=PAD,
+                        tau0=TAU0, n_events_dev=torch.tensor([count], dtype=torch.int64, device=dev), capacity=cap)
+    res = {k: v.cpu().numpy() for k, v in {**out, **lv}.items()}
+    res["type"] = types.cpu().numpy()
+    return res
+
+
+def test_row_contract(trace):
+    t = trace
+    w0, w1, typ, count = _contract_rows(t)
+    base = None
+    for ml in (3, 16):
+        g = _launch_sentinel(t, ml, w0, w1, typ, count)
+        below = np.arange(w0.size) < count
+        untouched = ~below | (typ != LONG)           # rows at or beyond the count, rows of other types
+        for k in ("params", "cost", "mean", "std"):
+            assert np.all(g[k][untouched] == SENT_F), k
+        for k in ("iters", "n_levels", "edges"):
+            assert np.all(g[k][untouched] == SENT_I), k
+        assert np.array_equal(g["type"][untouched], typ[untouched])
+        n = w1 - w0
+        rej = below & (typ == LONG) & ((w0 < 0) | (w1 > t["n_total"]) | (n <= 2 * PAD) | (n > stepfit.LONG_MAX_WINDOW))
+        assert rej.sum() == 7
+        assert np.all(g["type"][rej] == 7) and np.all(g["n_levels"][rej] == 0) and np.all(g["edges"][rej] == -1)
+        assert np.all(g["params"][rej] == 0) and np.all(g["cost"][rej] == 0) and np.all(g["iters"][rej] == 0)
+        assert np.all(g["mean"][rej] == SENT_F) and np.all(g["std"][rej] == SENT_F)
+        fit = below & (typ == LONG) & ~rej
+        ok, bad = fit & (g["type"] == 1), fit & (g["type"] == 7)
+        assert ok.sum() >= 10 and np.all(np.isin(g["type"][fit], (1, 7)))
+        assert np.all(g["n_levels"][ok] == 3) and np.all(g["edges"][ok, 4:] == -1)
+        assert np.all(g["mean"][ok, 3:] == SENT_F) and np.all(g["std"][ok, 3:] == SENT_F)
+        assert np.all(g["n_levels"][bad] == 0) and np.all(g["edges"][bad] == -1) and np.all(g["mean"][bad] == SENT_F)
+        assert np.all(g["iters"][fit] >= 1) and np.all(g["cost"][fit] > 0)
+        rows = {k: g[k] for k in ("params", "cost", "iters", "type", "n_levels")}
+        rows.update(edges=g["edges"][:, :4], mean=g["mean"][:, :3], std=g["std"][:, :3])
+        if base is None:
+            base = rows
+        for k in rows:
+            assert np.array_equal(rows[k], base[k]), (ml, k)
+
+
+def test_fallback_select_contract():
+    ty, nl, ov, wl = np.meshgrid(np.arange(8), np.arange(5), np.arange(2), np.array([8192, 8193]), indexing="ij")
+    ty, nl, ov, wl = (v.ravel() for v in (ty, nl, ov, wl))
+    count = ty.size
+    extra = 24                                               # rows beyond the count: type 0, no levels, long window
+    ty = np.concatenate((ty, np.zeros(extra, np.int64))).astype(np.int32)
+    nl = np.concatenate((nl, np.zeros(extra, np.int64))).astype(np.int32)
+    ov = np.concatenate((ov, np.zeros(extra, np.int64))).astype(np.uint8)
+    wl = np.concatenate((wl, np.full(extra, 20_000)))
+    w0 = np.arange(ty.size, dtype=np.int64) * 200_000
+    w1 = w0 + wl
+    types = torch.from_numpy(ty.copy()).cuda()
+    stepfit.select_fallback({"n_levels": torch.from_numpy(nl).cuda(), "overflow": torch.from_numpy(ov).cuda()},
+                            torch.from_numpy(w0).cuda(), torch.from_numpy(w1).cuda(), types,
+                            n_events_dev=torch.tensor([count], dtype=torch.int64, device="cuda"))
+    got = types.cpu().numpy()
+    want = ty.copy()
+    sel = (np.arange(ty.size) < count) & (ty == 0) & (ov == 0) & (nl < 3)
+    want[sel] = np.where(wl[sel] <= stepfit.MAX_WINDOW, 1, LONG)
+    assert np.array_equal(got, want)
+    assert np.count_nonzero(got != ty) == 6                 # type 0, no overflow: n_levels 0 / 1 / 2 x two windows
+
+
+# ---- the pipeline -------------------------------------------------------------------------------------------------
+S = synth.CHIMERA_SETTINGS
+SHALLOW = -180.0                        # below delta / 2 = 200 pA, 9 sigma of the filtered noise (20.5 pA)
+SHALLOW_LENGTHS = (9000, 20_000, 45_000, 90_000)
+PULSE = ((-1000.0, 100),)
+# baseline blocks only from samples within 5 sigma of the baseline: the shallow events must not shift it
+KW = dict(threshold=5.0, hysteresis=1.0, baseline_block=1 << 16, baseline_min=4900.0, baseline_max=5100.0,
+          cusum_h=10.0, stepfit_samples=500)
+
+
+def _mixed_trace(n=16_777_216, seed=300):
+    tpl = []
+    for L in SHALLOW_LENGTHS:
+        tpl += [synth.EVENT_LEVELS, PULSE, ((SHALLOW, L),)]
+    return synth.device_trace(n, "cuda:0", seed=seed, events_per_s=40.0, levels=tpl)
+
+
+def _final_types(h):
+    """ct_event_columns' type rule: 6 level overflow, 5 fewer than three levels, for the types 0 and 1."""
+    t = h["types"].astype(np.int64).copy()
+    fit = np.isin(t, (0, 1))
+    t[fit & (h["overflow"] != 0)] = 6
+    t[fit & (h["overflow"] == 0) & (h["n_levels"] < 3)] = 5
+    return t
+
+
+def _run_host(codes, **kw):
+    an = pipeline.TraceAnalyzer(codes.numel(), S, 1e5, 8, device="cuda:0", **{**KW, **kw})
+    r = an.run(codes)
+    h = {k: v.copy() for k, v in an.tables_to_host(r).items()}
+    return an, r, h
+
+
+@pytest.fixture(scope="module")
+def mixed():
+    codes = _mixed_trace()
+    runs = {}
+    for fb in (False, True):
+        runs[fb] = _run_host(codes, cusum_delta=400.0, stepfit_fallback=fb)
+    return codes, runs
+
+
+def test_pipeline_fallback_fits_the_shallow_events(mixed, record_property):
+    _, runs = mixed
+    h_off, h_on = runs[False][2], runs[True][2]
+    assert np.array_equal(h_off["starts"], h_on["starts"]) and np.array_equal(h_off["ends"], h_on["ends"])
+    length = h_off["ends"] - h_off["starts"]
+    shallow = length > 5000
+    assert shallow.sum() >= 40
+    t_off, t_on = _final_types(h_off), _final_types(h_on)
+    assert np.all(t_off[shallow] == 5)                       # the premise: CUSUM+ finds no sub-level in them
+    assert not np.any(h_on["types"] == LONG) and not np.any(h_off["types"] == LONG)
+    assert np.all(np.isin(t_on[shallow], (1, 7))) and np.mean(t_on[shallow] == 1) >= 0.95
+    ok = shallow & (t_on == 1)
+    depth = h_on["mean"][ok, 0] - h_on["mean"][ok, 1]
+    err = np.abs(depth - abs(SHALLOW)) / abs(SHALLOW)
+    assert np.median(err) <= 0.07, np.median(err)          # 0.049 measured: i0 rests on 2 x 100 baseline samples
+    record_property("shallow_type1_fraction", float(np.mean(t_on[shallow] == 1)))
+    record_property("shallow_depth_rel_err_median", float(np.median(err)))
+    # every other event: bit-equal rows
+    other = ~shallow
+    assert other.sum() >= 80
+    assert np.array_equal(t_on[other], t_off[other])
+    for k in ("types", "n_levels", "edges", "overflow", "stepfit_params", "stepfit_cost", "stepfit_iters"):
+        assert np.array_equal(h_on[k][other], h_off[k][other]), k
+    nl = h_off["n_levels"]
+    written = np.arange(h_off["mean"].shape[1])[None, :] < nl[:, None]
+    for k in ("mean", "std"):
+        assert np.array_equal(h_on[k][other][written[other]], h_off[k][other][written[other]]), k
+
+
+def test_pipeline_fallback_on_the_c2_template(record_property):
+    """Two-level events (the C2 template): CUSUM+ segments nearly all of them, and every event it segments keeps its
+    rows bit for bit; the few it leaves without a sub-level are fitted."""
+    codes = synth.device_trace(4_194_304, "cuda:0", seed=301)
+    kw = dict(baseline_min=4700.0, baseline_max=5300.0, stepfit_samples=0, cusum_delta=400.0)
+    _, r0, h0 = _run_host(codes, **kw)
+    _, r1, h1 = _run_host(codes, stepfit_fallback=True, **kw)
+    assert r0.stepfit is None and r1.stepfit is not None
+    t0 = _final_types(h0)
+    five = t0 == 5
+    record_property("c2_type5_events", int(five.sum()))
+    assert np.count_nonzero(t0 == 0) > 900 and five.sum() <= 0.01 * five.size
+    assert np.all(np.isin(h1["types"][five], (1, 7))) and not np.any(h1["types"] == LONG)
+    keep = ~five
+    nl = h0["n_levels"]
+    written = (np.arange(h0["mean"].shape[1])[None, :] < nl[:, None]) & keep[:, None]
+    for k in h0:
+        if k in ("mean", "std"):
+            assert np.array_equal(h0[k][written], h1[k][written]), k
+        else:
+            assert np.array_equal(h0[k][keep], h1[k][keep]), k
+    assert np.all(h1["stepfit_params"][keep] == 0) and np.all(h1["stepfit_iters"][keep] == 0)
+    assert torch.equal(r0.filtered, r1.filtered)
+
+
+def test_pipeline_fallback_without_cusum_fits_every_accepted_event(mixed):
+    codes, runs = mixed
+    h_ref = runs[False][2]
+    _, _, h = _run_host(codes, cusum_delta=None, stepfit_fallback=True)
+    accepted = np.isin(h_ref["types"], (0, 1))               # types 0 / 1 before ct_event_columns
+    assert np.array_equal(h["starts"], h_ref["starts"])
+    assert np.all(np.isin(h["types"][accepted], (1, 7))) and np.array_equal(h["types"][~accepted], h_ref["types"][~accepted])
+    assert np.mean(h["types"][accepted] == 1) >= 0.5           # 0.75 measured: the two-level events fit one level
+
+
+def test_streamed_form_equals_trace_analyzer(mixed):
+    codes, runs = mixed
+    h = runs[True][2]
+    san = pipeline.StreamingAnalyzer(codes.numel(), S, 1e5, 8, shards=3, first_blocks=2, device="cuda:0",
+                                     cusum_delta=400.0, stepfit_fallback=True, **KW)
+    t = san.run_from_host(codes.cpu().pin_memory()).tables
+    assert np.array_equal(t["starts"], h["starts"])
+    # a fit near the validity rule may end 1 in one form and 7 in the other (the samples differ in the last bits)
+    fitted = np.isin(h["types"], (1, 7))
+    assert np.array_equal(t["types"][~fitted], h["types"][~fitted]) and np.all(np.isin(t["types"][fitted], (1, 7)))
+    assert np.mean(t["types"][fitted] == h["types"][fitted]) >= 0.9
+    fit = (h["types"] == 1) & (t["types"] == 1)
+    dp = np.abs(t["stepfit_params"][fit] - h["stepfit_params"][fit])
+    # sub-shards differ from the whole trace by the IIR warm-up error only; on windows of 9 000 - 90 000 samples and up
+    # to 200 LM trials that moves the end point along the flat u / tau directions by up to 0.063 samples (measured)
+    assert np.percentile(dp[:, 1], 99) < 0.5 and np.percentile(dp[:, 2:], 99) < 0.2, dp.max(axis=0)
+    assert np.all(t["stepfit_iters"][~np.isin(h["types"], (1, 7))] == 0)
+
+
+def test_writer_lists_the_fallback_events(mixed, tmp_path):
+    _, runs = mixed
+    an, r, h = runs[True]
+    tab = writer.event_table_from_result(an, r, samplerate=FS)
+    length = h["ends"] - h["starts"]
+    ids = [int(r.first_event_id + i) for i in np.nonzero((length > 5000) & (h["types"] == 1))[0][:3]]
+    assert len(ids) == 3
+    samples = writer.gather_event_samples(an, r, ids, tab)
+    bl = r.baseline
+    out = str(tmp_path / "analysis")
+    writer.write_analysis_dir(out, tab, baseline_mean=bl.mean, baseline_std=bl.std, baseline_block=bl.block,
+                              samplerate=FS, threshold=5.0, hysteresis=1.0, cutoff=100000.0, poles=8,
+                              event_samples=samples, stepfit_samples=500, stepfit_fallback=True)
+    ev = pd.read_csv(os.path.join(out, "events.csv"), encoding="utf-8")
+    assert list(ev.columns) == writer.EVENT_COLUMNS
+    fb = ev[ev["id"].isin(ids)]
+    assert len(fb) == 3 and np.all(fb["type"] == 1) and np.all(fb["rc_const1_us"] > 0) and np.all(fb["rc_const2_us"] > 0)
+    assert np.all(fb["n_levels"] == 2)                       # mosaicConverter's count: sub-levels + 1
+    blk = np.array([np.array(a.split(";")[1:-1], dtype=float) for a in fb["blockages_pA"]])
+    assert np.all(np.abs(blk - abs(SHALLOW)) < 30)
+    for eid in ids:                                          # readevents.py:1318-1337: 4 columns for type 1
+        f = pd.read_csv(os.path.join(out, "events", "event_%08d.csv" % eid), encoding="utf-8")
+        f.columns = ["time", "current", "cusum", "stepfit"]
+        assert len(f) == samples[eid][1].size and np.allclose(f["stepfit"].values,
+                                                              stepfit.model(samples[eid][4], len(f)))
+    lines = open(os.path.join(out, "summary.txt")).read().splitlines()
+    assert "stepfit_fallback=1" in lines and "stepfit_samples=500" in lines
+
+
+def test_window_limit_is_checked():
+    with pytest.raises(ValueError, match="fallback"):
+        pipeline.TraceAnalyzer(1 << 22, S, 1e5, 8, device="cuda:0", stepfit_fallback=True,
+                               maxpoints=stepfit.LONG_MAX_WINDOW, **{**KW, "stepfit_samples": 0})
