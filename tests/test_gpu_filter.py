@@ -78,14 +78,28 @@ def test_unaligned_views():
 
 def test_run_length_is_invisible():
     """Runs are filtered independently with an Hw-sample warm-up, and the run length follows the trace
-    length (256 for short traces, 4096 for long ones): the same samples embedded in traces of different
-    lengths must come out the same (away from the ends)."""
+    length (256 for short traces, 4096 for long ones): the same samples embedded in a trace long enough for
+    runs of 2048 samples or more must come out as they do in short traces (away from the ends)."""
+    from cusumtools_b200 import _lib
+    H = filters.warmup_samples(bessel_lowpass(8, 2 * 1e5 / synth.FS))
+
+    def run(n):
+        return int(_lib.lib().ct_filtfilt_stats_granule(n, 1000, H)) // 64
+
+    lo, hi = 1, 1 << 40                  # the shortest trace with runs of 2048 samples (the run length grows with n)
+    while lo < hi:
+        mid = (lo + hi) // 2
+        lo, hi = (lo, mid) if run(mid) >= 2048 else (mid + 1, hi)
     codes, _ = synth.c1_trace(n=6_000_000, n_events=1400, seed=9)
+    raw = synth.device_trace(lo + 12_345, "cuda", seed=9)
+    raw[:codes.size] = torch.from_numpy(codes).cuda()
     med = (40800, 40800)                 # one pad value for all lengths (the median of a prefix is not the trace's)
-    full = gpu_filter(codes, 1e5, 8, median_codes=med)
-    for n in (300_000, 1_500_000):
+    full = filters.dequant_filtfilt(raw, S, 1e5, 8, median_codes=med)
+    assert run(raw.numel()) >= 2048
+    for n in (300_000, 1_500_000, 6_000_000):
+        assert run(n) < run(raw.numel())
         part = gpu_filter(codes[:n].copy(), 1e5, 8, median_codes=med)
-        assert np.abs(part[:n - 5000] - full[:n - 5000]).max() < 0.02
+        assert np.abs(part[:n - 5000] - full[:n - 5000].cpu().numpy()).max() < 0.02
 
 
 @pytest.mark.parametrize("cutoff,want_d", [(5e4, 4), (1e5, 4), (2.5e5, 2), (4e5, 2), (9e5, 1)])
