@@ -13,7 +13,7 @@ import math
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, median
 from .design import BesselDesign, bessel_lowpass
 
 DEFAULT_HALO_EPS = 1e-7      # truncated natural response relative to max |x - median|
@@ -119,55 +119,6 @@ def chimera_affine(settings) -> tuple[float, float]:
     return float((b1 - b0) / 32768.0), float(b0)
 
 
-# ----------------------------------------------------------------------- exact median
-def code_median(raw: torch.Tensor, mask: int = 0xFFFF) -> tuple[int, int]:
-    """The two middle order statistics (equal for odd n) of the masked codes, exactly.
-
-    A strided sample histogram locates the median; an exact counting pass over a window
-    of 8 adjacent codes verifies the ranks (and is repeated if the window missed)."""
-    if raw.dtype not in (torch.uint16, torch.int16):
-        raise TypeError("raw must hold the 16-bit ADC codes (torch.uint16 or the int16 view)")
-    _require_cuda(raw, "raw", raw.dtype)
-    L = _lib.lib()
-    n = raw.numel()
-    if n == 0:
-        raise ValueError("median of an empty trace")
-    shift = 0
-    while shift < 16 and not (mask >> shift) & 1:
-        shift += 1
-    step = 1 << shift
-    k1, k2 = (n - 1) // 2, n // 2
-    st = _stream_ptr(raw)
-
-    def sampled_hist(stride):
-        h = torch.zeros(65536, dtype=torch.int32, device=raw.device)
-        _lib.check(L.ct_hist_sampled_u16(raw.data_ptr(), n, stride, mask, h.data_ptr(), st), "ct_hist_sampled_u16")
-        return h.cpu().numpy().astype(np.int64)
-
-    stride = max(1, n // (1 << 20))
-    hist = sampled_hist(stride)
-    if stride == 1:
-        cdf = np.cumsum(hist)
-        return int(np.searchsorted(cdf, k1 + 1)), int(np.searchsorted(cdf, k2 + 1))
-    cdf = np.cumsum(hist)
-    est = int(np.searchsorted(cdf, (cdf[-1] + 1) // 2))
-    lo = max(0, (est >> shift) * step - 3 * step)
-    for _ in range(6):
-        cnt = torch.zeros(9, dtype=torch.int64, device=raw.device)
-        _lib.check(L.ct_count_window_u16(raw.data_ptr(), n, mask, lo, step, cnt.data_ptr(), st), "ct_count_window_u16")
-        c = cnt.cpu().numpy().astype(np.int64)
-        below, w = int(c[0]), c[1:]
-        cw = below + np.cumsum(w)
-        if below <= k1 and k2 < cw[-1]:
-            i1 = int(np.searchsorted(cw, k1 + 1))
-            i2 = int(np.searchsorted(cw, k2 + 1))
-            return lo + i1 * step, lo + i2 * step
-        lo = max(0, lo - 6 * step) if k1 < below else lo + 6 * step
-    # pathological distribution: exact full histogram
-    cdf = np.cumsum(sampled_hist(1))
-    return int(np.searchsorted(cdf, k1 + 1)), int(np.searchsorted(cdf, k2 + 1))
-
-
 # ------------------------------------------------------------------------ entry points
 def filtfilt_codes(raw: torch.Tensor, *, alpha: float, pad_value: float, median_code: float, mask: int,
                    design: BesselDesign, padding: int = 1000, forward_only: bool = False,
@@ -213,7 +164,7 @@ def dequant_filtfilt(raw: torch.Tensor, settings, cutoff: float, order: int = 8,
     design = bessel_lowpass(int(order), 2.0 * float(cutoff) / fs)
     mask = chimera_bitmask(settings)
     alpha, _ = chimera_affine(settings)
-    c1, c2 = median_codes if median_codes is not None else code_median(raw, mask)
+    c1, c2 = median_codes if median_codes is not None else median.code_median(raw, mask)
     vals = scale_codes_host(np.array([c1, c2], dtype=np.uint16), settings)
     pad_value = float(np.median(vals))
     return filtfilt_codes(raw, alpha=alpha, pad_value=pad_value, median_code=0.5 * (c1 + c2), mask=mask,

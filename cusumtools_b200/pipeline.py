@@ -7,7 +7,7 @@ One process per GPU.  A rank owns the samples [lo, hi) of the global trace and i
 them together with `halo` extra samples on each side (read from the shared file / host
 buffer, not exchanged: SURVEY.md section 8e).  The only collectives are
   * all_reduce(SUM) of the sampled code histogram and of the 9 window counters that give
-    the GLOBAL median pad value (so every rank subtracts the same constant), and
+    the GLOBAL median pad value (median.py: every rank subtracts the same constant), and
   * all_gather of per-rank event counts (global event ids); event rows stay rank-local.
 With `group=None` nothing is communicated and the functions are the single-GPU path.
 """
@@ -19,8 +19,9 @@ from dataclasses import dataclass
 import numpy as np
 import torch
 
-from . import _lib, cusum, detect, filters, stepfit
+from . import _lib, cusum, detect, filters, median, stepfit
 from .design import bessel_lowpass
+from .median import _all_reduce_
 
 
 @dataclass
@@ -32,163 +33,6 @@ class TraceResult:
     median_codes: tuple[int, int]
     first_event_id: int = 0         # global id of this rank's first event
     total_events: int = 0
-
-
-def _world(group) -> int:
-    import torch.distributed as dist
-    return dist.get_world_size(group)
-
-
-def _all_reduce_(t: torch.Tensor, group) -> torch.Tensor:
-    if group is not None:
-        import torch.distributed as dist
-        dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
-    return t
-
-
-@dataclass
-class MedianPlan:
-    """State of the exact-median search between its two phases (estimate, verify)."""
-    n: int                      # samples of all ranks
-    k1: int                     # ranks of the two middle order statistics
-    k2: int
-    step: int                   # spacing of the masked codes
-    shift: int
-    est: int                    # estimated median code (a multiple of step)
-    lo: int                     # first code of the 8-code verification window
-    exact: tuple[int, int] | None = None     # already exact (small traces: full histogram)
-    se: float = float("inf")    # standard error of the estimate in code steps: sqrt(sampled) / (2 x samples at the estimate)
-
-
-def median_estimate(n_local: int, mask: int, hist_fn, group=None, device=None, n_sampled: int | None = None) -> MedianPlan:
-    """Phase 1: a strided-sample histogram (summed over `group`) locates the median code.  `n_sampled`:
-    the histogram covers only that many of the rank's samples (streaming: the first chunk), so it
-    is an estimate even for small traces."""
-    shift = 0
-    while shift < 16 and not (mask >> shift) & 1:
-        shift += 1
-    step = 1 << shift
-    if group is None:
-        n = int(n_local)
-        if n == 0:
-            raise ValueError("median of an empty trace")
-        stride = max(1, (n if n_sampled is None else int(n_sampled)) // (1 << 20))  # ~1 M samples: median s.e. < 0.1 code
-        hist = hist_fn(stride)
-    else:
-        # every rank samples with the stride of ITS share (ranks own equal shares), and the sample count rides in the
-        # same all_reduce as the histogram: one collective for the phase
-        stride = max(1, (int(n_local) if n_sampled is None else int(n_sampled)) * _world(group) // (1 << 20))
-        h = hist_fn(stride).to(torch.int64)
-        packed = _all_reduce_(torch.cat((h, torch.tensor([int(n_local)], dtype=torch.int64, device=h.device))), group)
-        hist, n = packed[:-1], None                        # (the total comes back with the rank search: one read)
-    exact = stride == 1 and n_sampled is None
-    if group is not None and (exact or not hist.is_cuda):
-        n = int(packed[-1].item())
-    if exact:
-        if n == 0:
-            raise ValueError("median of an empty trace")
-        k1, k2 = (n - 1) // 2, n // 2
-        cdf = torch.cumsum(hist.to(torch.int64), 0)
-        want = torch.tensor([k1 + 1, k2 + 1], dtype=torch.int64, device=cdf.device)
-        c1, c2 = (int(v) for v in torch.searchsorted(cdf, want).tolist())
-        return MedianPlan(n, k1, k2, step, shift, c1, max(0, c1 - 3 * step), exact=(c1, c2))
-    # the rank search runs where the histogram lives: 24 (32) bytes come back instead of 65 536 bins
-    if hist.is_cuda and hist.dtype in (torch.int32, torch.int64) and hist.is_contiguous():
-        out = torch.empty(3, dtype=torch.int64, device=hist.device)
-        with torch.cuda.device(hist.device):
-            rc = _lib.lib().ct_hist_rank(hist.data_ptr(), int(hist.dtype == torch.int64), out.data_ptr(),
-                                         C.c_void_p(torch.cuda.current_stream(hist.device).cuda_stream))
-        _lib.check(rc, "ct_hist_rank")
-        vals = (torch.cat((out, packed[-1:])) if n is None else out).tolist()
-        i, dens, total = (int(v) for v in vals[:3])
-        if n is None:
-            n = int(vals[3])
-    else:                                                  # (CPU tensors: the gloo tests of the host logic)
-        hist = hist.to(torch.int64)
-        cdf = torch.cumsum(hist, 0)
-        idx = torch.searchsorted(cdf, (cdf[-1:] + 1) // 2).clamp_(max=hist.numel() - 1)
-        i, dens, total = (int(v) for v in torch.cat((idx, hist[idx], cdf[-1:])).tolist())
-    if n == 0:
-        raise ValueError("median of an empty trace")
-    k1, k2 = (n - 1) // 2, n // 2
-    est = (i >> shift) * step
-    # the sample median of m samples with density f at the median has s.e. 1 / (2 f sqrt(m)); f = dens / m per code step
-    se = 0.5 * float(np.sqrt(max(total, 1))) / max(dens, 1)
-    return MedianPlan(n, k1, k2, step, shift, est, max(0, est - 3 * step), se=se)
-
-
-def median_verify(plan: MedianPlan, counts9, group=None):
-    """Phase 2: the exact counts of the codes below / inside the window (summed over `group`) either pin
-    the two middle order statistics or say which way the window has to move (returns None, new lo)."""
-    c = _all_reduce_(counts9.to(torch.int64), group).cpu().numpy().astype(np.int64)
-    below, cw = int(c[0]), int(c[0]) + np.cumsum(c[1:])
-    if below <= plan.k1 and plan.k2 < cw[-1]:
-        return (plan.lo + int(np.searchsorted(cw, plan.k1 + 1)) * plan.step,
-                plan.lo + int(np.searchsorted(cw, plan.k2 + 1)) * plan.step), plan.lo
-    return None, (max(0, plan.lo - 6 * plan.step) if plan.k1 < below else plan.lo + 6 * plan.step)
-
-
-def median_search(n_local: int, mask: int, hist_fn, count_fn, group=None, device=None, plan: MedianPlan | None = None,
-                  first_counts=None) -> tuple[int, int]:
-    """Host side of the exact global median: the two middle order statistics of the masked
-    codes of ALL ranks.  `hist_fn(stride)` returns this rank's strided-sample histogram
-    (int tensor[65536]) and `count_fn(lo, step)` its 9 window counters (#codes < lo, then
-    #codes == lo + i*step); both are summed over `group` here, so every rank takes the same
-    decisions and returns the same pair.  (The device kernels are passed in, which is what
-    lets the world-size-2 gloo test drive this logic on CPU.)  `plan` / `first_counts`: an
-    estimate already made and the window counts a fused kernel already produced for it."""
-    if plan is None:
-        plan = median_estimate(n_local, mask, hist_fn, group, device)
-    if plan.exact is not None:
-        return plan.exact
-    counts = first_counts
-    for attempt in range(16):
-        if counts is None:
-            counts = count_fn(plan.lo, plan.step)
-        pair, plan.lo = median_verify(plan, counts, group)
-        if pair is not None:
-            return pair
-        if attempt == 0:
-            # the window missed: the estimate came from too small or too local a sample (streaming: the first
-            # piece of a drifting trace).  Re-estimate from a strided histogram of ALL the data before stepping.
-            again = median_estimate(n_local, mask, hist_fn, group, device)
-            if again.exact is not None:
-                return again.exact
-            plan.lo = again.lo                 # (plan.est stays: the filter has already subtracted it)
-        counts = None
-    cdf = np.cumsum(_all_reduce_(hist_fn(1).to(torch.int64), group).cpu().numpy())   # pathological distribution
-    return int(np.searchsorted(cdf, plan.k1 + 1)), int(np.searchsorted(cdf, plan.k2 + 1))
-
-
-def _median_kernels(raw_owned: torch.Tensor, mask: int):
-    """(hist_fn, count_fn) over this rank's owned codes."""
-    L = _lib.lib()
-    dev = raw_owned.device
-    n_local = raw_owned.numel()
-    st = filters._stream_ptr(raw_owned)
-
-    def hist_fn(stride):
-        h = torch.zeros(65536, dtype=torch.int32, device=dev)
-        if n_local:
-            _lib.check(L.ct_hist_sampled_u16(raw_owned.data_ptr(), n_local, stride, mask, h.data_ptr(), st), "ct_hist_sampled_u16")
-        return h
-
-    def count_fn(lo, step):
-        cnt = torch.zeros(9, dtype=torch.int64, device=dev)
-        if n_local:
-            _lib.check(L.ct_count_window_u16(raw_owned.data_ptr(), n_local, mask, lo, step, cnt.data_ptr(), st), "ct_count_window_u16")
-        return cnt
-
-    return hist_fn, count_fn
-
-
-def global_code_median(raw_owned: torch.Tensor, mask: int, group=None) -> tuple[int, int]:
-    """Exact median (two middle order statistics) of the masked codes of the WHOLE trace
-    when each rank passes its owned samples; identical to filters.code_median for one rank."""
-    if group is None:
-        return filters.code_median(raw_owned, mask)
-    hist_fn, count_fn = _median_kernels(raw_owned, mask)
-    return median_search(raw_owned.numel(), mask, hist_fn, count_fn, group, raw_owned.device)
 
 
 def event_id_offsets(n_local_events: int, group=None, device=None) -> tuple[int, int]:
@@ -402,16 +246,16 @@ class TraceAnalyzer:
         st = filters._stream_ptr(raw_ext)
         cur = torch.cuda.current_stream(self.device)
         # ---- median, phase 1: estimate (subtraction constant of the filter, verification window)
-        hist_fn, count_fn = _median_kernels(owned, self.mask)
+        hist_fn, count_fn = median.device_counters(owned, self.mask)
         if _fixed is not None:
             plan = _fixed[0]
         elif _arrivals is None:
-            plan = median_estimate(n_own, self.mask, hist_fn, self.group, self.device)
+            plan = median.estimate(n_own, self.mask, hist_fn, self.group)
         else:                                                  # only the first chunk has arrived: estimate from it
             bounds, events = _arrivals
             cur.wait_event(events[0])
             first = raw_ext[lo:max(lo + 1, min(bounds[1], lo + n_own))]
-            plan = median_estimate(n_own, self.mask, _median_kernels(first, self.mask)[0], self.group, self.device,
+            plan = median.estimate(n_own, self.mask, median.device_counters(first, self.mask)[0], self.group,
                                    n_sampled=first.numel())
         hook("median")
         if self.filter_ws is None:
@@ -423,55 +267,37 @@ class TraceAnalyzer:
         alpha, _ = filters.chimera_affine(self.settings)
         origin = 0
         # ---- forward pass with the estimate; it tallies the window counts of the owned codes on the side
-        counts = torch.zeros(9, dtype=torch.int64, device=self.device) if _fixed is None else None
-        fused = plan.exact is None and _fixed is None
+        route = median.route(plan, fixed=_fixed is not None, streamed=_arrivals is not None, fused_count=self.fused_count)
+        plan.lo = route.lo
+        counts = torch.zeros(9, dtype=torch.int64, device=self.device) if route.count else None
         pieces = [(0, 0, self.n_ext)] if _arrivals is None else [(2, a, b) for a, b in zip(_arrivals[0][:-1], _arrivals[0][1:])]
         pad_first = float(_fixed[1]) if _fixed is not None else 0.0
-        # The estimate of a resident trace comes from a sample of ALL of it, on every rank the same; its standard error
-        # follows from the density at the estimate (MedianPlan.se, in code steps).  Up to 0.8 the eight-code window
-        # est - 3 .. est + 4 holds the median (4 sigma) and is verified on the device; the tally rides on the forward pass
-        # (4.1 instructions per code) or runs as its own kernel (four codes est - 1 .. est + 2 when se <= 0.25).  Beyond
-        # that - a drifting baseline - or from a partial trace (streaming): the host loop.
-        device_ok = fused and _arrivals is None and plan.se <= 0.8
-        ride = device_ok and self.fused_count and plan.step <= 4
-        narrow = device_ok and not ride and plan.se <= 0.25
-        nbins = 4 if narrow else 8
-        if narrow:
-            plan.lo = max(0, plan.est - plan.step)
         for i, (part, a, b) in enumerate(pieces):
             if _arrivals is not None:
                 cur.wait_event(_arrivals[1][i])
             rc = L.ct_filter_forward_u16(raw_ext.data_ptr(), self.n_ext, self.padding, float(plan.est), self.mask, pad_first,
                                          C.byref(coef), self.H, origin, part, plan.lo, plan.step, lo, lo + n_own,
-                                         counts.data_ptr() if ride else None, a, b,
+                                         counts.data_ptr() if route.count == "ride" else None, a, b,
                                          self.filter_ws.data_ptr(), self.filter_ws.numel(), st)
             _lib.check(rc, "ct_filter_forward_u16")
-            if fused and not ride:                 # the window count of this piece's owned codes as its own kernel
-                ca, cb = max(a, lo), min(b, lo + n_own)
-                if cb > ca:
-                    count = L.ct_count_window4_u16 if narrow else L.ct_count_window_u16
-                    rc = count(raw_ext[ca:cb].data_ptr(), cb - ca, self.mask, plan.lo, plan.step, counts.data_ptr(), st)
-                    _lib.check(rc, "ct_count_window_u16")
+            if route.count == "kernel":            # the window count of this piece's owned codes as its own kernel
+                median.count_window(raw_ext[max(a, lo):min(b, lo + n_own)], self.mask, plan.lo, plan.step, counts, route.nbins)
         # everything the backward launch needs that does not depend on the exact median is prepared BEFORE the host waits
         # for the counts: the GPU idles from the end of the forward pass to the backward launch
         bl = detect.new_baseline(self.n_det, self.block, self.bmin, self.bmax, self.device) if self.fuse_stats else None
         stats = detect.stats_args(bl, origin=0) if bl is not None else None
         offset = float(filters.scale_codes_host(np.array([plan.est], dtype=np.uint16), self.settings)[0])
         # ---- median, phase 2: exact order statistics
-        on_device = device_ok and not _host_median
+        on_device = route.device and not _host_median
         self.last_median_route = "device" if on_device else ("host after a device miss" if _host_median else "host")
         if on_device:
             # no host round trip between the passes: one thread turns the (summed) counts into the two middle codes and the
             # pad of the filter ends, the end groups re-run with it (their CTAs return at once when the estimate was the
             # median), and the backward pass follows; the codes reach the host with the step's one synchronisation.  If
             # the window missed them (status != 0) the step is redone the host-driven way.
-            _all_reduce_(counts, self.group)
-            res = self.median_result
-            rc = L.ct_median_verify(counts.data_ptr(), nbins, plan.k1, plan.k2, plan.lo, plan.step, float(plan.est),
-                                    res.data_ptr(), st)
-            _lib.check(rc, "ct_median_verify")
+            median.verify_on_device(plan, counts, route.nbins, self.median_result, self.group)
             rc = L.ct_filter_forward_ends_u16(raw_ext.data_ptr(), self.n_ext, self.padding, float(plan.est), self.mask,
-                                              res[2:].data_ptr(), C.byref(coef), self.H, origin,
+                                              self.median_result[2:].data_ptr(), C.byref(coef), self.H, origin,
                                               self.filter_ws.data_ptr(), self.filter_ws.numel(), st)
             _lib.check(rc, "ct_filter_forward_ends_u16")
             c1 = c2 = None
@@ -479,8 +305,7 @@ class TraceAnalyzer:
             if _fixed is not None:
                 c1, c2 = _fixed[2]
             else:
-                c1, c2 = median_search(n_own, self.mask, hist_fn, count_fn, self.group, self.device, plan=plan,
-                                       first_counts=counts if fused else None)
+                c1, c2 = median.search(n_own, self.mask, hist_fn, count_fn, self.group, plan=plan, first_counts=counts)
             pad_x = 0.5 * (c1 + c2) - plan.est if _fixed is None else 0.0
             if pad_x != 0.0:        # the pad holds median - estimate: redo the groups at the two ends of the trace
                 rc = L.ct_filter_forward_u16(raw_ext.data_ptr(), self.n_ext, self.padding, float(plan.est), self.mask,
@@ -787,7 +612,7 @@ class StreamingAnalyzer:
             self._pin[name] = t = new
         return t
 
-    def _process(self, i: int, plan: MedianPlan, pad_x: float, med: tuple[int, int], row0: int, bl: detect.Baseline,
+    def _process(self, i: int, plan: median.MedianPlan, pad_x: float, med: tuple[int, int], row0: int, bl: detect.Baseline,
                  end_at: int | None = None) -> int:
         """Analyse sub-shard i (its data must be resident), store its owned samples, blocks and table rows
         (from row `row0`, or ending at row `end_at`); returns its event count (-1: more rows than `end_at`)."""
@@ -836,8 +661,7 @@ class StreamingAnalyzer:
     def _run_stream(self, feed, dtype) -> StreamResult:
         if self.raw_dev is None or self.raw_dev.dtype != dtype:
             self.raw_dev = torch.empty(self.n_ext, dtype=dtype, device=self.device)
-        L = _lib.lib()
-        cur = torch.cuda.current_stream(self.device)
+        cur =torch.cuda.current_stream(self.device)
         a0, b_end = self.lo_halo, self.lo_halo + self.n_own
         # ---- the copy, cut where each sub-shard's extended range is complete
         ends = [eb for (_, _, _, eb) in self.sub]
@@ -848,21 +672,20 @@ class StreamingAnalyzer:
             prev = max(prev, e)
         feed.start(self, arrivals, cur)
         try:
-            return self._consume(feed, arrivals, L, cur, a0, b_end)
+            return self._consume(feed, arrivals, cur, a0, b_end)
         finally:
             feed.finish()
 
-    def _consume(self, feed, arrivals, L, cur, a0, b_end) -> StreamResult:
+    def _consume(self, feed, arrivals, cur, a0, b_end) -> StreamResult:
         # ---- median estimate from the first piece
         feed.wait(0, cur)
         first = self.raw_dev[a0:max(a0 + 1, min(arrivals[0][1], b_end))]
-        plan = median_estimate(self.n_own, self.mask, _median_kernels(first, self.mask)[0], self.group, self.device,
+        plan = median.estimate(self.n_own, self.mask, median.device_counters(first, self.mask)[0], self.group,
                                n_sampled=first.numel())
         self.last_plan = plan
         counts = torch.zeros(9, dtype=torch.int64, device=self.device)
-        hist_fn, count_fn = _median_kernels(self.raw_dev[a0:b_end], self.mask)
+        hist_fn, count_fn = median.device_counters(self.raw_dev[a0:b_end], self.mask)
         bl = detect.new_baseline(self.n_own, self.block, self.bmin, self.bmax, self.device)
-        st = filters._stream_ptr(self.raw_dev)
         # The first sub-shard holds the true start of the trace, whose pad needs the exact median: it is analysed
         # with the estimate right away and again at the end if the estimate was off.  Its rows sit RIGHT-ALIGNED
         # in a reserved head of the tables, so a different event count the second time moves nothing else.
@@ -887,14 +710,11 @@ class StreamingAnalyzer:
 
         for i, (pa, pe) in enumerate(arrivals):
             feed.wait(i, cur)
-            ca, cb = max(pa, a0), min(pe, b_end)
-            if plan.exact is None and cb > ca:           # exact-median window count of this piece's owned codes
-                rc = L.ct_count_window_u16(self.raw_dev[ca:cb].data_ptr(), cb - ca, self.mask, plan.lo, plan.step,
-                                           counts.data_ptr(), st)
-                _lib.check(rc, "ct_count_window_u16")
+            if plan.exact is None:                        # exact-median window count of this piece's owned codes
+                median.count_window(self.raw_dev[max(pa, a0):min(pe, b_end)], self.mask, plan.lo, plan.step, counts)
             last = i == len(arrivals) - 1
             if last:                                      # everything has arrived: exact order statistics
-                med = median_search(self.n_own, self.mask, hist_fn, count_fn, self.group, self.device, plan=plan,
+                med = median.search(self.n_own, self.mask, hist_fn, count_fn, self.group, plan=plan,
                                     first_counts=counts if plan.exact is None else None)
                 pad_x = 0.5 * (med[0] + med[1]) - plan.est
             if failed:

@@ -12,7 +12,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import torch
 
-from cusumtools_b200 import _lib, detect, filters, synth
+from cusumtools_b200 import _lib, detect, filters, median, synth
 from cusumtools_b200.design import bessel_lowpass
 
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 2_499_999_600
@@ -44,7 +44,7 @@ def report(name, ms, bytes_per_sample):
           f"= {bytes_per_sample * n / ms / 1e6 / PEAK:.3f} of {PEAK:.0f}", flush=True)
 
 
-c1, c2 = filters.code_median(raw, mask)
+c1, c2 = median.code_median(raw, mask)
 est = float(c1)
 offset = float(filters.scale_codes_host(np.array([c1], dtype=np.uint16), S)[0])
 for cutoff in cutoffs:

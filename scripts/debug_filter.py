@@ -1,7 +1,7 @@
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
-from cusumtools_b200 import filters, synth
+from cusumtools_b200 import filters, median, synth
 from oracle import trace_oracle as to
 S = synth.CHIMERA_SETTINGS
 for n, ne in ((300000, 70), (24001, 5), (5000, 1)):
@@ -9,7 +9,7 @@ for n, ne in ((300000, 70), (24001, 5), (5000, 1)):
     want = to.filter_data(to.scale_raw_data(codes, S), synth.FS, 1e5, 8)
     raw = torch.from_numpy(codes).cuda()
     mask = filters.chimera_bitmask(S)
-    c1, c2 = filters.code_median(raw, mask)
+    c1, c2 = median.code_median(raw, mask)
     srt = np.sort(codes & mask)
     print("n", n, "median codes", c1, c2, "true", srt[(n - 1) // 2], srt[n // 2])
     y = filters.dequant_filtfilt(raw, S, 1e5, 8).cpu().numpy()

@@ -3,7 +3,7 @@ another launch of the same kind / in a long loop?).  Tuning experiment."""
 import ctypes as C, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
-from cusumtools_b200 import _lib, detect, filters, synth
+from cusumtools_b200 import _lib, detect, filters, median, synth
 from cusumtools_b200.design import bessel_lowpass
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 2_499_999_600
 S = synth.CHIMERA_SETTINGS; L = _lib.lib()
@@ -15,7 +15,7 @@ d = bessel_lowpass(8, 2 * 1e5 / synth.FS); coef = filters.make_coef(d); H = filt
 wsb = int(L.ct_filtfilt_workspace_bytes(n, 1000, H)); ws = torch.empty(wsb, dtype=torch.uint8, device="cuda")
 mm = torch.empty(2 * int(L.ct_filter_summary_count(n, 1000, H)), dtype=torch.float32, device="cuda")
 bl = detect.new_baseline(n, 1 << 20, 4700.0, 5300.0, "cuda"); stats = detect.stats_args(bl, origin=0)
-c1, c2 = filters.code_median(raw, mask)
+c1, c2 = median.code_median(raw, mask)
 def fwd(est):
     rc = L.ct_filter_forward_u16(raw.data_ptr(), n, 1000, est, mask, 0.0, C.byref(coef), H, 0, 0, 0, 1, 0, 0, None, 0, 0, ws.data_ptr(), wsb, st); assert rc == 0
 def bwd(est):

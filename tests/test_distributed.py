@@ -11,7 +11,7 @@ import torch
 import torch.distributed as dist
 import torch.multiprocessing as mp
 
-from cusumtools_b200 import pipeline, psd
+from cusumtools_b200 import median, pipeline, psd
 
 
 def _free_port():
@@ -56,7 +56,7 @@ def _median_job(rank, world, group):
         out = [np.sum(c < lo_)] + [np.sum(c == lo_ + i * step) for i in range(8)]
         return torch.tensor(out, dtype=torch.int64)
 
-    return pipeline.median_search(len(codes), mask, hist_fn, count_fn, group)
+    return median.search(len(codes), mask, hist_fn, count_fn, group)
 
 
 def _drift_job(rank, world, group):
@@ -79,8 +79,8 @@ def _drift_job(rank, world, group):
         c = (codes & mask).astype(np.int64)
         return torch.tensor([np.sum(c < lo_)] + [np.sum(c == lo_ + i * step) for i in range(8)], dtype=torch.int64)
 
-    plan = pipeline.median_estimate(len(codes), mask, first_piece_hist, group, None, n_sampled=100_000)
-    pair = pipeline.median_search(len(codes), mask, hist_fn, count_fn, group, plan=plan)
+    plan = median.estimate(len(codes), mask, first_piece_hist, group, n_sampled=100_000)
+    pair = median.search(len(codes), mask, hist_fn, count_fn, group, plan=plan)
     return pair, calls["count"]
 
 
@@ -181,14 +181,14 @@ def test_event_tables_are_gathered_in_rank_order():
 def test_standard_error_of_the_estimate_follows_the_density_at_the_median():
     """MedianPlan.se = sqrt(samples) / (2 x samples at the estimate), in code steps: small for a trace that sits on its
     baseline, large when the median falls where few samples are (a drifting baseline; the tail between two levels) -
-    what decides between the device-verified window and the host loop (pipeline.TraceAnalyzer._run)."""
+    what decides between the device-verified window and the host loop (median.route)."""
     rng = np.random.default_rng(5)
     n, mask = 4_000_000, 0xFFFC
 
     def plan_for(codes):
         def hist_fn(stride):
             return torch.from_numpy(np.bincount(codes[::stride] & mask, minlength=65536).astype(np.int32))
-        return pipeline.median_estimate(len(codes), mask, hist_fn)
+        return median.estimate(len(codes), mask, hist_fn)
 
     quiet = _codes(1, n)
     p = plan_for(quiet)

@@ -11,7 +11,7 @@ import pytest
 import torch
 from scipy.signal import bessel, lfilter, lfilter_zi
 
-from cusumtools_b200 import filters, synth
+from cusumtools_b200 import filters, median, synth
 from cusumtools_b200.design import bessel_lowpass
 from oracle import trace_oracle as to
 
@@ -186,12 +186,12 @@ def test_code_median_is_exact():
     rng = np.random.default_rng(11)
     for n in (1, 2, 1001, 65536, 5_000_001):
         codes = (rng.normal(40000, 60, n).astype(np.int64) & 0xFFFC).astype(np.uint16)
-        c1, c2 = filters.code_median(torch.from_numpy(codes).cuda(), 0xFFFC)
+        c1, c2 = median.code_median(torch.from_numpy(codes).cuda(), 0xFFFC)
         srt = np.sort(codes)
         assert (c1, c2) == (int(srt[(n - 1) // 2]), int(srt[n // 2]))
     # bimodal: the window search must recover when the sample estimate is off
     codes = np.concatenate((np.full(500000, 1000), np.full(500001, 60000))).astype(np.uint16)
-    assert filters.code_median(torch.from_numpy(codes).cuda(), 0xFFFF) == (60000, 60000)
+    assert median.code_median(torch.from_numpy(codes).cuda(), 0xFFFF) == (60000, 60000)
 
 
 def test_large_trace_properties():
@@ -200,7 +200,7 @@ def test_large_trace_properties():
     an interior window."""
     n = 1 << 27
     raw = synth.device_trace(n, "cuda", seed=99)
-    c1, c2 = filters.code_median(raw, filters.chimera_bitmask(S))
+    c1, c2 = median.code_median(raw, filters.chimera_bitmask(S))
     y = filters.dequant_filtfilt(raw, S, 1e5, 8, median_codes=(c1, c2))
     yr = filters.dequant_filtfilt(torch.flip(raw.view(torch.int16), [0]).view(torch.uint16).contiguous(), S, 1e5, 8, median_codes=(c1, c2))
     assert torch.max(torch.abs(torch.flip(yr, [0]) - y)).item() < 0.05
@@ -240,7 +240,7 @@ def test_integration_stub_binds_the_c_abi_directly():
     H = filters.warmup_samples(design)
     mask = filters.chimera_bitmask(S)
     alpha, _ = filters.chimera_affine(S)
-    c1, c2 = filters.code_median(raw, mask)
+    c1, c2 = median.code_median(raw, mask)
     median_code = 0.5 * (c1 + c2)
     pad_value = float(np.median(filters.scale_codes_host(np.array([c1, c2], dtype=np.uint16), S)))
     out = torch.empty(raw.numel(), dtype=torch.float32, device="cuda")

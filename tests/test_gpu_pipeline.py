@@ -431,10 +431,10 @@ def test_device_side_pad_when_the_estimate_is_off_by_two_codes():
 
 
 def test_median_verify_entry_point_against_the_host_logic():
-    """ct_median_verify (one device thread) == pipeline.median_verify (numpy) on random window counts: found / window
+    """ct_median_verify (one device thread) == median.verify (numpy) on random window counts: found / window
     above the median / window below it, four and eight codes, odd and even totals."""
     import ctypes as C
-    from cusumtools_b200 import _lib, filters
+    from cusumtools_b200 import _lib, median
     L = _lib.lib()
     rng = np.random.default_rng(3)
     st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
@@ -449,8 +449,8 @@ def test_median_verify_entry_point_against_the_host_logic():
             continue
         k1, k2 = (n - 1) // 2, n // 2
         lo, step, est = 4000 + 4 * int(rng.integers(0, 50)), 4, 4100.0
-        plan = pipeline.MedianPlan(n, k1, k2, step, 2, int(est), lo)
-        want, _ = pipeline.median_verify(plan, torch.from_numpy(c[:9].copy()))
+        plan = median.MedianPlan(n, k1, k2, step, 2, int(est), lo)
+        want, _ = median.verify(plan, torch.from_numpy(c[:9].copy()))
         if nb == 4 and want is not None and max(want) >= lo + 4 * step:
             want = None                                         # the host logic always looks at eight codes
         dev = torch.from_numpy(c).cuda()
