@@ -5,9 +5,9 @@ The reference has no implementation (it consumes `level_current_pA`, `level_dura
 record: oracle/events_oracle.py (cusum_event / level_stats)."""
 from __future__ import annotations
 
-import ctypes as C
-from dataclasses import dataclass
+from dataclasses import dataclass, fields
 
+import numpy as np
 import torch
 
 from . import _lib
@@ -28,6 +28,29 @@ class LevelTable:
     overflow: torch.Tensor     # uint8 [E]  1 = more jumps than max_levels - 1
     max_levels: int
 
+    @classmethod
+    def empty(cls, rows: int, max_levels: int, device) -> LevelTable:
+        """Uninitialised buffers for `rows` events."""
+        return cls(torch.empty(rows, dtype=torch.int32, device=device),
+                   torch.empty((rows, max_levels + 1), dtype=torch.int32, device=device),
+                   torch.empty((rows, max_levels), dtype=torch.float64, device=device),
+                   torch.empty((rows, max_levels), dtype=torch.float64, device=device),
+                   torch.empty(rows, dtype=torch.uint8, device=device), int(max_levels))
+
+    @classmethod
+    def from_columns(cls, cols: dict, device) -> LevelTable:
+        """The level rows of host event-table columns (pipeline.AnalysisResult.columns: named as the fields) on `device`."""
+        t = [torch.from_numpy(np.ascontiguousarray(cols[f.name])).to(device) for f in fields(cls)[:5]]
+        return cls(*t, int(t[2].shape[1]))         # mean: [E, max_levels]
+
+    def rows(self, n: int) -> LevelTable:
+        """The first `n` rows, as views of these buffers."""
+        return LevelTable(*(getattr(self, f.name)[:n] for f in fields(self)[:5]), self.max_levels)
+
+    def clear(self) -> None:
+        """Every row without levels: n_levels 0, no overflow, edges -1 (mean and std are left as they are)."""
+        self.n_levels.zero_(); self.overflow.zero_(); self.edges.fill_(-1)
+
 
 def cusum_levels(y: torch.Tensor, win_start: torch.Tensor, win_end: torch.Tensor, *, delta: float, h: float,
                  max_levels: int = DEFAULT_MAX_LEVELS, types: torch.Tensor | None = None) -> LevelTable:
@@ -43,21 +66,19 @@ def cusum_levels(y: torch.Tensor, win_start: torch.Tensor, win_end: torch.Tensor
     dev = y.device
     if types is not None:
         _require_cuda(types, "types", torch.int32)
-    nl = torch.zeros(E, dtype=torch.int32, device=dev)
-    ed = torch.empty((E, max_levels + 1), dtype=torch.int32, device=dev)
-    mu = torch.zeros((E, max_levels), dtype=torch.float64, device=dev)
-    sd = torch.zeros((E, max_levels), dtype=torch.float64, device=dev)
-    ov = torch.zeros(E, dtype=torch.uint8, device=dev)
+    lv = LevelTable.empty(E, max_levels, dev)
+    for t in (lv.n_levels, lv.mean, lv.std, lv.overflow):     # ct_cusum_batch writes every edges row
+        t.zero_()
     L = _lib.lib()
     wsb = int(L.ct_cusum_workspace_bytes(E))
     ws = torch.empty((wsb + 7) // 8, dtype=torch.int64, device=dev)
     with torch.cuda.device(dev):        # the library launches on the current device
         rc = L.ct_cusum_batch(y.data_ptr(), y.numel(), win_start.data_ptr(), win_end.data_ptr(),
                               types.data_ptr() if types is not None else None, E, float(delta), float(h),
-                              int(max_levels), nl.data_ptr(), ed.data_ptr(), mu.data_ptr(), sd.data_ptr(),
-                              ov.data_ptr(), ws.data_ptr(), wsb, _stream_ptr(y))
+                              lv.max_levels, lv.n_levels.data_ptr(), lv.edges.data_ptr(), lv.mean.data_ptr(),
+                              lv.std.data_ptr(), lv.overflow.data_ptr(), ws.data_ptr(), wsb, _stream_ptr(y))
     _lib.check(rc, "ct_cusum_batch")
-    return LevelTable(nl, ed, mu, sd, ov, int(max_levels))
+    return lv
 
 
 def cusum_flat(samples: torch.Tensor, offsets: torch.Tensor, **kw) -> LevelTable:

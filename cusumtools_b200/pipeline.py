@@ -95,6 +95,22 @@ class AnalysisResult:
     intra: "tuple[torch.Tensor, torch.Tensor] | None" = None     # (count int32 [E], pairs int32 [E, 2K]) crossings
     stepfit: "stepfit.StepFitTable | None" = None                # step-response fit of the short events (type 1 / 7)
 
+    def columns(self, index_offset: int = 0) -> dict:
+        """The per-event columns by name, in the order of the host event tables (`TraceAnalyzer.tables_to_host`,
+        `StreamResult.tables`); `index_offset` is added to starts and ends."""
+        starts, ends = self.events.starts, self.events.ends
+        if index_offset:
+            starts, ends = starts + index_offset, ends + index_offset
+        cols = {"starts": starts, "ends": ends, "types": self.types}
+        if self.levels is not None:
+            lv = self.levels
+            cols.update(n_levels=lv.n_levels, edges=lv.edges, mean=lv.mean, std=lv.std, overflow=lv.overflow)
+        if self.intra is not None:
+            cols.update(intra_count=self.intra[0], intra_pairs=self.intra[1])
+        if self.stepfit is not None:
+            cols.update(stepfit_params=self.stepfit.params, stepfit_cost=self.stepfit.cost, stepfit_iters=self.stepfit.iters)
+        return cols
+
 
 class TraceAnalyzer:
     """Stages 1-3 over a time shard with every buffer allocated once and a single host
@@ -174,7 +190,7 @@ class TraceAnalyzer:
         self._alloc_events(int(event_capacity) if event_capacity else max(1024, self.n_det // 2048))
 
     def _alloc_events(self, cap: int) -> None:
-        dev, ML = self.device, self.max_levels
+        dev = self.device
         self.cap = cap
         self.starts = torch.empty(cap, dtype=torch.int64, device=dev)
         self.ends = torch.empty(cap, dtype=torch.int64, device=dev)
@@ -183,21 +199,16 @@ class TraceAnalyzer:
         self.typ = torch.empty(cap, dtype=torch.int32, device=dev)
         self.scalars = torch.zeros(4, dtype=torch.int64, device=dev)     # n_starts, n_ends, n_kept, first kept index
         self.median_result = torch.zeros(4, dtype=torch.int32, device=dev)   # CtMedianResult: code1, code2, pad_x (float bits), status
-        if self.intra_threshold > 0:
-            self.ic = torch.zeros(cap, dtype=torch.int32, device=dev)
-            self.ip = torch.full((cap, 2 * self.max_crossings), -1, dtype=torch.int32, device=dev)
-        if self.delta is not None or self.fit_on:
-            self.nl = torch.empty(cap, dtype=torch.int32, device=dev)
-            self.ed = torch.empty((cap, ML + 1), dtype=torch.int32, device=dev)
-            self.mu = torch.empty((cap, ML), dtype=torch.float64, device=dev)
-            self.sd = torch.empty((cap, ML), dtype=torch.float64, device=dev)
-            self.ov = torch.empty(cap, dtype=torch.uint8, device=dev)
+        self.intra = ((torch.zeros(cap, dtype=torch.int32, device=dev),
+                       torch.full((cap, 2 * self.max_crossings), -1, dtype=torch.int32, device=dev))
+                      if self.intra_threshold > 0 else None)
+        self.levels = cusum.LevelTable.empty(cap, self.max_levels, dev) if self.delta is not None or self.fit_on else None
         if self.stepfit_fallback:
             self.sf_counter = torch.empty(1, dtype=torch.int64, device=dev)     # rows claimed by the long fit
-        if self.fit_on:
-            self.sf = {"params": torch.empty((cap, 6), dtype=torch.float64, device=dev),
-                       "cost": torch.empty(cap, dtype=torch.float64, device=dev),
-                       "iters": torch.empty(cap, dtype=torch.int32, device=dev)}
+        self.fit = (stepfit.StepFitTable(torch.empty((cap, 6), dtype=torch.float64, device=dev),
+                                         torch.empty(cap, dtype=torch.float64, device=dev),
+                                         torch.empty(cap, dtype=torch.int32, device=dev), self.typ)
+                    if self.fit_on else None)
         if self.delta is not None:
             self.cws_bytes = int(_lib.lib().ct_cusum_workspace_bytes(cap))
             self.cws = torch.empty((self.cws_bytes + 7) // 8, dtype=torch.int64, device=dev)
@@ -341,30 +352,29 @@ class TraceAnalyzer:
             if self.stepfit_samples:             # before CUSUM+, which then skips the short events
                 stepfit.select_short(self.w0, self.w1, self.typ, padding=self.event_padding,
                                      stepfit_samples=self.stepfit_samples, n_events_dev=sc[2:])
+            lv = self.levels
             if self.delta is not None:
                 rc = L.ct_cusum_batch_dev(yd.data_ptr(), self.n_det, self.w0.data_ptr(), self.w1.data_ptr(),
                                           self.typ.data_ptr(), sc[2:].data_ptr(), self.cap, float(self.delta),
-                                          float(self.h), self.max_levels, self.nl.data_ptr(), self.ed.data_ptr(),
-                                          self.mu.data_ptr(), self.sd.data_ptr(), self.ov.data_ptr(), self.cws.data_ptr(),
+                                          float(self.h), self.max_levels, lv.n_levels.data_ptr(), lv.edges.data_ptr(),
+                                          lv.mean.data_ptr(), lv.std.data_ptr(), lv.overflow.data_ptr(), self.cws.data_ptr(),
                                           self.cws_bytes, st)
                 _lib.check(rc, "ct_cusum_batch_dev")
             elif self.fit_on:                    # no CUSUM+: the rows of the events the fit does not take stay empty
-                self.nl.zero_(); self.ov.zero_(); self.ed.fill_(-1)
+                lv.clear()
             if self.stepfit_fallback:            # the events CUSUM+ left without a sub-level: type 1, or 8 (long)
-                stepfit.select_fallback({"n_levels": self.nl, "overflow": self.ov}, self.w0, self.w1, self.typ,
-                                        n_events_dev=sc[2:], capacity=self.cap)
+                stepfit.select_fallback(lv, self.w0, self.w1, self.typ, n_events_dev=sc[2:], capacity=self.cap)
             if self.fit_on:                      # after CUSUM+, which writes n_levels = 0 for every event not of type 0
-                lvd = {"n_levels": self.nl, "edges": self.ed, "mean": self.mu, "std": self.sd}
-                stepfit.launch(yd, self.w0, self.w1, self.typ, self.sf, lvd, padding=self.event_padding, tau0=self.tau0,
+                stepfit.launch(yd, self.w0, self.w1, self.typ, self.fit, lv, padding=self.event_padding, tau0=self.tau0,
                                n_events_dev=sc[2:], capacity=self.cap)
             if self.stepfit_fallback:            # after the short fit, which zeroes the params of every row not of type 1
-                stepfit.launch_long(yd, self.w0, self.w1, self.typ, self.sf, lvd, padding=self.event_padding,
+                stepfit.launch_long(yd, self.w0, self.w1, self.typ, self.fit, lv, padding=self.event_padding,
                                     tau0=self.tau0, n_events_dev=sc[2:], capacity=self.cap, row_counter=self.sf_counter)
-            if self.intra_threshold > 0:
+            if self.intra is not None:
                 # the block of the event start: win_start + padding (windows are compacted, the start list is not)
                 detect.intra_crossings(yd, self.w0, self.w1, self.w0 + self.event_padding, bl, self.intra_threshold,
                                        self.intra_hysteresis, max_pairs=self.max_crossings, n_events_dev=sc[2:],
-                                       out=(self.ic, self.ip))
+                                       out=self.intra)
             hook("cusum")
             tail = (self.median_result.to(torch.int64),) if on_device else ()
             host = torch.cat((sc[:4], bl.dev["status"].to(torch.int64)) + tail).cpu().numpy()   # the step's one sync
@@ -394,15 +404,12 @@ class TraceAnalyzer:
             open_start = o if 0 <= o < n_own else -1
         # event indices are reported relative to the first owned sample
         ev = detect.EventList(self.starts[i0:i0 + nk] - lo, self.ends[i0:i0 + nk] - lo, open_start)
-        lv = sf = None
-        if self.delta is not None or self.fit_on:
-            lv = cusum.LevelTable(self.nl[:nk], self.ed[:nk], self.mu[:nk], self.sd[:nk], self.ov[:nk], self.max_levels)
-        if self.fit_on:
-            sf = stepfit.StepFitTable(self.sf["params"][:nk], self.sf["cost"][:nk], self.sf["iters"][:nk], self.typ[:nk])
         return AnalysisResult(filtered=y[lo:lo + n_own], detect_trace=yd, lo_halo=lo, baseline=bl, events=ev,
-                              win_start=self.w0[:nk], win_end=self.w1[:nk], types=self.typ[:nk], levels=lv,
+                              win_start=self.w0[:nk], win_end=self.w1[:nk], types=self.typ[:nk],
+                              levels=None if self.levels is None else self.levels.rows(nk),
                               pad_value=pad_value, median_codes=(c1, c2), first_event_id=first_id, total_events=total,
-                              intra=(self.ic[:nk], self.ip[:nk]) if self.intra_threshold > 0 else None, stepfit=sf)
+                              intra=None if self.intra is None else (self.intra[0][:nk], self.intra[1][:nk]),
+                              stepfit=None if self.fit is None else self.fit.rows(nk))
 
 
     def tables_to_host(self, r: AnalysisResult) -> dict:
@@ -413,16 +420,8 @@ class TraceAnalyzer:
         if getattr(self, "_pinned_cap", 0) < self.cap:
             self._pinned = {}
             self._pinned_cap = self.cap
-        src = {"starts": r.events.starts, "ends": r.events.ends, "types": r.types}
-        if r.levels is not None:
-            src.update(n_levels=r.levels.n_levels, edges=r.levels.edges, mean=r.levels.mean, std=r.levels.std,
-                       overflow=r.levels.overflow)
-        if r.intra is not None:
-            src.update(intra_count=r.intra[0], intra_pairs=r.intra[1])
-        if r.stepfit is not None:
-            src.update(stepfit_params=r.stepfit.params, stepfit_cost=r.stepfit.cost, stepfit_iters=r.stepfit.iters)
         out = {}
-        for k, t in src.items():
+        for k, t in r.columns().items():
             if k not in self._pinned:
                 self._pinned[k] = torch.empty((self.cap,) + tuple(t.shape[1:]), dtype=t.dtype, pin_memory=True)
             h = self._pinned[k][:nk]
@@ -438,8 +437,7 @@ class StreamResult:
     table on the device, the event / level tables already in (pinned) host memory."""
     filtered: torch.Tensor          # float32 CUDA, the rank's owned samples
     baseline: detect.Baseline       # blocks of the owned range
-    tables: dict                    # numpy: starts, ends (relative to the first owned sample), types[, n_levels, edges, mean, std,
-                                    # overflow][, stepfit_params, stepfit_cost, stepfit_iters]
+    tables: dict                    # numpy: AnalysisResult.columns of the sub-shards, starts / ends from the first owned sample
     pad_value: float
     median_codes: tuple[int, int]
     first_event_id: int = 0
@@ -566,9 +564,6 @@ class StreamingAnalyzer:
         self.block = int(kw.get("baseline_block", detect.DEFAULT_BASELINE_BLOCK))
         self.padding = int(kw.get("padding", 1000))
         self.mask = filters.chimera_bitmask(settings)
-        self.max_levels = int(kw.get("max_levels", cusum.DEFAULT_MAX_LEVELS))
-        self.with_levels = (kw.get("cusum_delta") is not None or bool(kw.get("stepfit_samples"))
-                            or bool(kw.get("stepfit_fallback")))
         fs = float(np.floor(np.squeeze(settings["ADCSAMPLERATE"])))
         max_event = int(kw.get("maxpoints", 100_000)) + 2 * int(kw.get("event_padding", 100))
         self.h = required_halo(self.cutoff, self.order, fs, max_event, self.padding, block=self.block)
@@ -625,19 +620,11 @@ class StreamingAnalyzer:
         for name in ("cnt", "s1", "s2", "mean", "std", "sign", "t_start", "t_end"):
             bl.dev[name][g0:g0 + nbk].copy_(r.baseline.dev[name][k0:k0 + nbk])
         nk = int(r.events.starts.numel())
-        cols = {"starts": r.events.starts + (a - a0), "ends": r.events.ends + (a - a0), "types": r.types}
-        if r.levels is not None:
-            cols.update(n_levels=r.levels.n_levels, edges=r.levels.edges, mean=r.levels.mean, std=r.levels.std,
-                        overflow=r.levels.overflow)
-        if r.intra is not None:
-            cols.update(intra_count=r.intra[0], intra_pairs=r.intra[1])
-        if r.stepfit is not None:
-            cols.update(stepfit_params=r.stepfit.params, stepfit_cost=r.stepfit.cost, stepfit_iters=r.stepfit.iters)
         if end_at is not None:
             if nk > end_at:
                 return -1
             row0 = end_at - nk
-        for name, t in cols.items():
+        for name, t in r.columns(a - a0).items():
             self._pinned(name, t, row0 + nk)[row0:row0 + nk].copy_(t, non_blocking=True)
         return nk
 

@@ -52,6 +52,11 @@ class StepFitTable:
     status: torch.Tensor       # int32 [E]
     levels: LevelTable | None = None     # the three level rows of every valid fit (standalone calls)
 
+    def rows(self, n: int) -> StepFitTable:
+        """The first `n` rows, as views of these buffers."""
+        return StepFitTable(self.params[:n], self.cost[:n], self.iters[:n], self.status[:n],
+                            None if self.levels is None else self.levels.rows(n))
+
 
 def zero_phase_rise_tau(samplerate: float, cutoff: float, order: int = 8) -> float:
     """tau0 of the initial guess: (t90 - t10) / ln 9 in samples, t10 / t90 the first samples at which the step
@@ -77,15 +82,15 @@ def select_short(win_start: torch.Tensor, win_end: torch.Tensor, types: torch.Te
     _lib.check(rc, "ct_stepfit_select")
 
 
-def select_fallback(levels: dict, win_start: torch.Tensor, win_end: torch.Tensor, types: torch.Tensor, *,
+def select_fallback(levels: LevelTable, win_start: torch.Tensor, win_end: torch.Tensor, types: torch.Tensor, *,
                     n_events_dev: torch.Tensor | None = None, capacity: int | None = None) -> None:
     """In place, after CUSUM+: every event still of type 0 with no level overflow and fewer than three levels
-    (levels = {n_levels, overflow}) becomes type 1 if its window is at most MAX_WINDOW samples, else
+    (`levels.n_levels`, `levels.overflow`) becomes type 1 if its window is at most MAX_WINDOW samples, else
     TYPE_STEPFIT_LONG (ct_stepfit_fallback_select).  No other row changes."""
     _require_cuda(types, "types", torch.int32)
     cap = int(types.numel() if capacity is None else capacity)
     with torch.cuda.device(types.device):
-        rc = _lib.lib().ct_stepfit_fallback_select(levels["n_levels"].data_ptr(), levels["overflow"].data_ptr(),
+        rc = _lib.lib().ct_stepfit_fallback_select(levels.n_levels.data_ptr(), levels.overflow.data_ptr(),
                                                    win_start.data_ptr(), win_end.data_ptr(), types.data_ptr(),
                                                    n_events_dev.data_ptr() if n_events_dev is not None else None, cap,
                                                    _stream_ptr(types))
@@ -99,22 +104,22 @@ def _launch(fn: str, y, win_start, win_end, types, out, levels, padding, tau0, m
         rc = getattr(_lib.lib(), fn)(
             y.data_ptr(), y.numel(), win_start.data_ptr(), win_end.data_ptr(), types.data_ptr(),
             n_events_dev.data_ptr() if n_events_dev is not None else None, cap, int(padding), float(tau0), int(max_iters),
-            int(levels["mean"].shape[1]), out["params"].data_ptr(), out["cost"].data_ptr(), out["iters"].data_ptr(),
-            levels["n_levels"].data_ptr(), levels["edges"].data_ptr(), levels["mean"].data_ptr(), levels["std"].data_ptr(),
+            levels.max_levels, out.params.data_ptr(), out.cost.data_ptr(), out.iters.data_ptr(),
+            levels.n_levels.data_ptr(), levels.edges.data_ptr(), levels.mean.data_ptr(), levels.std.data_ptr(),
             *extra, _stream_ptr(y))
     _lib.check(rc, fn)
 
 
-def launch(y: torch.Tensor, win_start: torch.Tensor, win_end: torch.Tensor, types: torch.Tensor, out: dict, levels: dict, *,
-           padding: int, tau0: float, max_iters: int = DEFAULT_MAX_ITERS, n_events_dev: torch.Tensor | None = None,
-           capacity: int | None = None) -> None:
-    """ct_stepfit_batch into caller-owned buffers: out = {params, cost, iters}, levels = {n_levels, edges, mean, std}
-    (`max_levels` = mean.shape[1]).  `types` is updated in place (7 where a fit fails)."""
+def launch(y: torch.Tensor, win_start: torch.Tensor, win_end: torch.Tensor, types: torch.Tensor, out: StepFitTable,
+           levels: LevelTable, *, padding: int, tau0: float, max_iters: int = DEFAULT_MAX_ITERS,
+           n_events_dev: torch.Tensor | None = None, capacity: int | None = None) -> None:
+    """ct_stepfit_batch into caller-owned buffers: the params, cost and iters of `out` and the n_levels, edges, mean
+    and std rows of `levels` (overflow is not touched).  `types` is updated in place (7 where a fit fails)."""
     _launch("ct_stepfit_batch", y, win_start, win_end, types, out, levels, padding, tau0, max_iters, n_events_dev, capacity)
 
 
-def launch_long(y: torch.Tensor, win_start: torch.Tensor, win_end: torch.Tensor, types: torch.Tensor, out: dict,
-                levels: dict, *, padding: int, tau0: float, max_iters: int = LONG_DEFAULT_MAX_ITERS,
+def launch_long(y: torch.Tensor, win_start: torch.Tensor, win_end: torch.Tensor, types: torch.Tensor, out: StepFitTable,
+                levels: LevelTable, *, padding: int, tau0: float, max_iters: int = LONG_DEFAULT_MAX_ITERS,
                 n_events_dev: torch.Tensor | None = None, capacity: int | None = None,
                 row_counter: torch.Tensor | None = None) -> None:
     """ct_stepfit_long_batch, the mirror of `launch`: fits the rows of type TYPE_STEPFIT_LONG (one CTA per event) and
@@ -140,18 +145,14 @@ def _fit_all(fn, selected: int, y, win_start, win_end, padding, tau0, max_iters,
     else:
         _require_cuda(types, "types", torch.int32)
         st = types.clone()
-    out = {"params": torch.zeros((E, 6), dtype=torch.float64, device=dev),
-           "cost": torch.zeros(E, dtype=torch.float64, device=dev),
-           "iters": torch.zeros(E, dtype=torch.int32, device=dev)}
-    lv = {"n_levels": torch.zeros(E, dtype=torch.int32, device=dev),
-          "edges": torch.full((E, max_levels + 1), -1, dtype=torch.int32, device=dev),
-          "mean": torch.zeros((E, max_levels), dtype=torch.float64, device=dev),
-          "std": torch.zeros((E, max_levels), dtype=torch.float64, device=dev)}
+    out = StepFitTable(torch.zeros((E, 6), dtype=torch.float64, device=dev), torch.zeros(E, dtype=torch.float64, device=dev),
+                       torch.zeros(E, dtype=torch.int32, device=dev), st, LevelTable.empty(E, max_levels, dev))
+    out.levels.clear()
+    for t in (out.levels.mean, out.levels.std):
+        t.zero_()
     if E:
-        fn(y, win_start, win_end, st, out, lv, padding=padding, tau0=tau0, max_iters=max_iters)
-    levels = LevelTable(lv["n_levels"], lv["edges"], lv["mean"], lv["std"], torch.zeros(E, dtype=torch.uint8, device=dev),
-                        int(max_levels))
-    return StepFitTable(out["params"], out["cost"], out["iters"], st, levels)
+        fn(y, win_start, win_end, st, out, out.levels, padding=padding, tau0=tau0, max_iters=max_iters)
+    return out
 
 
 def step_fit(y: torch.Tensor, win_start: torch.Tensor, win_end: torch.Tensor, *, padding: int, tau0: float,

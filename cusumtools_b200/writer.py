@@ -46,7 +46,7 @@ from dataclasses import dataclass
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, cusum
 from .filters import _require_cuda, _stream_ptr
 
 EVENT_COLUMNS = ["id", "type", "start_time_s", "event_delay_s", "duration_us", "threshold", "baseline_before_pA",
@@ -178,10 +178,6 @@ class EventTable:
         return len(self.events["id"])
 
 
-def _fmt_list(v) -> str:
-    return ";".join("%.16g" % x for x in v)        # mosaicConverter.py:139-148 ('%.16g;' joined, last ';' cut)
-
-
 def build_event_table(*, starts, ends, types, n_levels, edges, level_mean, level_std, overflow, xmin, xmax,
                       samplerate: float, threshold: float, baseline_mean, baseline_std, baseline_block: int,
                       padding: int, first_id: int = 0, time_offset_s: float = 0.0, index_offset: int = 0,
@@ -267,20 +263,25 @@ def build_event_table(*, starts, ends, types, n_levels, edges, level_mean, level
     return EventTable(events=events, rate=rate)
 
 
+def _table_from_host(tabs: dict, levels, types, y, win_start, win_end, baseline, **kw) -> EventTable:
+    """`build_event_table` over the host columns of an analyzer (pipeline.AnalysisResult.columns), with the derived
+    columns and the extrema of the windows y[win_start:win_end] computed on the device (`event_columns`)."""
+    lo, hi = event_extrema(y, win_start, win_end)
+    cols, ty = event_columns(levels, types, lo, hi)
+    return build_event_table(columns=(cols.cpu().numpy(), ty.cpu().numpy()), starts=tabs["starts"], ends=tabs["ends"],
+                             types=tabs["types"], n_levels=tabs["n_levels"], edges=tabs["edges"], level_mean=tabs["mean"],
+                             level_std=tabs["std"], overflow=tabs["overflow"], xmin=lo.cpu().numpy(), xmax=hi.cpu().numpy(),
+                             baseline_mean=baseline.mean, baseline_std=baseline.std, intra_count=tabs.get("intra_count"),
+                             intra_pairs=tabs.get("intra_pairs"), stepfit_params=tabs.get("stepfit_params"), **kw)
+
+
 def event_table_from_result(an, r, *, samplerate: float, time_offset_s: float = 0.0, index_offset: int = 0) -> EventTable:
     """Event table of one `pipeline.TraceAnalyzer.run` result (device -> host, then
     `build_event_table`)."""
-    lo, hi = event_extrema(r.detect_trace, r.win_start, r.win_end)
-    cols = event_columns(r.levels, r.types, lo, hi) if r.levels is not None else None
-    tabs = an.tables_to_host(r)
-    return build_event_table(columns=None if cols is None else (cols[0].cpu().numpy(), cols[1].cpu().numpy()), starts=tabs["starts"], ends=tabs["ends"], types=tabs["types"], n_levels=tabs["n_levels"],
-                             edges=tabs["edges"], level_mean=tabs["mean"], level_std=tabs["std"],
-                             overflow=tabs["overflow"], xmin=lo.cpu().numpy(), xmax=hi.cpu().numpy(),
-                             samplerate=samplerate, threshold=an.threshold, baseline_mean=r.baseline.mean,
-                             baseline_std=r.baseline.std, baseline_block=an.block, padding=an.event_padding,
-                             first_id=r.first_event_id, time_offset_s=time_offset_s, index_offset=index_offset,
-                             block_offset=r.lo_halo, intra_count=tabs.get("intra_count"), intra_pairs=tabs.get("intra_pairs"),
-                             stepfit_params=tabs.get("stepfit_params"))
+    return _table_from_host(an.tables_to_host(r), r.levels, r.types, r.detect_trace, r.win_start, r.win_end, r.baseline,
+                            samplerate=samplerate, threshold=an.threshold, baseline_block=an.block,
+                            padding=an.event_padding, first_id=r.first_event_id, time_offset_s=time_offset_s,
+                            index_offset=index_offset, block_offset=r.lo_halo)
 
 
 def event_table_from_stream(san, rs, *, samplerate: float, time_offset_s: float = 0.0, index_offset: int = 0) -> EventTable:
@@ -292,22 +293,11 @@ def event_table_from_stream(san, rs, *, samplerate: float, time_offset_s: float 
     dev = rs.filtered.device
     w0 = torch.from_numpy(np.clip(t["starts"] - pad, 0, n)).to(dev)
     w1 = torch.from_numpy(np.clip(t["ends"] + pad, 0, n)).to(dev)
-    lo, hi = event_extrema(rs.filtered, w0, w1)
-    cols = None
-    if "mean" in t:          # the level table went to the host sub-shard by sub-shard: one upload for the derived columns
-        from .cusum import LevelTable
-        lv = LevelTable(*(torch.from_numpy(np.ascontiguousarray(t[k])).to(dev) for k in ("n_levels", "edges", "mean", "std", "overflow")),
-                        int(t["mean"].shape[1]))
-        c, ty = event_columns(lv, torch.from_numpy(np.ascontiguousarray(t["types"])).to(dev), lo, hi)
-        cols = (c.cpu().numpy(), ty.cpu().numpy())
-    return build_event_table(columns=cols, starts=t["starts"], ends=t["ends"], types=t["types"], n_levels=t["n_levels"],
-                             edges=t["edges"], level_mean=t["mean"], level_std=t["std"], overflow=t["overflow"],
-                             xmin=lo.cpu().numpy(), xmax=hi.cpu().numpy(), samplerate=samplerate,
-                             threshold=float(san.kw.get("threshold", 5.0)), baseline_mean=rs.baseline.mean,
-                             baseline_std=rs.baseline.std, baseline_block=san.block, padding=pad,
-                             first_id=rs.first_event_id, time_offset_s=time_offset_s, index_offset=index_offset,
-                             intra_count=t.get("intra_count"), intra_pairs=t.get("intra_pairs"),
-                             stepfit_params=t.get("stepfit_params"))
+    # the level rows went to the host sub-shard by sub-shard: one upload for the derived columns
+    types = torch.from_numpy(np.ascontiguousarray(t["types"])).to(dev)
+    return _table_from_host(t, cusum.LevelTable.from_columns(t, dev), types, rs.filtered, w0, w1, rs.baseline,
+                            samplerate=samplerate, threshold=float(san.kw.get("threshold", 5.0)), baseline_block=san.block,
+                            padding=pad, first_id=rs.first_event_id, time_offset_s=time_offset_s, index_offset=index_offset)
 
 
 def _write_csv(path: str, columns, table: dict) -> None:

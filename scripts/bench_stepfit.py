@@ -16,7 +16,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import torch
 
-from cusumtools_b200 import pipeline, stepfit, synth
+from cusumtools_b200 import cusum, pipeline, stepfit, synth
 
 
 def gpu_info() -> dict:
@@ -38,10 +38,10 @@ def bench_kernel(n_events: int, launches: int) -> dict:
     tau0 = stepfit.zero_phase_rise_tau(synth.FS, 1e5, 8)
     types0 = torch.full((E,), stepfit.TYPE_STEPFIT, dtype=torch.int32, device=dev)
     types = types0.clone()
-    out = {"params": torch.zeros((E, 6), dtype=torch.float64, device=dev), "cost": torch.zeros(E, dtype=torch.float64, device=dev),
-           "iters": torch.zeros(E, dtype=torch.int32, device=dev)}
-    lv = {"n_levels": torch.zeros(E, dtype=torch.int32, device=dev), "edges": torch.zeros((E, 4), dtype=torch.int32, device=dev),
-          "mean": torch.zeros((E, 3), dtype=torch.float64, device=dev), "std": torch.zeros((E, 3), dtype=torch.float64, device=dev)}
+    out = stepfit.StepFitTable(torch.zeros((E, 6), dtype=torch.float64, device=dev),
+                               torch.zeros(E, dtype=torch.float64, device=dev), torch.zeros(E, dtype=torch.int32, device=dev),
+                               types)
+    lv = cusum.LevelTable.empty(E, 3, dev)
     times = []
     for i in range(2 + launches):
         types.copy_(types0)                         # the launch marks failed fits in place: every launch starts alike
@@ -53,7 +53,7 @@ def bench_kernel(n_events: int, launches: int) -> dict:
         if i >= 2:
             times.append(a.elapsed_time(b) * 1e-3)
     t = np.array(times)
-    it = out["iters"].cpu().numpy()
+    it = out.iters.cpu().numpy()
     st = types.cpu().numpy()
     nsamp = int(off[-1].item())
     med = float(np.median(t))
@@ -61,7 +61,7 @@ def bench_kernel(n_events: int, launches: int) -> dict:
     by_len = {}
     for lo_, hi_ in ((20, 60), (60, 100), (100, 200), (200, 401)):
         m = (ln >= lo_) & (ln < hi_) & (st == 1)
-        p = out["params"].cpu().numpy()[m]
+        p = out.params.cpu().numpy()[m]
         dd = np.abs(depth.cpu().numpy()[m])
         by_len[f"{lo_}-{hi_ - 1}"] = {"events": int(((ln >= lo_) & (ln < hi_)).sum()),
                                       "median_depth_error": float(np.median(np.abs(np.abs(p[:, 1]) - dd) / dd)) if m.any() else None}

@@ -18,7 +18,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import torch
 
-from cusumtools_b200 import pipeline, stepfit, synth
+from cusumtools_b200 import cusum, pipeline, stepfit, synth
 from scripts.bench_stepfit import gpu_info
 
 
@@ -31,10 +31,10 @@ def bench_kernel(n_events: int, launches: int) -> dict:
     tau0 = stepfit.zero_phase_rise_tau(synth.FS, 1e5, 8)
     types0 = torch.full((E,), stepfit.TYPE_STEPFIT_LONG, dtype=torch.int32, device=dev)
     types = types0.clone()
-    out = {"params": torch.zeros((E, 6), dtype=torch.float64, device=dev), "cost": torch.zeros(E, dtype=torch.float64, device=dev),
-           "iters": torch.zeros(E, dtype=torch.int32, device=dev)}
-    lv = {"n_levels": torch.zeros(E, dtype=torch.int32, device=dev), "edges": torch.zeros((E, 4), dtype=torch.int32, device=dev),
-          "mean": torch.zeros((E, 3), dtype=torch.float64, device=dev), "std": torch.zeros((E, 3), dtype=torch.float64, device=dev)}
+    out = stepfit.StepFitTable(torch.zeros((E, 6), dtype=torch.float64, device=dev),
+                               torch.zeros(E, dtype=torch.float64, device=dev), torch.zeros(E, dtype=torch.int32, device=dev),
+                               types)
+    lv = cusum.LevelTable.empty(E, 3, dev)
     times = []
     for i in range(1 + launches):
         types.copy_(types0)                         # the launch sets every row to 1 / 7: every launch starts alike
@@ -46,7 +46,7 @@ def bench_kernel(n_events: int, launches: int) -> dict:
         if i >= 1:
             times.append(a.elapsed_time(b) * 1e-3)
     t = np.array(times)
-    it = out["iters"].cpu().numpy()
+    it = out.iters.cpu().numpy()
     st = types.cpu().numpy()
     ln = lens.cpu().numpy()
     win = ln + 2 * synth.SHORT_PAD
@@ -54,7 +54,7 @@ def bench_kernel(n_events: int, launches: int) -> dict:
     nsamp = int(win.sum())
     # `iters` also counts the few trials that are never evaluated: window samples x iters bounds the passes from above
     sample_trials = float((win.astype(np.float64) * it).sum())
-    p = out["params"].cpu().numpy()
+    p = out.params.cpu().numpy()
     dd = np.abs(depth.cpu().numpy())
     by_len = {}
     for lo_, hi_ in ((8000, 16000), (16000, 32000), (32000, 64000), (64000, 100_001)):

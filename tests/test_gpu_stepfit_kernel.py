@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from cusumtools_b200 import pipeline, stepfit, synth
+from cusumtools_b200 import cusum, pipeline, stepfit, synth
 from oracle import stepfit_oracle as so
 from oracle import stepfit_twin as tw
 
@@ -210,18 +210,17 @@ def _launch_sentinel(t, max_levels, w0, w1, typ, count):
     dev = t["y"].device
     cap = w0.size
     types = torch.from_numpy(typ.copy()).to(dev)
-    out = {"params": torch.full((cap, 6), SENT_F, dtype=torch.float64, device=dev),
-           "cost": torch.full((cap,), SENT_F, dtype=torch.float64, device=dev),
-           "iters": torch.full((cap,), SENT_I, dtype=torch.int32, device=dev)}
-    lv = {"n_levels": torch.full((cap,), SENT_I, dtype=torch.int32, device=dev),
-          "edges": torch.full((cap, max_levels + 1), SENT_I, dtype=torch.int32, device=dev),
-          "mean": torch.full((cap, max_levels), SENT_F, dtype=torch.float64, device=dev),
-          "std": torch.full((cap, max_levels), SENT_F, dtype=torch.float64, device=dev)}
+    out = stepfit.StepFitTable(torch.full((cap, 6), SENT_F, dtype=torch.float64, device=dev),
+                               torch.full((cap,), SENT_F, dtype=torch.float64, device=dev),
+                               torch.full((cap,), SENT_I, dtype=torch.int32, device=dev), types)
+    lv = cusum.LevelTable.empty(cap, max_levels, dev)
+    for buf, v in ((lv.n_levels, SENT_I), (lv.edges, SENT_I), (lv.mean, SENT_F), (lv.std, SENT_F)):
+        buf.fill_(v)
     stepfit.launch(t["y"], torch.from_numpy(w0).to(dev), torch.from_numpy(w1).to(dev), types, out, lv, padding=PAD,
                    tau0=TAU0, n_events_dev=torch.tensor([count], dtype=torch.int64, device=dev), capacity=cap)
-    res = {k: v.cpu().numpy() for k, v in {**out, **lv}.items()}
-    res["type"] = types.cpu().numpy()
-    return res
+    res = {"params": out.params, "cost": out.cost, "iters": out.iters, "n_levels": lv.n_levels, "edges": lv.edges,
+           "mean": lv.mean, "std": lv.std, "type": types}
+    return {k: v.cpu().numpy() for k, v in res.items()}
 
 
 def test_row_contract(trace):
