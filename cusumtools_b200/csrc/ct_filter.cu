@@ -305,8 +305,10 @@ int ct_hist_sampled_u16(const uint16_t* raw, int64_t n, int64_t stride, uint16_t
 
 static int count_window(const uint16_t* raw, int64_t n, uint16_t mask, uint32_t lo, uint32_t step, uint64_t* counts9,
                         bool wide, void* stream) {
-    if (!raw || !counts9 || n < 0 || step < 1 || (step & (step - 1)) || (lo & (step - 1))) {
-        ct_set_error("count_window: bad argument (step must be a power of two and lo a multiple of it)"); return CT_ERR_ARG;
+    // a mask bit below step would let the vector path shift the high code's low bits into the low code of a word
+    if (!raw || !counts9 || n < 0 || step < 1 || (step & (step - 1)) || (lo & (step - 1)) || (mask & (step - 1))) {
+        ct_set_error("count_window: bad argument (step must be a power of two, lo and every masked code multiples of it)");
+        return CT_ERR_ARG;
     }
     if (n == 0) return CT_OK;
     long long blocks = (long long)ct_sm_count() * 8;

@@ -1084,6 +1084,10 @@ int ct_filter_forward_seq(const void* in, int in_kind, int64_t n, int64_t pad, f
     a.scratch_floats = (ct_filtfilt_workspace_bytes(n, pad, H) - 256) / 4;
     if (counts9 && part != 1 && in_kind == 0) {
         if (!cw_step || (cw_step & (cw_step - 1))) { ct_set_error("filter: window step must be a power of two"); return CT_ERR_ARG; }
+        if ((cw_lo & (cw_step - 1)) || (mask & (cw_step - 1))) {     // the tally's nibble index 4 (code - lo) / step
+            ct_set_error("filter: the window's first code and every masked code must be multiples of the window step");
+            return CT_ERR_ARG;
+        }
         if (cw_step > 4) { ct_set_error("filter: the fused window count needs a window step <= 4 (ADC of 14 bits or more)"); return CT_ERR_UNSUPPORTED; }
         a.cw_k = 4u / cw_step; a.cw_c = 0u - (0x4B000000u + cw_lo) * a.cw_k; a.cw_out = (unsigned long long*)counts9;
         a.cw_p0 = cw_begin < 0 ? 0 : cw_begin; a.cw_p1 = cw_end > n ? n : cw_end;

@@ -93,7 +93,8 @@ int ct_filtfilt_f32(const float* x, int64_t n, int64_t pad, float pad_value, con
  *     filtfilt(code - m) + m == filtfilt(code - c) + c      for ANY constant c,
  * provided the pad holds m - c instead of 0.  So the forward pass may subtract an estimate c
  * (`sub_code`) with pad_x = 0; it can tally, on the side, the window counts that pin the exact
- * median m (counts9: as ct_count_window_u16, window_step <= 4, zeroed by the caller); if m != c the caller re-runs
+ * median m (counts9: as ct_count_window_u16, window_step <= 4, window_lo and every masked code multiples of window_step,
+ * else CT_ERR_ARG and counts9 untouched; zeroed by the caller); if m != c the caller re-runs
  * only the groups the pad influences (`part` = 1, pad_x = m - c) and then runs the backward
  * pass with the same sub_code and offset = value(sub_code).  `origin` (>= 0) aligns the run grid with
  * baseline blocks counted from that output sample; both passes must get the same value.  Only codes at
@@ -135,6 +136,8 @@ int ct_filter_backward(int64_t n, int64_t pad, float sub_code, float scale, floa
  * (plot-trace.py:319): a strided-sample histogram to locate it and an exact count of
  * the codes below / inside a window of 8 codes {lo + i*step} to verify it.
  *   hist65536: uint32[65536], caller-zeroed; counts9: uint64[9], caller-zeroed.
+ * The window counts need step a power of two and lo and mask multiples of it (mask & (step - 1) == 0: every masked
+ * code is some lo + i*step or outside the window); any other step, lo or mask returns CT_ERR_ARG with counts9 untouched.
  * ct_count_window4_u16 counts only the first four window codes (counts9[5..8] untouched): the
  * cheaper first attempt when the estimate comes from a sample of the whole trace.         */
 int ct_hist_sampled_u16(const uint16_t* raw, int64_t n, int64_t stride, uint16_t mask,

@@ -189,7 +189,8 @@ def test_code_median_is_exact():
         c1, c2 = median.code_median(torch.from_numpy(codes).cuda(), 0xFFFC)
         srt = np.sort(codes)
         assert (c1, c2) == (int(srt[(n - 1) // 2]), int(srt[n // 2]))
-    # bimodal: the window search must recover when the sample estimate is off
+    # bimodal, 1 000 001 codes: under 2^21 samples the stride is 1 and the estimate's full histogram is already exact
+    # (the window search over the device counters is test_gpu_median_kernels.py's)
     codes = np.concatenate((np.full(500000, 1000), np.full(500001, 60000))).astype(np.uint16)
     assert median.code_median(torch.from_numpy(codes).cuda(), 0xFFFF) == (60000, 60000)
 
