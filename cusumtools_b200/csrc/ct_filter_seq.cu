@@ -267,7 +267,8 @@ static __device__ __forceinline__ void out_write_slot(unsigned outb, int lane, i
     sts128(a0 + 32 * 128, y[0].y, y[1].y, y[2].y, y[3].y);
     sts128(a1 + 32 * 128, y[4].y, y[5].y, y[6].y, y[7].y);
 }
-// guarded copy of half-tile hb (positions first + r*R + [0, 32), r = 0..63) to the natural-layout output
+// guarded copy of half-tile hb (positions first + r*R + [0, 32), r = 0..63) to the natural-layout output; the caller
+// syncs the warp after it
 static __device__ void out_store_guarded(const SeqArgs& a, unsigned outb, int hb, long long first, int lane) {
     for (int r = 0; r < kRuns; ++r) {
         const long long p = first + (long long)r * a.R + lane;
@@ -276,6 +277,9 @@ static __device__ void out_store_guarded(const SeqArgs& a, unsigned outb, int hb
         asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(addr));
         if (p >= 0 && p < a.n_out) a.out[p] = v;
     }
+    // this half-tile commits no bulk group, so the callers' paced waits (which count groups) would not cover a tile
+    // store of the OTHER half that is still reading it when that half is rewritten next: drain them here
+    if (lane == 0) bulk_wait_read<0>();
 }
 
 // ------------------------------------------------------------------ baseline block sums + chunk extrema (BWD epilogue)

@@ -217,11 +217,13 @@ def bessel_filtfilt(x: torch.Tensor, samplerate: float, cutoff: float, order: in
     `filter_data` on float data)."""
     _require_cuda(x, "x", torch.float32)
     n = x.numel()
-    if pad_value is None:            # np.pad(mode='median'), plot-trace.py:319
-        pad_value = float_median(x)
     if out is None:
         out = torch.empty(n, dtype=torch.float32, device=x.device)
     _require_cuda(out, "out", torch.float32)
+    if out.numel() != n:
+        raise ValueError("out has the wrong length")
+    if pad_value is None:            # np.pad(mode='median'), plot-trace.py:319
+        pad_value = float_median(x)
     design = bessel_lowpass(int(order), 2.0 * float(cutoff) / float(samplerate))
     coef = make_coef(design)
     H = warmup_samples(design, halo_eps)
