@@ -665,6 +665,8 @@ int ct_baseline_finalize(const int64_t* cnt, const int64_t* s1, const int64_t* s
     if (!cnt || !s1 || !s2 || !mean || !stdev || !sign || !t_start || !t_end || !status || nb < 0) {
         ct_set_error("baseline_finalize: bad argument"); return CT_ERR_ARG;
     }
+    // the end line must lie between the start line and the baseline (NaN thresholds, hysteresis 0, stay allowed)
+    if (!(hysteresis >= 0.0)) { ct_set_error("baseline_finalize: hysteresis must be >= 0 (a negative one crosses the lines)"); return CT_ERR_ARG; }
     if (nb == 0) return CT_OK;
     CT_COUNT_LAUNCH();
     ct_baseline_finalize_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(

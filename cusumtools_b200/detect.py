@@ -32,6 +32,12 @@ def stats_shift(half_width: float, block: int) -> int:
     return s
 
 
+def check_hysteresis(name: str, value) -> None:
+    """Raise ValueError unless `value` >= 0: the end line must lie between the start line and the baseline."""
+    if not float(value) >= 0.0:
+        raise ValueError(f"{name} must be >= 0, got {value} (a negative hysteresis crosses the start and end lines)")
+
+
 class Baseline:
     """Per-block baseline table (the rows of baseline.csv) plus the float32 lines the
     detector compares against.  When produced by `baseline_blocks` everything lives on the
@@ -91,7 +97,10 @@ class Baseline:
 
     def with_thresholds(self, threshold: float, hysteresis: float) -> "Baseline":
         """plot-trace.py:408-411: start line = baseline - sign*threshold*stdev, end line =
-        baseline - sign*(threshold - hysteresis)*stdev, rounded to float32."""
+        baseline - sign*(threshold - hysteresis)*stdev, rounded to float32.  `hysteresis` must be
+        >= 0: a negative one puts the end line beyond the start line, where the detector's
+        definition no longer holds."""
+        check_hysteresis("hysteresis", hysteresis)
         self.threshold, self.hysteresis = float(threshold), float(hysteresis)
         if self.dev is not None:
             d = self.dev

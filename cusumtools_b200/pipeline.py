@@ -133,6 +133,8 @@ class TraceAnalyzer:
                  fused_count: bool = True, intra_threshold: float = 0.0, intra_hysteresis: float = 0.0,
                  max_crossings: int = 8, halos_clipped_by_trace_ends: bool = False, stepfit_samples: int = 0,
                  stepfit_fallback: bool = False):
+        detect.check_hysteresis("hysteresis", hysteresis)
+        detect.check_hysteresis("intra_hysteresis", intra_hysteresis)
         self.n_ext, self.lo_halo, self.hi_halo = int(n_ext), int(lo_halo), int(hi_halo)
         self.n_own = self.n_ext - self.lo_halo - self.hi_halo
         self.n_det = self.n_ext
@@ -557,6 +559,9 @@ class StreamingAnalyzer:
 
     def __init__(self, n_ext: int, settings, cutoff: float, order: int = 8, *, lo_halo: int = 0, hi_halo: int = 0,
                  shards: int = 16, first_blocks: int = 4, group=None, device="cuda", **kw):
+        # the sub-shard analyzers are built lazily: reject what they would reject before anything is allocated
+        detect.check_hysteresis("hysteresis", kw.get("hysteresis", 1.0))
+        detect.check_hysteresis("intra_hysteresis", kw.get("intra_hysteresis", 0.0))
         self.n_ext, self.lo_halo, self.hi_halo = int(n_ext), int(lo_halo), int(hi_halo)
         self.n_own = self.n_ext - self.lo_halo - self.hi_halo
         self.settings, self.cutoff, self.order = settings, float(cutoff), int(order)

@@ -164,7 +164,8 @@ int ct_block_stats_f32(const float* y, int64_t n, int64_t block, float bmin, flo
  *   individually rounded float64 operations; blocks with cnt < min_count inherit the nearest
  *   earlier valid block; sign = sign(mean); t_start = (float)(mean - sign*threshold*std);
  *   t_end = (float)(mean - sign*(threshold - hysteresis)*std).  status[0] = 1 if no block
- *   is valid (nothing else is written then).  All arrays have nb entries.                */
+ *   is valid (nothing else is written then).  All arrays have nb entries.  hysteresis must be
+ *   >= 0 (CT_ERR_ARG before any launch otherwise): a negative one crosses the two lines.   */
 int ct_baseline_finalize(const int64_t* cnt, const int64_t* s1, const int64_t* s2, int64_t nb, float c0, int shift,
                          int64_t min_count, double threshold, double hysteresis, double* mean, double* stdev,
                          int32_t* sign, float* t_start, float* t_end, int32_t* status, void* stream);
@@ -175,7 +176,10 @@ int64_t ct_detect_workspace_bytes(int64_t n);
  * [starts[i], ends[i]) for i < n_ends and starts[n_ends] (if any) is still open.
  * chunk_minmax (may be NULL): the (min, max) pairs ct_filter_backward left for the 64-sample chunks of y,
  * entry c covering samples [64 c - minmax_shift, 64 c - minmax_shift + 64); whole chunks are then classified
- * against the block's lines and only chunks that hold a crossing are read from y (same result).   */
+ * against the block's lines and only chunks that hold a crossing are read from y (same result).
+ * Precondition: sign*t_start <= sign*t_end in every block (the end line lies between the start line and
+ * the baseline, as ct_baseline_finalize makes it).  With crossed lines a sample between them would be both
+ * "beyond the start line" and "back beyond the end line", and the result is not defined.              */
 int ct_detect_f32(const float* y, int64_t n, int64_t block, const int32_t* sign, const float* t_start,
                   const float* t_end, int state_in, const float* chunk_minmax, int64_t minmax_shift, void* workspace,
                   int64_t workspace_bytes, int64_t* starts, int64_t* ends, int64_t capacity, uint64_t* counts2, void* stream);

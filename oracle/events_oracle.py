@@ -143,7 +143,11 @@ def detect_events(y, block, sign, t_start, t_end, state_in=False):
     sample beyond the start line while outside an event and ENDS at the first sample back
     beyond the end line while inside one; the event occupies [start, end).  Returns
     (starts int64[E], ends int64[E], open_start) where open_start is the start index of an
-    event still open at the end of the data (or -1)."""
+    event still open at the end of the data (or -1).
+
+    Precondition: sign*t_start <= sign*t_end in every block (hysteresis >= 0).  With crossed
+    lines a sample between them is both beyond the start line and back beyond the end line,
+    and this vectorised form no longer agrees with `detect_events_sequential`."""
     y = np.asarray(y, dtype=np.float32)
     n = y.size
     if n == 0:

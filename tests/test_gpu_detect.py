@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 import torch
 
-from cusumtools_b200 import detect, filters, synth
+from cusumtools_b200 import _lib, detect, filters, synth
 from oracle import c_twin, events_oracle as eo
 
 pytestmark = pytest.mark.gpu
@@ -69,17 +69,19 @@ def test_detection_edge_cases():
 
 
 def test_random_symbol_streams_match_sequential_definition():
-    rng = np.random.default_rng(5)
     block = 4096
-    for n in (1, 31, 32, 33, 4095, 4096, 4097, 100000):
-        y = rng.choice(np.array([80, 92, 100], np.float32), size=n, p=[0.02, 0.9, 0.08])
-        nb = (n + block - 1) // block
-        bl = detect.Baseline(block, np.full(nb, 100.0), np.ones(nb), np.ones(nb, np.int64))
-        bl.sign = np.ones(nb, np.int32); bl.t_start = np.full(nb, 90, np.float32); bl.t_end = np.full(nb, 95, np.float32)
-        for state_in in (False, True):
-            ev = detect.detect_events(torch.from_numpy(y).cuda(), bl, state_in=state_in)
-            s, e, o = c_twin.detect_events(y, block, bl.sign, bl.t_start, bl.t_end, state_in=state_in)
-            assert ev.starts.tolist() == s.tolist() and ev.ends.tolist() == e.tolist() and ev.open_start == o
+    # end line 95 above the start line 90, and the two lines equal (hysteresis 0): a sample on 90 is then neither symbol
+    for t_end, values, p in ((95.0, [80, 92, 100], [0.02, 0.9, 0.08]), (90.0, [80, 90, 92, 100], [0.02, 0.05, 0.85, 0.08])):
+        rng = np.random.default_rng(5)
+        for n in (1, 31, 32, 33, 4095, 4096, 4097, 100000):
+            y = rng.choice(np.array(values, np.float32), size=n, p=p)
+            nb = (n + block - 1) // block
+            bl = detect.Baseline(block, np.full(nb, 100.0), np.ones(nb), np.ones(nb, np.int64))
+            bl.sign = np.ones(nb, np.int32); bl.t_start = np.full(nb, 90, np.float32); bl.t_end = np.full(nb, t_end, np.float32)
+            for state_in in (False, True):
+                ev = detect.detect_events(torch.from_numpy(y).cuda(), bl, state_in=state_in)
+                s, e, o = c_twin.detect_events(y, block, bl.sign, bl.t_start, bl.t_end, state_in=state_in)
+                assert ev.starts.tolist() == s.tolist() and ev.ends.tolist() == e.tolist() and ev.open_start == o, (t_end, n)
 
 
 @pytest.mark.parametrize("block,nb", [(4096, 37), (4096, 2500), (8192, 1)])
@@ -108,3 +110,39 @@ def test_blocks_without_baseline_samples_inherit_the_nearest_earlier_valid_block
     assert np.array_equal(bl.mean, mean) and np.array_equal(bl.std, std)
     sign, ts, te = eo.thresholds(mean, std, 5.0, 1.0)
     assert np.array_equal(bl.sign, sign) and np.array_equal(bl.t_start, ts) and np.array_equal(bl.t_end, te)
+
+
+@pytest.mark.parametrize("hysteresis", [-1.0, -1e-9, float("nan")])
+def test_baseline_finalize_rejects_crossed_lines(hysteresis):
+    """A negative hysteresis puts the end line beyond the start line, where the detector's definition does not hold:
+    ct_baseline_finalize refuses it before any launch and leaves every output as it was.  A NaN threshold (no lines
+    wanted) with hysteresis 0 still passes."""
+    L = _lib.lib()
+    nb = 5
+    cnt = torch.full((nb,), 100, dtype=torch.int64, device="cuda")
+    s1 = torch.zeros(nb, dtype=torch.int64, device="cuda"); s2 = torch.full((nb,), 400, dtype=torch.int64, device="cuda")
+    outs = [torch.full((nb,), -3.0, dtype=torch.float64, device="cuda"), torch.full((nb,), -3.0, dtype=torch.float64, device="cuda"),
+            torch.full((nb,), 7, dtype=torch.int32, device="cuda"), torch.full((nb,), -3.0, dtype=torch.float32, device="cuda"),
+            torch.full((nb,), -3.0, dtype=torch.float32, device="cuda"), torch.full((1,), 9, dtype=torch.int32, device="cuda")]
+    st = torch.cuda.current_stream().cuda_stream
+    args = lambda thr, hys: (cnt.data_ptr(), s1.data_ptr(), s2.data_ptr(), nb, 5000.0, 0, 16, thr, hys,
+                             *[t.data_ptr() for t in outs], st)
+    before = [t.clone() for t in outs]
+    assert L.ct_baseline_finalize(*args(5.0, hysteresis)) != 0
+    assert "hysteresis" in _lib.lib().ct_last_error().decode()
+    torch.cuda.synchronize()
+    assert all(torch.equal(a, b) for a, b in zip(outs, before))
+    assert L.ct_baseline_finalize(*args(float("nan"), 0.0)) == 0
+    assert L.ct_baseline_finalize(*args(5.0, 0.0)) == 0
+    torch.cuda.synchronize()
+    assert int(outs[5].item()) == 0 and torch.equal(outs[3], outs[4])
+
+
+def test_device_table_rejects_negative_hysteresis():
+    y = torch.full((1 << 16,), 5000.0, device="cuda")
+    bl = detect.baseline_blocks(y, 4096, 4700.0, 5300.0)
+    with pytest.raises(ValueError, match="hysteresis"):
+        bl.with_thresholds(5.0, -1.0)
+    with pytest.raises(ValueError, match="hysteresis"):
+        detect.intra_crossings(y, torch.zeros(1, dtype=torch.int64, device="cuda"), torch.ones(1, dtype=torch.int64, device="cuda"),
+                               torch.zeros(1, dtype=torch.int64, device="cuda"), bl, 50.0, -5.0)
