@@ -31,6 +31,11 @@ class CtFilterCoef(C.Structure):
 _vp, _i64, _i32, _f32, _u16, _u32 = C.c_void_p, C.c_int64, C.c_int32, C.c_float, C.c_uint16, C.c_uint32
 
 
+class CtMedianPlan(C.Structure):
+    _fields_ = [("bin", C.c_int64), ("dens", C.c_int64), ("total", C.c_int64), ("n", C.c_int64), ("se", C.c_double),
+                ("sub_code", C.c_float), ("est", C.c_uint32), ("lo", C.c_uint32), ("step", C.c_uint32)]
+
+
 class CtFilterStats(C.Structure):
     _fields_ = [("origin", C.c_int64), ("block", C.c_int64), ("bmin", C.c_float), ("bmax", C.c_float),
                 ("c0", C.c_float), ("shift", C.c_int32), ("cnt", C.c_void_p), ("s1", C.c_void_p), ("s2", C.c_void_p)]
@@ -50,6 +55,8 @@ SIGNATURES = {
     "ct_filtfilt_stats_granule": (_i64, [_i64, _i64, C.c_int]),
     "ct_filter_forward_u16": (C.c_int, [_vp, _i64, _i64, _f32, _u16, _f32, C.POINTER(CtFilterCoef), C.c_int, _i64, C.c_int,
                                         _u32, _u32, _i64, _i64, _vp, _i64, _i64, _vp, _i64, _vp]),
+    "ct_filter_forward_planned_u16": (C.c_int, [_vp, _i64, _i64, _vp, _u16, _f32, C.POINTER(CtFilterCoef), C.c_int, _i64,
+                                                C.c_int, _u32, _i64, _i64, _vp, _i64, _i64, _vp, _i64, _vp]),
     "ct_median_verify": (C.c_int, [_vp, C.c_int, _i64, _i64, _u32, _u32, _f32, _vp, _vp]),
     "ct_filter_forward_ends_u16": (C.c_int, [_vp, _i64, _i64, _f32, _u16, _vp, C.POINTER(CtFilterCoef), C.c_int, _i64, _vp, _i64,
                                              _vp]),
@@ -61,6 +68,7 @@ SIGNATURES = {
                                   C.c_int, _vp, _vp, _i64, C.POINTER(CtFilterStats), _vp]),
     "ct_hist_sampled_u16": (C.c_int, [_vp, _i64, _i64, _u16, _vp, _vp]),
     "ct_hist_rank": (C.c_int, [_vp, C.c_int, _vp, _vp]),
+    "ct_median_plan": (C.c_int, [_vp, C.c_int, C.c_int, _vp, _vp, _vp]),
     "ct_count_window_u16": (C.c_int, [_vp, _i64, _u16, _u32, _u32, _vp, _vp]),
     "ct_count_window4_u16": (C.c_int, [_vp, _i64, _u16, _u32, _u32, _vp, _vp]),
     "ct_block_stats_f32": (C.c_int, [_vp, _i64, _i64, _f32, _f32, _f32, C.c_int, _vp, _vp, _vp, _vp]),

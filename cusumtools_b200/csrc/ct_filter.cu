@@ -44,8 +44,26 @@ __global__ void __launch_bounds__(1024) ct_hist_sampled_kernel(const uint16_t* _
 // Rank search in a 65 536-bin histogram on the device: out[0] = first bin whose cumulative count reaches ceil(total / 2)
 // (the sampled median), out[1] = its count (the density that gives the estimate's standard error), out[2] = total.
 // One CTA of 1024 threads, 64 bins each; replaces a cumsum / searchsorted / gather chain of ten small launches.
-template <typename T>
-__global__ void __launch_bounds__(1024) ct_hist_rank_kernel(const T* __restrict__ hist, long long* __restrict__ out) {
+// PLAN: `out` is a CtMedianPlan, completed from the three values (median.estimate's arithmetic, se in correctly rounded
+// float64 as numpy computes it).
+__device__ void put_rank(long long* out, long long bin, long long dens, long long total) { out[0] = bin; out[1] = dens; out[2] = total; }
+__device__ void put_rank(CtMedianPlan* p, long long bin, long long dens, long long total, int shift, const long long* n_total) {
+    const unsigned step = 1u << shift, est = ((unsigned)bin >> shift) << shift;
+    p->bin = bin; p->dens = dens; p->total = total;
+    p->n = n_total ? *n_total : 0;
+    p->se = __ddiv_rn(0.5 * __dsqrt_rn((double)(total > 1 ? total : 1)), (double)(dens > 1 ? dens : 1));
+    p->sub_code = (float)est;
+    p->est = est;
+    p->lo = est > 3 * step ? est - 3 * step : 0u;
+    p->step = step;
+}
+template <typename T, bool PLAN>
+__global__ void __launch_bounds__(1024) ct_hist_rank_kernel(const T* __restrict__ hist, void* __restrict__ outp, int shift,
+                                                            const long long* __restrict__ n_total) {
+    auto put = [&](long long bin, long long dens, long long total) {
+        if (PLAN) put_rank(reinterpret_cast<CtMedianPlan*>(outp), bin, dens, total, shift, n_total);
+        else put_rank(reinterpret_cast<long long*>(outp), bin, dens, total);
+    };
     __shared__ long long part[1024];
     const int t = threadIdx.x;
     long long s = 0;
@@ -66,10 +84,10 @@ __global__ void __launch_bounds__(1024) ct_hist_rank_kernel(const T* __restrict_
         for (int k = 0; k < 64; ++k) {
             const long long h = (long long)hist[t * 64 + k];
             c += h;
-            if (c >= want) { out[0] = t * 64 + k; out[1] = h; out[2] = total; break; }
+            if (c >= want) { put(t * 64 + k, h, total); break; }
         }
     }
-    if (total == 0 && t == 0) { out[0] = 0; out[1] = 0; out[2] = 0; }
+    if (total == 0 && t == 0) put(0, 0, 0);
 }
 
 constexpr int kWin = 8;
@@ -222,7 +240,8 @@ int ct_filtfilt_seq(const void* in, int in_kind, int64_t n, int64_t pad, float s
 int ct_filter_forward_seq(const void* in, int in_kind, int64_t n, int64_t pad, float sub, uint16_t mask, float pad_x,
                           const CtFilterCoef* coef, int H, int64_t origin, int part, uint32_t cw_lo, uint32_t cw_step,
                           int64_t cw_begin, int64_t cw_end, uint64_t* counts9, int64_t from_pos, int64_t to_pos,
-                          void* workspace, int64_t workspace_bytes, const float* pad_x_dev, cudaStream_t st);
+                          void* workspace, int64_t workspace_bytes, const float* pad_x_dev, const CtMedianPlan* plan_dev,
+                          cudaStream_t st);
 int ct_filter_backward_seq(int64_t n, int64_t pad, float sub, float scale, float offset, const CtFilterCoef* coef, int H,
                            int64_t origin, float* out, const void* workspace, int64_t workspace_bytes,
                            const CtFilterStats* stats, float* summaries, cudaStream_t st);
@@ -235,7 +254,20 @@ int ct_filter_forward_u16(const uint16_t* raw, int64_t n, int64_t pad, float sub
                           int64_t to_pos, void* workspace, int64_t workspace_bytes, void* stream) {
     if (!raw || !coef || n <= 0 || pad < 0 || H < 0 || origin < 0) { ct_set_error("filter_forward: bad argument"); return CT_ERR_ARG; }
     return ct_filter_forward_seq(raw, 0, n, pad, sub_code, mask, pad_x, coef, H, origin, part, window_lo, window_step,
-                                 count_begin, count_end, counts9, from_pos, to_pos, workspace, workspace_bytes, nullptr,
+                                 count_begin, count_end, counts9, from_pos, to_pos, workspace, workspace_bytes, nullptr, nullptr,
+                                 (cudaStream_t)stream);
+}
+
+int ct_filter_forward_planned_u16(const uint16_t* raw, int64_t n, int64_t pad, const CtMedianPlan* plan, uint16_t mask,
+                                  float pad_x, const CtFilterCoef* coef, int H, int64_t origin, int part, uint32_t window_step,
+                                  int64_t count_begin, int64_t count_end, uint64_t* counts9, int64_t from_pos, int64_t to_pos,
+                                  void* workspace, int64_t workspace_bytes, void* stream) {
+    if (!raw || !plan || !coef || n <= 0 || pad < 0 || H < 0 || origin < 0) {
+        ct_set_error("filter_forward_planned: bad argument"); return CT_ERR_ARG;
+    }
+    // the window's first code is not known here: 0 stands for it in the host-side checks (plan->lo is a multiple of step)
+    return ct_filter_forward_seq(raw, 0, n, pad, 0.f, mask, pad_x, coef, H, origin, part, 0, window_step, count_begin,
+                                 count_end, counts9, from_pos, to_pos, workspace, workspace_bytes, nullptr, plan,
                                  (cudaStream_t)stream);
 }
 
@@ -246,7 +278,7 @@ int ct_filter_forward_ends_u16(const uint16_t* raw, int64_t n, int64_t pad, floa
         ct_set_error("filter_forward_ends: bad argument"); return CT_ERR_ARG;
     }
     return ct_filter_forward_seq(raw, 0, n, pad, sub_code, mask, 0.f, coef, H, origin, 1, 0, 1, 0, 0, nullptr, 0, 0, workspace,
-                                 workspace_bytes, pad_x_dev, (cudaStream_t)stream);
+                                 workspace_bytes, pad_x_dev, nullptr, (cudaStream_t)stream);
 }
 
 int ct_median_verify(const uint64_t* counts9, int nbins, int64_t k1, int64_t k2, uint32_t lo, uint32_t step, float sub_code,
@@ -327,8 +359,17 @@ static int count_window(const uint16_t* raw, int64_t n, uint16_t mask, uint32_t 
 int ct_hist_rank(const void* hist65536, int is_int64, int64_t* out3, void* stream) {
     if (!hist65536 || !out3) { ct_set_error("hist_rank: null pointer"); return CT_ERR_ARG; }
     CT_COUNT_LAUNCH();
-    if (is_int64) ct_hist_rank_kernel<long long><<<1, 1024, 0, (cudaStream_t)stream>>>((const long long*)hist65536, (long long*)out3);
-    else ct_hist_rank_kernel<unsigned><<<1, 1024, 0, (cudaStream_t)stream>>>((const unsigned*)hist65536, (long long*)out3);
+    if (is_int64) ct_hist_rank_kernel<long long, false><<<1, 1024, 0, (cudaStream_t)stream>>>((const long long*)hist65536, out3, 0, nullptr);
+    else ct_hist_rank_kernel<unsigned, false><<<1, 1024, 0, (cudaStream_t)stream>>>((const unsigned*)hist65536, out3, 0, nullptr);
+    return ct_check_launch("ct_hist_rank_kernel");
+}
+
+int ct_median_plan(const void* hist65536, int is_int64, int shift, const int64_t* n_total, CtMedianPlan* plan, void* stream) {
+    if (!hist65536 || !plan || shift < 0 || shift > 16) { ct_set_error("median_plan: null pointer or shift outside 0..16"); return CT_ERR_ARG; }
+    const long long* nt = reinterpret_cast<const long long*>(n_total);
+    CT_COUNT_LAUNCH();
+    if (is_int64) ct_hist_rank_kernel<long long, true><<<1, 1024, 0, (cudaStream_t)stream>>>((const long long*)hist65536, plan, shift, nt);
+    else ct_hist_rank_kernel<unsigned, true><<<1, 1024, 0, (cudaStream_t)stream>>>((const unsigned*)hist65536, plan, shift, nt);
     return ct_check_launch("ct_hist_rank_kernel");
 }
 

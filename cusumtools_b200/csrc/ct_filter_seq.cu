@@ -230,15 +230,15 @@ static __device__ __forceinline__ unsigned shl_clamp(unsigned v, unsigned amt) {
 // 1.53 / 1.54 / 1.65): the loop body with the tally is 235 instructions, and the instruction cache decides
 constexpr int kFwdUnroll = CT_FWD_UNROLL;
 struct CwAcc { unsigned tot[9], below, c4, ce, co; int since; };
-static __device__ __forceinline__ unsigned cw_amount(unsigned pat, const SeqArgs& a) { return pat * a.cw_k + a.cw_c; }
-static __device__ __forceinline__ void cw_tally2(unsigned pat0, unsigned pat1, const SeqArgs& a, CwAcc& w) {
-    const unsigned a0 = cw_amount(pat0, a), a1 = cw_amount(pat1, a);
+static __device__ __forceinline__ unsigned cw_amount(unsigned pat, const SeqArgs& a, unsigned cw_c) { return pat * a.cw_k + cw_c; }
+static __device__ __forceinline__ void cw_tally2(unsigned pat0, unsigned pat1, const SeqArgs& a, unsigned cw_c, CwAcc& w) {
+    const unsigned a0 = cw_amount(pat0, a, cw_c), a1 = cw_amount(pat1, a, cw_c);
     w.below += a0 >> 31;
     w.below += a1 >> 31;
     w.c4 += shl_clamp(1u, a0) + shl_clamp(1u, a1);
 }
-static __device__ __forceinline__ void cw_tally1(unsigned pat, const SeqArgs& a, CwAcc& w) {
-    const unsigned a0 = cw_amount(pat, a);
+static __device__ __forceinline__ void cw_tally1(unsigned pat, const SeqArgs& a, unsigned cw_c, CwAcc& w) {
+    const unsigned a0 = cw_amount(pat, a, cw_c);
     w.below += a0 >> 31;
     w.c4 += shl_clamp(1u, a0);
 }
@@ -329,7 +329,8 @@ static __device__ __forceinline__ long long next_group(const SeqArgs& a, long lo
 template <int NSEC, typename InT, int MODE, bool COUNT, bool EDGE>
 __device__ __forceinline__ void fwd_group(const SeqArgs& a, const CtFilterCoef& k, const CUtensorMap* in_map, const CUtensorMap* out_map,
                                           const long long g, const int lane, const unsigned stage0, const unsigned bar0,
-                                          const unsigned outb, unsigned& phase, const Coefs<NSEC>& cf, const float pad_x) {
+                                          const unsigned outb, unsigned& phase, const Coefs<NSEC>& cf, const float pad_x,
+                                          const int isub, const unsigned cw_c) {
     constexpr bool U16 = sizeof(InT) == 2;
     constexpr int SPT = U16 ? 1 : 2;             // stages per tile (a stage row is 128 bytes)
     constexpr int SLOTS = kG / SPT;              // slots per stage
@@ -341,7 +342,7 @@ __device__ __forceinline__ void fwd_group(const SeqArgs& a, const CtFilterCoef& 
     const int nstages = ntiles * SPT;
     const InT* in = reinterpret_cast<const InT*>(a.in);
     const unsigned m2 = a.mask | (a.mask << 16);
-    const f2 kmagic = splat(-(8388608.f + (float)a.isub));
+    const f2 kmagic = splat(-(8388608.f + (float)isub));
 
     constexpr int TAPS = 2 * NSEC + 1;              // binomial FIR taps (orders below 2 NSEC have zero tails)
     constexpr int HIST = TAPS - 1 > 8 ? 16 : 8;     // all-pole outputs of the previous slot(s) the FIR reaches back into
@@ -454,18 +455,18 @@ __device__ __forceinline__ void fwd_group(const SeqArgs& a, const CtFilterCoef& 
                         if (!cw_part) {
 #pragma unroll
                             for (int w = 0; w < 4; ++w) {
-                                cw_tally2(pl[w][0], ph[w][0], a, cw);
-                                cw_tally2(pl[w][1], ph[w][1], a, cw);
+                                cw_tally2(pl[w][0], ph[w][0], a, cw_c, cw);
+                                cw_tally2(pl[w][1], ph[w][1], a, cw_c, cw);
                                 if (w & 1) cw_spread(cw);      // 8 tallies
                             }
                         } else {
 #pragma unroll 1
                             for (int w = 0; w < 4; ++w) {
                                 const long long pa0 = lo0 + jj * 8 + 2 * w, pb0 = lo1 + jj * 8 + 2 * w;
-                                if (pa0 >= a.cw_p0 && pa0 < a.cw_p1) cw_tally1(pl[w][0], a, cw);
-                                if (pa0 + 1 >= a.cw_p0 && pa0 + 1 < a.cw_p1) cw_tally1(ph[w][0], a, cw);
-                                if (pb0 >= a.cw_p0 && pb0 < a.cw_p1) cw_tally1(pl[w][1], a, cw);
-                                if (pb0 + 1 >= a.cw_p0 && pb0 + 1 < a.cw_p1) cw_tally1(ph[w][1], a, cw);
+                                if (pa0 >= a.cw_p0 && pa0 < a.cw_p1) cw_tally1(pl[w][0], a, cw_c, cw);
+                                if (pa0 + 1 >= a.cw_p0 && pa0 + 1 < a.cw_p1) cw_tally1(ph[w][0], a, cw_c, cw);
+                                if (pb0 >= a.cw_p0 && pb0 < a.cw_p1) cw_tally1(pl[w][1], a, cw_c, cw);
+                                if (pb0 + 1 >= a.cw_p0 && pb0 + 1 < a.cw_p1) cw_tally1(ph[w][1], a, cw_c, cw);
                                 if (w & 1) cw_spread(cw);
                             }
                         }
@@ -560,12 +561,24 @@ __device__ __forceinline__ void fwd_group(const SeqArgs& a, const CtFilterCoef& 
 
 template <int NSEC, typename InT, int MODE, bool COUNT>
 __global__ void __launch_bounds__(kWarps * 32, kCtasPerSm)
-ct_filter_fwd_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_constant__ CUtensorMap out_map, SeqArgs a, CtFilterCoef k) {
+ct_filter_fwd_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_constant__ CUtensorMap out_map, SeqArgs a, CtFilterCoef k,
+                     const CtMedianPlan* __restrict__ plan) {
+    // plan (uint16, may be NULL): sub and the count window's first code come from the estimate on the device; isub = floor(sub),
+    // cw_c from lo, and the fraction of sub joins pad_x, as split_sub and the host do for the values passed in `a`.  (Its own
+    // argument: a field of SeqArgs would move the coefficients behind it off the alignment of their 128-bit constant loads.)
     extern __shared__ __align__(1024) unsigned char smem[];
     constexpr int kPerWarp = 2 * kStage + (MODE == 0 ? 2 * kStage : 0);
     const int lane = ct_lane();
     const int wib = threadIdx.x >> 5;
     float pad_x = a.pad_x;
+    int isub = a.isub;
+    unsigned cw_c = a.cw_c;
+    if (sizeof(InT) == 2 && plan) {
+        const float sub = __ldg(&plan->sub_code), fl = floorf(sub);
+        isub = (int)fl;
+        pad_x += sub - fl;
+        if (COUNT) cw_c = 0u - (0x4B000000u + __ldg(&plan->lo)) * a.cw_k;
+    }
     if (a.pad_x_dev) {                                       // the end groups re-run with the exact median's pad: a no-op when
         const float d = __ldg(a.pad_x_dev);                  // the estimate was the median
         if (d == 0.f) return;
@@ -594,8 +607,8 @@ ct_filter_fwd_kernel(const __grid_constant__ CUtensorMap in_map, const __grid_co
         bool interior = a.tma_in && p_lo >= 0 && p_hi <= a.n_in;
         if (MODE == 0) interior = interior && a.tma_out && p_hi <= a.n_out;
         if (COUNT) interior = interior && p_lo + a.Hw >= a.cw_p0 && p_hi <= a.cw_p1;
-        if (interior) fwd_group<NSEC, InT, MODE, COUNT, false>(a, k, &in_map, &out_map, g, lane, stage0, bar0, outb, phase, cf, pad_x);
-        else fwd_group<NSEC, InT, MODE, COUNT, true>(a, k, &in_map, &out_map, g, lane, stage0, bar0, outb, phase, cf, pad_x);
+        if (interior) fwd_group<NSEC, InT, MODE, COUNT, false>(a, k, &in_map, &out_map, g, lane, stage0, bar0, outb, phase, cf, pad_x, isub, cw_c);
+        else fwd_group<NSEC, InT, MODE, COUNT, true>(a, k, &in_map, &out_map, g, lane, stage0, bar0, outb, phase, cf, pad_x, isub, cw_c);
     }
     if (MODE == 0 && lane == 0) bulk_wait_read<0>();         // shared memory must outlive the last tile store
 }
@@ -912,13 +925,14 @@ long long grid_for(const void* kern, int smem, long long ngroups) {
 }
 
 template <int NSEC, typename InT, int MODE, bool COUNT>
-int launch_fwd(const SeqArgs& a, const CtFilterCoef& k, const CUtensorMap& im, const CUtensorMap& om, cudaStream_t st) {
+int launch_fwd(const SeqArgs& a, const CtFilterCoef& k, const CUtensorMap& im, const CUtensorMap& om, const CtMedianPlan* plan,
+               cudaStream_t st) {
     auto kern = ct_filter_fwd_kernel<NSEC, InT, MODE, COUNT>;
     const int smem = kWarps * (2 * kStage + (MODE == 0 ? 2 * kStage : 0)) + kWarps * 16;
     cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
     const long long grid = grid_for(reinterpret_cast<const void*>(kern), smem, a.ngroups - a.g_first);
     CT_COUNT_LAUNCH();
-    kern<<<(unsigned)grid, kWarps * 32, smem, st>>>(im, om, a, k);
+    kern<<<(unsigned)grid, kWarps * 32, smem, st>>>(im, om, a, k, plan);
     return ct_check_launch("ct_filter_fwd_kernel");
 }
 template <int NSEC, int D, bool STATS, bool SUMM>
@@ -944,11 +958,12 @@ int launch_bwd(const SeqArgs& a, const CtFilterCoef& k, const CUtensorMap& om, c
     return CT_ERR_ARG;
 
 template <typename InT, int MODE>
-int dispatch_fwd(const SeqArgs& a, const CtFilterCoef& k, const CUtensorMap& im, const CUtensorMap& om, cudaStream_t st) {
+int dispatch_fwd(const SeqArgs& a, const CtFilterCoef& k, const CUtensorMap& im, const CUtensorMap& om, cudaStream_t st,
+                 const CtMedianPlan* plan = nullptr) {
     if (sizeof(InT) == 2 && MODE != 0 && a.cw_out) {
-        CT_NSEC_SWITCH(k.nsec, (launch_fwd<NS, uint16_t, MODE == 0 ? 1 : MODE, true>(a, k, im, om, st)))
+        CT_NSEC_SWITCH(k.nsec, (launch_fwd<NS, uint16_t, MODE == 0 ? 1 : MODE, true>(a, k, im, om, plan, st)))
     }
-    CT_NSEC_SWITCH(k.nsec, (launch_fwd<NS, InT, MODE, false>(a, k, im, om, st)))
+    CT_NSEC_SWITCH(k.nsec, (launch_fwd<NS, InT, MODE, false>(a, k, im, om, plan, st)))
 }
 template <int D>
 int dispatch_bwd(const SeqArgs& a, const CtFilterCoef& k, const CUtensorMap& om, cudaStream_t st) {
@@ -1074,15 +1089,19 @@ void split_sub(SeqArgs& a, float sub, float pad_x) {
 // Forward pass into the scratch.  in_kind: 0 = uint16 codes, 1 = float32 samples.  part: 0 = whole
 // trace, 1 = only the groups whose result depends on pad_x (the two ends of the trace), 2 = streaming.
 // counts9 != NULL (uint16 only, part 0/2): also tally the window count for the exact median.
+// plan_dev != NULL (uint16 only): sub and cw_lo are read from it on the device, the values passed here are ignored.
 int ct_filter_forward_seq(const void* in, int in_kind, int64_t n, int64_t pad, float sub, uint16_t mask, float pad_x,
                           const CtFilterCoef* coef, int H, int64_t origin, int part, uint32_t cw_lo, uint32_t cw_step,
                           int64_t cw_begin, int64_t cw_end, uint64_t* counts9, int64_t from_pos, int64_t to_pos,
-                          void* workspace, int64_t workspace_bytes, const float* pad_x_dev, cudaStream_t st) {
+                          void* workspace, int64_t workspace_bytes, const float* pad_x_dev, const CtMedianPlan* plan_dev,
+                          cudaStream_t st) {
     int rc = check_ws(workspace, workspace_bytes, n, pad, H); if (rc) return rc;
     const Plan p = make_plan(n, pad, H, origin);
     SeqArgs a; init_args(a);
     a.in = in; a.n_in = n; a.mask = mask; a.Hw = p.Hw; a.R = p.R; a.base = p.base;
-    if (in_kind == 0) split_sub(a, sub, pad_x); else { a.fsub = sub; a.pad_x = pad_x; }
+    if (plan_dev) { a.pad_x = pad_x; cw_lo = 0; }        // the kernel does the rest of split_sub and of cw_c
+    else if (in_kind == 0) split_sub(a, sub, pad_x);
+    else { a.fsub = sub; a.pad_x = pad_x; }
     a.out = reinterpret_cast<float*>(workspace);
     a.pad_x_dev = part == 1 ? pad_x_dev : nullptr;
     a.scratch_floats = (ct_filtfilt_workspace_bytes(n, pad, H) - 256) / 4;
@@ -1110,9 +1129,9 @@ int ct_filter_forward_seq(const void* in, int in_kind, int64_t n, int64_t pad, f
             if (D == 2) return dispatch_fwd<float, 2>(x, *coef, im, om, st);
             return dispatch_fwd<float, 1>(x, *coef, im, om, st);
         }
-        if (D == 4) return dispatch_fwd<uint16_t, 4>(x, *coef, im, om, st);
-        if (D == 2) return dispatch_fwd<uint16_t, 2>(x, *coef, im, om, st);
-        return dispatch_fwd<uint16_t, 1>(x, *coef, im, om, st);
+        if (D == 4) return dispatch_fwd<uint16_t, 4>(x, *coef, im, om, st, plan_dev);
+        if (D == 2) return dispatch_fwd<uint16_t, 2>(x, *coef, im, om, st, plan_dev);
+        return dispatch_fwd<uint16_t, 1>(x, *coef, im, om, st, plan_dev);
     };
     if (part == 0) { a.g_first = 0; a.ngroups = p.ng_fwd; return go(a); }
     if (part == 2) {
@@ -1194,7 +1213,7 @@ int ct_filtfilt_seq(const void* in, int in_kind, int64_t n, int64_t pad, float s
     }
     const int64_t origin = stats ? stats->origin : 0;
     int rc = ct_filter_forward_seq(in, in_kind, n, pad, sub, mask, 0.f, coef, H, origin, 0, 0, 1, 0, 0, nullptr, 0, 0, workspace,
-                                   workspace_bytes, nullptr, st);
+                                   workspace_bytes, nullptr, nullptr, st);
     if (rc) return rc;
     return ct_filter_backward_seq(n, pad, in_kind == 0 ? sub : 0.f, scale, offset, coef, H, origin, out, workspace, workspace_bytes,
                                   stats, nullptr, st);

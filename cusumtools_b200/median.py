@@ -48,14 +48,58 @@ class MedianPlan:
     se: float = float("inf")    # standard error of the estimate in code steps: sqrt(sampled) / (2 x samples at the estimate)
 
 
+def mask_step(mask: int) -> tuple[int, int]:
+    """(shift, step): the spacing of the masked codes, step = 1 << shift."""
+    shift = 0
+    while shift < 16 and not (mask >> shift) & 1:
+        shift += 1
+    return shift, 1 << shift
+
+
+class PlanBuffer:
+    """Where the device rank search leaves its CtMedianPlan (`dev`, read by ct_filter_forward_planned_u16) and the pinned
+    host copy the host reads it from; reusable from one estimate to the next."""
+
+    def __init__(self, device):
+        nbytes = C.sizeof(_lib.CtMedianPlan)
+        self.dev = torch.empty(nbytes, dtype=torch.uint8, device=device)
+        self.host = torch.empty(nbytes, dtype=torch.uint8, pin_memory=True)
+        self.copied = torch.cuda.Event()
+
+
+class Estimate:
+    """Phase 1 under way.  `plan_dev`: the device CtMedianPlan the stream holds once the rank search has run (None when
+    the estimate was made on the host); `result()` waits for its host copy only, so kernels that take `plan_dev` can be
+    queued before it."""
+
+    def __init__(self, plan: MedianPlan | None = None, buf: PlanBuffer | None = None, n: int | None = None,
+                 shift: int = 0, step: int = 1):
+        self._plan, self._buf, self._n, self._shift, self._step = plan, buf, n, shift, step
+        self.plan_dev = buf.dev if buf is not None else None
+
+    def result(self) -> MedianPlan:
+        if self._plan is None:
+            self._buf.copied.synchronize()
+            p = _lib.CtMedianPlan.from_buffer_copy(self._buf.host.numpy())
+            n = self._n if self._n is not None else int(p.n)
+            if n == 0:
+                raise ValueError("median of an empty trace")
+            self._plan = MedianPlan(n, (n - 1) // 2, n // 2, self._step, self._shift, int(p.est), int(p.lo), se=float(p.se))
+        return self._plan
+
+
 def estimate(n_local: int, mask: int, hist_fn, group=None, n_sampled: int | None = None) -> MedianPlan:
     """Phase 1: a strided-sample histogram (summed over `group`) locates the median code.  `n_sampled`:
     the histogram covers only that many of the rank's samples (streaming: the first chunk), so it
     is an estimate even for small traces."""
-    shift = 0
-    while shift < 16 and not (mask >> shift) & 1:
-        shift += 1
-    step = 1 << shift
+    return estimate_start(n_local, mask, hist_fn, group, n_sampled).result()
+
+
+def estimate_start(n_local: int, mask: int, hist_fn, group=None, n_sampled: int | None = None,
+                   buf: PlanBuffer | None = None) -> Estimate:
+    """`estimate` without waiting for its result: a device histogram is ranked on the device into `buf` (or a new
+    PlanBuffer), which is then copied to the host behind an event."""
+    shift, step = mask_step(mask)
     if group is None:
         n = int(n_local)
         if n == 0:
@@ -79,29 +123,30 @@ def estimate(n_local: int, mask: int, hist_fn, group=None, n_sampled: int | None
         cdf = torch.cumsum(hist.to(torch.int64), 0)
         want = torch.tensor([k1 + 1, k2 + 1], dtype=torch.int64, device=cdf.device)
         c1, c2 = (int(v) for v in torch.searchsorted(cdf, want).tolist())
-        return MedianPlan(n, k1, k2, step, shift, c1, max(0, c1 - 3 * step), exact=(c1, c2))
-    # the rank search runs where the histogram lives: 24 (32) bytes come back instead of 65 536 bins
+        return Estimate(MedianPlan(n, k1, k2, step, shift, c1, max(0, c1 - 3 * step), exact=(c1, c2)))
+    # the rank search runs where the histogram lives: a 56-byte CtMedianPlan comes back instead of 65 536 bins (with the
+    # total of all ranks in it: one read); ct_median_plan computes est, lo and se as the host branch below does
     if hist.is_cuda and hist.dtype in (torch.int32, torch.int64) and hist.is_contiguous():
-        out = torch.empty(3, dtype=torch.int64, device=hist.device)
+        buf = buf if buf is not None else PlanBuffer(hist.device)
         with torch.cuda.device(hist.device):
-            rc = _lib.lib().ct_hist_rank(hist.data_ptr(), int(hist.dtype == torch.int64), out.data_ptr(), _stream(hist))
-        _lib.check(rc, "ct_hist_rank")
-        vals = (torch.cat((out, packed[-1:])) if n is None else out).tolist()
-        i, dens, total = (int(v) for v in vals[:3])
-        if n is None:
-            n = int(vals[3])
-    else:                                                  # (CPU tensors: the gloo tests of the host logic)
-        hist = hist.to(torch.int64)
-        cdf = torch.cumsum(hist, 0)
-        idx = torch.searchsorted(cdf, (cdf[-1:] + 1) // 2).clamp_(max=hist.numel() - 1)
-        i, dens, total = (int(v) for v in torch.cat((idx, hist[idx], cdf[-1:])).tolist())
+            rc = _lib.lib().ct_median_plan(hist.data_ptr(), int(hist.dtype == torch.int64), shift,
+                                           packed[-1:].data_ptr() if n is None else None, buf.dev.data_ptr(), _stream(hist))
+            _lib.check(rc, "ct_median_plan")
+            buf.host.copy_(buf.dev, non_blocking=True)
+            buf.copied.record()
+        return Estimate(buf=buf, n=n, shift=shift, step=step)
+    # (CPU tensors: the gloo tests of the host logic)
+    hist = hist.to(torch.int64)
+    cdf = torch.cumsum(hist, 0)
+    idx = torch.searchsorted(cdf, (cdf[-1:] + 1) // 2).clamp_(max=hist.numel() - 1)
+    i, dens, total = (int(v) for v in torch.cat((idx, hist[idx], cdf[-1:])).tolist())
     if n == 0:
         raise ValueError("median of an empty trace")
     k1, k2 = (n - 1) // 2, n // 2
     est = (i >> shift) * step
     # the sample median of m samples with density f at the median has s.e. 1 / (2 f sqrt(m)); f = dens / m per code step
     se = 0.5 * float(np.sqrt(max(total, 1))) / max(dens, 1)
-    return MedianPlan(n, k1, k2, step, shift, est, max(0, est - 3 * step), se=se)
+    return Estimate(MedianPlan(n, k1, k2, step, shift, est, max(0, est - 3 * step), se=se))
 
 
 def verify(plan: MedianPlan, counts9, group=None):
@@ -167,10 +212,11 @@ def verify_on_device(plan: MedianPlan, counts: torch.Tensor, nbins: int, result:
     _lib.check(rc, "ct_median_verify")
 
 
-def device_counters(raw: torch.Tensor, mask: int):
-    """(hist_fn, count_fn) of `search` over the codes of `raw` (this rank's owned samples)."""
+def device_counters(raw: torch.Tensor, mask: int, hist: torch.Tensor | None = None):
+    """(hist_fn, count_fn) of `search` over the codes of `raw` (this rank's owned samples).  `hist`: an int32[65536]
+    device buffer that hist_fn zeroes and fills (each histogram is consumed on the stream before the next is made)."""
     def hist_fn(stride):
-        h = torch.zeros(65536, dtype=torch.int32, device=raw.device)
+        h = torch.zeros(65536, dtype=torch.int32, device=raw.device) if hist is None else hist.zero_()
         if raw.numel():
             _lib.check(_lib.lib().ct_hist_sampled_u16(raw.data_ptr(), raw.numel(), stride, mask, h.data_ptr(), _stream(raw)),
                        "ct_hist_sampled_u16")

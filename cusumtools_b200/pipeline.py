@@ -113,8 +113,11 @@ class AnalysisResult:
 
 
 class TraceAnalyzer:
-    """Stages 1-3 over a time shard with every buffer allocated once and a single host
-    synchronisation at the end of the step (the median needs two small ones up front).
+    """Stages 1-3 over a time shard with every buffer allocated once and no idle GPU waiting for
+    the host: the median's estimate is read while the forward filter pass that already uses it
+    runs, and the step's counts while CUSUM+ runs.  `run` may therefore return before the last
+    kernels of the step have finished; its tensors are ready in stream order (as for any CUDA
+    work), and a host copy such as `.cpu()` or `tables_to_host` waits for them.
 
     `raw_ext` = [lo_halo | owned | hi_halo] codes.  The filter runs over the extended range
     (its constant pad only matters at the true ends of the trace), and so do the baseline
@@ -184,6 +187,13 @@ class TraceAnalyzer:
         self.fuse_stats = (bool(fuse_stats) and self.block >= 65536
                            and self.block % filters.stats_granule(self.n_ext, self.padding, self.design) == 0)
         self.fused_count = bool(fused_count)     # the exact-median window tally rides on the forward pass (+0.35 ms against 0.79 ms as its own kernel on C2)
+        self.coef = filters.make_coef(self.design)
+        self.alpha = filters.chimera_affine(settings)[0]
+        self.step = median.mask_step(self.mask)[1]
+        self.hist = torch.empty(65536, dtype=torch.int32, device=self.device)   # the estimate's sampled histogram
+        self.plan_buf = None                                                    # and its rank search (median.PlanBuffer)
+        self.counts = torch.empty(9, dtype=torch.int64, device=self.device)     # the exact median's window counts
+        self._pad_value = (None, 0.0)                                           # (codes, pad value) of the last step
         self.filter_ws = None
         self.minmax = None                         # (min, max) of every 64-sample chunk of y, left by the backward pass
         self.H = max(1, self.design.impulse_tail(filters.DEFAULT_HALO_EPS))
@@ -259,11 +269,14 @@ class TraceAnalyzer:
         st = filters._stream_ptr(raw_ext)
         cur = torch.cuda.current_stream(self.device)
         # ---- median, phase 1: estimate (subtraction constant of the filter, verification window)
-        hist_fn, count_fn = median.device_counters(owned, self.mask)
+        hist_fn, count_fn = median.device_counters(owned, self.mask, self.hist)
+        pending = None
         if _fixed is not None:
             plan = _fixed[0]
         elif _arrivals is None:
-            plan = median.estimate(n_own, self.mask, hist_fn, self.group)
+            if self.plan_buf is None:
+                self.plan_buf = median.PlanBuffer(self.device)
+            pending = median.estimate_start(n_own, self.mask, hist_fn, self.group, buf=self.plan_buf)
         else:                                                  # only the first chunk has arrived: estimate from it
             bounds, events = _arrivals
             cur.wait_event(events[0])
@@ -272,33 +285,49 @@ class TraceAnalyzer:
                                    n_sampled=first.numel())
         hook("median")
         if self.filter_ws is None:
+            self.host_read = torch.empty(10, dtype=torch.int64, pin_memory=True)   # the step's read (see the detection stage)
+            self.host_read_done = torch.cuda.Event()
             need = int(L.ct_filtfilt_workspace_bytes(self.n_ext, self.padding, self.H))
             self.filter_ws = torch.empty(need, dtype=torch.uint8, device=self.device)
             self.minmax = torch.empty(2 * int(L.ct_filter_summary_count(self.n_ext, self.padding, self.H)), dtype=torch.float32,
                                       device=self.device)
-        coef = filters.make_coef(self.design)
-        alpha, _ = filters.chimera_affine(self.settings)
+        coef = self.coef
         origin = 0
         # ---- forward pass with the estimate; it tallies the window counts of the owned codes on the side
-        route = median.route(plan, fixed=_fixed is not None, streamed=_arrivals is not None, fused_count=self.fused_count)
-        plan.lo = route.lo
-        counts = torch.zeros(9, dtype=torch.int64, device=self.device) if route.count else None
-        pieces = [(0, 0, self.n_ext)] if _arrivals is None else [(2, a, b) for a, b in zip(_arrivals[0][:-1], _arrivals[0][1:])]
-        pad_first = float(_fixed[1]) if _fixed is not None else 0.0
-        for i, (part, a, b) in enumerate(pieces):
-            if _arrivals is not None:
-                cur.wait_event(_arrivals[1][i])
-            rc = L.ct_filter_forward_u16(raw_ext.data_ptr(), self.n_ext, self.padding, float(plan.est), self.mask, pad_first,
-                                         C.byref(coef), self.H, origin, part, plan.lo, plan.step, lo, lo + n_own,
-                                         counts.data_ptr() if route.count == "ride" else None, a, b,
-                                         self.filter_ws.data_ptr(), self.filter_ws.numel(), st)
-            _lib.check(rc, "ct_filter_forward_u16")
-            if route.count == "kernel":            # the window count of this piece's owned codes as its own kernel
-                median.count_window(raw_ext[max(a, lo):min(b, lo + n_own)], self.mask, plan.lo, plan.step, counts, route.nbins)
-        # everything the backward launch needs that does not depend on the exact median is prepared BEFORE the host waits
-        # for the counts: the GPU idles from the end of the forward pass to the backward launch
+        # An estimate ranked on the device whose eight-code window can ride on the pass needs nothing from the host: the
+        # pass reads it there and is queued before the host waits for its copy, so no idle GPU between the two.
+        planned = pending is not None and pending.plan_dev is not None and self.fused_count and self.step <= 4
+        if planned:
+            counts = self.counts.zero_()
+            rc = L.ct_filter_forward_planned_u16(raw_ext.data_ptr(), self.n_ext, self.padding, pending.plan_dev.data_ptr(),
+                                                 self.mask, 0.0, C.byref(coef), self.H, origin, 0, self.step, lo, lo + n_own,
+                                                 counts.data_ptr(), 0, 0, self.filter_ws.data_ptr(), self.filter_ws.numel(), st)
+            _lib.check(rc, "ct_filter_forward_planned_u16")
+        else:
+            plan = pending.result() if pending is not None else plan
+            route = median.route(plan, fixed=_fixed is not None, streamed=_arrivals is not None, fused_count=self.fused_count)
+            plan.lo = route.lo
+            counts = self.counts.zero_() if route.count else None
+            pieces = [(0, 0, self.n_ext)] if _arrivals is None else [(2, a, b) for a, b in zip(_arrivals[0][:-1], _arrivals[0][1:])]
+            pad_first = float(_fixed[1]) if _fixed is not None else 0.0
+            for i, (part, a, b) in enumerate(pieces):
+                if _arrivals is not None:
+                    cur.wait_event(_arrivals[1][i])
+                rc = L.ct_filter_forward_u16(raw_ext.data_ptr(), self.n_ext, self.padding, float(plan.est), self.mask, pad_first,
+                                             C.byref(coef), self.H, origin, part, plan.lo, plan.step, lo, lo + n_own,
+                                             counts.data_ptr() if route.count == "ride" else None, a, b,
+                                             self.filter_ws.data_ptr(), self.filter_ws.numel(), st)
+                _lib.check(rc, "ct_filter_forward_u16")
+                if route.count == "kernel":            # the window count of this piece's owned codes as its own kernel
+                    median.count_window(raw_ext[max(a, lo):min(b, lo + n_own)], self.mask, plan.lo, plan.step, counts, route.nbins)
+        # what the backward launch needs is prepared while the forward pass runs, before the host waits for anything
         bl = detect.new_baseline(self.n_det, self.block, self.bmin, self.bmax, self.device) if self.fuse_stats else None
         stats = detect.stats_args(bl, origin=0) if bl is not None else None
+        if planned:
+            plan = pending.result()
+            # the counts are those of the window est - 3 .. est + 4 either way: verified on the device, or the first
+            # counts of the host loop when the estimate is too uncertain for the window (se > 0.8)
+            route = median.route(plan)
         offset = float(filters.scale_codes_host(np.array([plan.est], dtype=np.uint16), self.settings)[0])
         # ---- median, phase 2: exact order statistics
         on_device = route.device and not _host_median
@@ -326,7 +355,7 @@ class TraceAnalyzer:
                                              self.filter_ws.data_ptr(), self.filter_ws.numel(), st)
                 _lib.check(rc, "ct_filter_forward_u16")
         y = self.y
-        rc = L.ct_filter_backward(self.n_ext, self.padding, float(plan.est), float(alpha), offset, C.byref(coef), self.H, origin,
+        rc = L.ct_filter_backward(self.n_ext, self.padding, float(plan.est), float(self.alpha), offset, C.byref(coef), self.H, origin,
                                   y.data_ptr(), self.filter_ws.data_ptr(), self.filter_ws.numel(),
                                   C.byref(stats) if stats is not None else None, self.minmax.data_ptr(), st)
         _lib.check(rc, "ct_filter_backward")
@@ -351,6 +380,14 @@ class TraceAnalyzer:
                                     self.w1.data_ptr(), self.typ.data_ptr(), sc[2:].data_ptr(), st)
             _lib.check(rc, "ct_event_windows")
             hook("detect")
+            # the step's one read: the counts, the baseline status, the start of an event still open at the end and the
+            # device median are final here.  They leave now and the host waits for them while CUSUM+ runs, so the host's
+            # work after the read and the next step's first launches queue behind CUSUM+ instead of finding the GPU idle.
+            tail = (self.median_result.to(torch.int64),) if on_device else ()
+            last = self.starts.index_select(0, sc[1:2].clamp(max=self.cap - 1))
+            read = torch.cat((sc[:4], bl.dev["status"].to(torch.int64), last) + tail)
+            self.host_read[:read.numel()].copy_(read, non_blocking=True)
+            self.host_read_done.record()
             if self.stepfit_samples:             # before CUSUM+, which then skips the short events
                 stepfit.select_short(self.w0, self.w1, self.typ, padding=self.event_padding,
                                      stepfit_samples=self.stepfit_samples, n_events_dev=sc[2:])
@@ -378,18 +415,21 @@ class TraceAnalyzer:
                                        self.intra_hysteresis, max_pairs=self.max_crossings, n_events_dev=sc[2:],
                                        out=self.intra)
             hook("cusum")
-            tail = (self.median_result.to(torch.int64),) if on_device else ()
-            host = torch.cat((sc[:4], bl.dev["status"].to(torch.int64)) + tail).cpu().numpy()   # the step's one sync
+            self.host_read_done.synchronize()
+            host = self.host_read.tolist()
             if on_device:
-                if int(host[8]) != 0:                # the four-code window missed the median (every rank sees the same counts)
+                if host[9] != 0:                     # the four-code window missed the median (every rank sees the same counts)
                     return self._run(raw_ext, stage_hook, _arrivals, _fixed, _host_median=True)
-                c1, c2 = int(host[5]), int(host[6])
+                c1, c2 = host[6], host[7]
             ns, ne, nk, i0 = int(host[0]), int(host[1]), int(host[2]), int(host[3])
             if max(ns, ne) <= self.cap:
                 break
             self._alloc_events(max(ns, ne))          # more events than planned: grow and redo stages 2-3
         self.last_median = (c1, c2)
-        pad_value = float(np.median(filters.scale_codes_host(np.array([c1, c2], dtype=np.uint16), self.settings)))
+        if self._pad_value[0] != (c1, c2):          # host arithmetic while the GPU idles: only when the median moved
+            self._pad_value = ((c1, c2), float(np.median(filters.scale_codes_host(np.array([c1, c2], dtype=np.uint16),
+                                                                                  self.settings))))
+        pad_value = self._pad_value[1]
         status = int(host[4]) != 0
         if _fixed is None:
             # the error decision is collective: the flag rides with the event counts, then every rank raises
@@ -402,7 +442,7 @@ class TraceAnalyzer:
         bl._checked = True
         open_start = -1
         if ns > ne:                                   # an event still open at the end of the data
-            o = int(self.starts[ne].item()) - lo
+            o = host[5] - lo
             open_start = o if 0 <= o < n_own else -1
         # event indices are reported relative to the first owned sample
         ev = detect.EventList(self.starts[i0:i0 + nk] - lo, self.ends[i0:i0 + nk] - lo, open_start)

@@ -147,6 +147,27 @@ int ct_hist_sampled_u16(const uint16_t* raw, int64_t n, int64_t stride, uint16_t
  * (the sampled median), out3[1] = its count, out3[2] = the total.  hist65536: uint32[65536], or int64[65536] (is_int64)
  * after an all_reduce over ranks. */
 int ct_hist_rank(const void* hist65536, int is_int64, int64_t* out3, void* stream);
+/* The same rank search, leaving in device memory what the two filter passes and the verification need from the estimate,
+ * so that the forward pass can be queued behind it before the host has read anything (ct_filter_forward_planned_u16).
+ * shift: log2 of the masked codes' spacing (0..16); n_total (may be NULL): device int64, copied to `n` (the sample count
+ * of all ranks, which travels with the histogram's all_reduce). */
+typedef struct CtMedianPlan {
+    int64_t bin, dens, total;  /* as out3 of ct_hist_rank */
+    int64_t n;                 /* *n_total, 0 without it */
+    double se;                 /* standard error of the estimate in code steps: 0.5 sqrt(max(total, 1)) / max(dens, 1) */
+    float sub_code;            /* est: what the forward pass subtracts */
+    uint32_t est;              /* (bin >> shift) << shift */
+    uint32_t lo;               /* first code of the eight-code window: max(0, est - 3 step) */
+    uint32_t step;             /* 1 << shift */
+} CtMedianPlan;
+int ct_median_plan(const void* hist65536, int is_int64, int shift, const int64_t* n_total, CtMedianPlan* plan, void* stream);
+/* ct_filter_forward_u16 with sub_code and window_lo read from `plan` on the device (once per CTA) instead of passed by
+ * value; window_step must be plan->step (every masked code a multiple of it: the entry checks the mask).  Same scratch
+ * and counts as the by-value entry given plan->sub_code and plan->lo. */
+int ct_filter_forward_planned_u16(const uint16_t* raw, int64_t n, int64_t pad, const CtMedianPlan* plan, uint16_t mask,
+                                  float pad_x, const CtFilterCoef* coef, int H, int64_t origin, int part, uint32_t window_step,
+                                  int64_t count_begin, int64_t count_end, uint64_t* counts9, int64_t from_pos, int64_t to_pos,
+                                  void* workspace, int64_t workspace_bytes, void* stream);
 int ct_count_window_u16(const uint16_t* raw, int64_t n, uint16_t mask, uint32_t lo, uint32_t step,
                         uint64_t* counts9, void* stream);
 int ct_count_window4_u16(const uint16_t* raw, int64_t n, uint16_t mask, uint32_t lo, uint32_t step,
