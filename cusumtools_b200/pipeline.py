@@ -193,6 +193,9 @@ class TraceAnalyzer:
         self.hist = torch.empty(65536, dtype=torch.int32, device=self.device)   # the estimate's sampled histogram
         self.plan_buf = None                                                    # and its rank search (median.PlanBuffer)
         self.counts = torch.empty(9, dtype=torch.int64, device=self.device)     # the exact median's window counts
+        # CtMedianResult of the device route: code1, code2, pad_x (float bits), status.  Written once per step, before the
+        # detection loop, and read on every pass of it: it must outlive a regrowth of the event buffers.
+        self.median_result = torch.zeros(4, dtype=torch.int32, device=self.device)
         self._pad_value = (None, 0.0)                                           # (codes, pad value) of the last step
         self.filter_ws = None
         self.minmax = None                         # (min, max) of every 64-sample chunk of y, left by the backward pass
@@ -210,7 +213,6 @@ class TraceAnalyzer:
         self.w1 = torch.empty(cap, dtype=torch.int64, device=dev)
         self.typ = torch.empty(cap, dtype=torch.int32, device=dev)
         self.scalars = torch.zeros(4, dtype=torch.int64, device=dev)     # n_starts, n_ends, n_kept, first kept index
-        self.median_result = torch.zeros(4, dtype=torch.int32, device=dev)   # CtMedianResult: code1, code2, pad_x (float bits), status
         self.intra = ((torch.zeros(cap, dtype=torch.int32, device=dev),
                        torch.full((cap, 2 * self.max_crossings), -1, dtype=torch.int32, device=dev))
                       if self.intra_threshold > 0 else None)

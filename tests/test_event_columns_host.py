@@ -68,8 +68,12 @@ def test_rows_are_views_of_the_capacity_buffers():
         part, whole = getattr(fit, f), getattr(an.fit, f)
         assert part.data_ptr() == whole.data_ptr() and part.shape == (NK,) + whole.shape[1:], f
     assert an.fit.status.data_ptr() == an.typ.data_ptr() and an.fit.levels is None and fit.levels is None
-    # more events than planned: the tables grow with the other event buffers, the fit status is still the type column
+    # more events than planned: the tables grow with the other event buffers, the fit status is still the type column;
+    # the device median, written before the detection loop, is not an event buffer and survives (held here, so that a
+    # new tensor at the freed address cannot pass)
+    median_result = an.median_result
     an._alloc_events(2 * CAP)
+    assert an.median_result is median_result
     assert an.levels.n_levels.shape == (2 * CAP,) and an.levels.edges.shape == (2 * CAP, ML + 1)
     assert an.fit.params.shape == (2 * CAP, 6) and an.fit.status.data_ptr() == an.typ.data_ptr()
     assert an.intra[1].shape == (2 * CAP, 2 * K) and torch.all(an.intra[1] == -1) and torch.all(an.intra[0] == 0)
