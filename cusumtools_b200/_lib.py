@@ -78,7 +78,7 @@ SIGNATURES = {
     "ct_welch_workspace_bytes": (_i64, [_i32, _i32]),
     "ct_welch_f32": (C.c_int, [_vp, _i64, _i32, _f32, _i32, _i32, _vp, _i64, _vp, _vp, _vp]),
     "ct_bin_be_f64_to_f32": (C.c_int, [_vp, _i64, _vp, _vp]),
-    "ct_i2be_to_f32": (C.c_int, [_vp, _i64, _f32, _vp, _vp]),
+    "ct_i2be_to_f32": (C.c_int, [_vp, _i64, C.c_double, _vp, _vp]),
     "ct_dequant_u16": (C.c_int, [_vp, _i64, _u16, C.c_double, C.c_double, _vp, _vp]),
     "ct_radix_hist_f32": (C.c_int, [_vp, _i64, _u32, _i32, _i32, _vp, _vp]),
     "ct_baseline_finalize": (C.c_int, [_vp, _vp, _vp, _i64, _f32, C.c_int, _i64, C.c_double, C.c_double, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),

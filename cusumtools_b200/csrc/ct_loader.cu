@@ -22,13 +22,14 @@ __global__ void bin_be_kernel(const uint4* __restrict__ rec, long long n, float*
         out[i] = (float)__hiloint2double((int)hi, (int)lo);
     }
 }
-__global__ void i2be_kernel(const unsigned* __restrict__ rec, long long n, float gain, float* __restrict__ out) {
+// savegain * current is a float64 product in the reference: rounded once to float32 here, not through a float32 gain
+__global__ void i2be_kernel(const unsigned* __restrict__ rec, long long n, double gain, float* __restrict__ out) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long st = (long long)gridDim.x * blockDim.x;
     for (; i < n; i += st) {
         unsigned r = rec[i];                              // bytes 0-1: big-endian int16 current
         short v = (short)(((r & 0xffu) << 8) | ((r >> 8) & 0xffu));
-        out[i] = gain * (float)v;
+        out[i] = (float)(gain * (double)v);
     }
 }
 __global__ void dequant_kernel(const uint16_t* __restrict__ raw, long long n, unsigned mask, double alpha,
@@ -87,7 +88,7 @@ int ct_bin_be_f64_to_f32(const void* records, int64_t n, float* out, void* strea
     bin_be_kernel<<<(unsigned)grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>((const uint4*)records, n, out);
     return ct_check_launch("bin_be_kernel");
 }
-int ct_i2be_to_f32(const void* records, int64_t n, float gain, float* out, void* stream) {
+int ct_i2be_to_f32(const void* records, int64_t n, double gain, float* out, void* stream) {
     if (!records || !out || n < 0 || (reinterpret_cast<uintptr_t>(records) & 3)) { ct_set_error("i2: bad argument / unaligned"); return CT_ERR_ARG; }
     if (n == 0) return CT_OK;
     CT_COUNT_LAUNCH();

@@ -350,13 +350,14 @@ int ct_welch_single_f32(const float* x, int64_t n, double mean, int32_t use_abs,
 /* ---- loaders: the byte formats either side of the path ---------------------------
  * ".bin" records (>f8 curr_pA, >f8 volt_mV), print_trace.py:33-34 / noise-fit.py:90-91:
  * n records of 16 bytes -> float32 current.  Legacy (>i2, >i2) records times savegain,
- * legacy/minimal_psd.py:188-193.  ct_dequant_u16 is plot-trace.py:272-287 alone (float64
- * affine, rounded once), for series whose files have different gains.  ct_radix_hist_f32 is
+ * legacy/minimal_psd.py:188-193 (float64 product, rounded once).  ct_dequant_u16 is
+ * plot-trace.py:272-287 alone (float64 affine, rounded once), for series whose files have
+ * different gains.  ct_radix_hist_f32 is
  * one 8-bit digit pass (most significant first) of an exact radix select over the
  * order-preserving uint32 keys of the floats (hist256: uint64[256], caller-zeroed): the
  * median np.pad(mode='median') needs for float input.                                    */
 int ct_bin_be_f64_to_f32(const void* records, int64_t n, float* out, void* stream);
-int ct_i2be_to_f32(const void* records, int64_t n, float gain, float* out, void* stream);
+int ct_i2be_to_f32(const void* records, int64_t n, double gain, float* out, void* stream);
 int ct_dequant_u16(const uint16_t* raw, int64_t n, uint16_t mask, double alpha, double beta, float* out,
                    void* stream);
 int ct_radix_hist_f32(const float* x, int64_t n, uint32_t prefix, int32_t prefix_bits, int32_t use_abs,

@@ -49,3 +49,29 @@ def test_window_reader_reads_ranges_across_files(tmp_path):
             rd.read_into(buf, x, y)
             assert np.array_equal(buf[:y - x], allc[lo + x:lo + y]) and not buf[y - x:].any()
         rd.close()
+    # files of odd lengths; windows inside files at both ends, from a file boundary (an empty first piece) and inside
+    # one file; about 200 ranges each: empty ones, single samples, every file boundary crossed, the whole window and
+    # random ones.  Nothing past b - a of the destination is written.
+    odd = os.path.join(str(tmp_path), "odd")
+    os.makedirs(odd)
+    first, allc = _write_series(odd, [5001, 7003, 3007], seed=5)
+    s = loader.ChimeraSeries(first)
+    fs, fsi = s.samplerate, s.file_start_index
+    rng = np.random.default_rng(6)
+    for a, b in ((101, 14_000), (5001, 14_900), (5100, 11_000)):
+        rd = s.reader((a + 0.25) / fs, (b + 0.25) / fs)
+        assert rd.n == b - a
+        bounds = [int(f) - a for f in fsi if a < f < b]
+        ranges = [(0, 0), (rd.n, rd.n), (0, 1), (rd.n - 1, rd.n), (0, rd.n)]
+        ranges += [(c, c) for c in bounds] + [(c - 1, c + 1) for c in bounds] + [(c, c + 1) for c in bounds]
+        if len(bounds) == 2:
+            ranges.append((bounds[0] - 3, bounds[1] + 3))
+        while len(ranges) < 200:
+            x, y = sorted(rng.integers(0, rd.n + 1, 2))
+            ranges.append((int(x), int(y)))
+        for x, y in ranges:
+            buf = np.full(y - x + 5, 0xA5A5, np.uint16)
+            rd.read_into(buf, x, y)
+            assert np.array_equal(buf[:y - x], allc[a + x:a + y]), (a, b, x, y)
+            assert np.all(buf[y - x:] == 0xA5A5), (a, b, x, y)
+        rd.close()
